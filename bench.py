@@ -8,6 +8,10 @@ plus train crops/sec and the projection's GB/s as extra keys on the same JSON li
 A step = one 512x512 summary image through the full 8x-TTA prediction on every rank (independent
 images per rank: weak scaling, no data-path collective).  `value` is device-timed with the input
 already in HBM; `e2e` goes through UNet2DSummary.predict with host buffers in and the mask out.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/mask.npy (float32 0/1) and
+DIR/act.npy (float64, the 8x-TTA averaged probability); inputs and weights are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -100,14 +104,22 @@ class ClockSampler(object):
 
 # ---------------------------------------------------------------------------------------------- CPU arm
 def cpu_forward_tta(w, s, spec, n_images):
-    """oracle port of predict(augmentation=True) (unet_2d_summary.py:585-595) in float32 on all host cores"""
+    """oracle port of predict(augmentation=True) (unet_2d_summary.py:585-595) in float32 on all host cores
+    -> (seconds, (mask, act) of the last image)"""
     import torch
     import oracle
     torch.set_num_threads(_HOST_CORES)
     t0 = time.perf_counter()
     for _ in range(n_images):
-        oracle.tta_predict(w, s, spec, augmentation=True, dtype=torch.float32)
-    return time.perf_counter() - t0
+        out = oracle.tta_predict(w, s, spec, augmentation=True, dtype=torch.float32)
+    return time.perf_counter() - t0, out
+
+
+def dump_outputs(path, mask, act):
+    """--dump-outputs: the arrays the timed path returned in its last step"""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, 'mask.npy'), np.asarray(mask, dtype=np.float32))
+    np.save(os.path.join(path, 'act.npy'), np.asarray(act, dtype=np.float64))
 
 
 def run_reference(args):
@@ -121,7 +133,9 @@ def run_reference(args):
     s = np.random.default_rng(865).standard_normal((512, 512)).astype(np.float32)
     for _ in range(min(args.warmup, 1)):
         cpu_forward_tta(w, s, spec, 1)
-    dt = cpu_forward_tta(w, s, spec, args.steps)
+    dt, (mask, act) = cpu_forward_tta(w, s, spec, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, mask, act)
     val = args.steps / dt
     cores = torch.get_num_threads()
     line = {'impl': 'reference', 'metric': METRIC, 'value': val, 'unit': 'images/s', 'n_gpus': args.gpus,
@@ -205,7 +219,7 @@ def cpu_baselines(w, img_host):
     # 8x TTA inference (the headline metric)
     cpu_forward_tta(w, img_host[:128, :128].copy(), ospec, 1)
     n_cpu = 2
-    dt = cpu_forward_tta(w, img_host, ospec, n_cpu)
+    dt = cpu_forward_tta(w, img_host, ospec, n_cpu)[0]
     head = {'value': n_cpu / dt, 'unit': 'images/s', 'cores': cores, 'kind': 'port',
             'sample': '%d TTA images (16 fp32 forwards) of the torch-CPU oracle port of the Keras graph' % n_cpu}
     # training step (fwd + bwd + Keras-Adam), fp32, the C3 batch
@@ -416,10 +430,12 @@ def run_ours(args):
     t_w0 = time.time()
     e0.record()
     for i in range(args.steps):
-        eng.predict_tta(imgs[i % n_img])
+        mask, act = eng.predict_tta(imgs[i % n_img])
     e1.record()
     barrier()
     t_w1 = time.time()
+    # predict_tta returns static buffers, which the end-to-end arm below overwrites
+    last = (mask.cpu().numpy(), act.cpu().numpy()) if args.dump_outputs and rank == 0 else None
     ms = max_over_ranks(e0.elapsed_time(e1))
     launches = eng.launches - launches0
     value = world * args.steps / (ms / 1e3)
@@ -540,6 +556,8 @@ def run_ours(args):
                 line['cpu_baseline'] = {'error': repr(ex)}
         else:
             line['cpu_baseline'] = None
+        if last is not None:
+            dump_outputs(args.dump_outputs, *last)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -840,7 +858,11 @@ def main():
                     help="activation / weight storage of the inference path: fp16 and bf16 run the same tcgen05 kind::f16 MMAs "
                          "(fp32 accumulate) at the same rate; fp16 meets the north star's 1e-2 logit tolerance, bf16 cannot "
                          "(tests/test_gpu_unet.py, DESIGN.md section 4); training extras always run in bf16 (or fp32)")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the mask and activation the last timed step returned as DIR/mask.npy and DIR/act.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -1,7 +1,10 @@
 """The pure-Python HDF5 subset (deepcalcium/utils/hdf5_lite.py) behind the reference's file formats (SURVEY N1 / N4):
 pinned against a GENUINE libhdf5-written file - the MATLAB v7.3 test file that ships with scipy - and by write / read
 round trips of the two layouts the reference uses (dataset schema of datasets/nf.py:39-44 and the Keras 2.0.6 model
-layout of utils/keras_helpers.py:24-68)."""
+layout of utils/keras_helpers.py:24-68).
+
+tests/golden/testhdf5_7.4_GLNX86.mat and testdouble_7.4_GLNX86.mat are copies of scipy's io/matlab test data,
+Copyright (c) 2001-2002 Enthought, Inc. 2003, SciPy Developers, under scipy's BSD 3-clause licence."""
 import os
 
 import numpy as np
@@ -10,26 +13,18 @@ import pytest
 from deepcalcium.utils import hdf5_lite as h5
 
 
-def _scipy_fixture(name):
-    import scipy.io
-    p = os.path.join(os.path.dirname(scipy.io.__file__), 'matlab', 'tests', 'data', name)
-    if not os.path.exists(p):
-        pytest.skip('scipy test data not installed')
-    return p
-
-
-def test_reads_a_genuine_libhdf5_file():
+def test_reads_a_genuine_libhdf5_file(golden_dir):
     """superblock v0 behind a 512-byte user block, symbol-table root group, v1 object header, contiguous float64 dataset
     (layout message v2), fixed-length string attribute - written by MATLAB 7.4 through libhdf5 in 2008.  The expected
     values come from the SAME variable stored in MATLAB's own (non-HDF5) v7 format, read by scipy."""
     import scipy.io
-    with h5.File(_scipy_fixture('testhdf5_7.4_GLNX86.mat'), 'r') as f:
+    with h5.File(os.path.join(golden_dir, 'testhdf5_7.4_GLNX86.mat'), 'r') as f:
         assert f.keys() == ['testdouble'] and 'testdouble' in f and 'nope' not in f
         ds = f['testdouble']
         assert ds.shape == (9, 1) and ds.dtype == np.dtype('<f8')
         assert ds.attrs['MATLAB_class'] == b'double'
         got = ds[...]
-    ref = scipy.io.loadmat(_scipy_fixture('testdouble_7.4_GLNX86.mat'))['testdouble']
+    ref = scipy.io.loadmat(os.path.join(golden_dir, 'testdouble_7.4_GLNX86.mat'))['testdouble']
     assert np.array_equal(got.ravel(), ref.ravel())
     assert np.allclose(got.ravel(), np.linspace(0, 2 * np.pi, 9))
 

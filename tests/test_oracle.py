@@ -6,6 +6,7 @@ import torch
 
 import oracle
 from oracle import losses as ol
+from oracle.make_golden import as_stored, golden_weights
 from oracle.unet import _convT2x2, keras_adam_update
 
 
@@ -97,14 +98,14 @@ def test_golden_projection(golden_dir):
 def test_golden_unet_forward_tta_train(golden_dir):
     z = np.load(golden_dir + '/unet_nfb4_32.npz')
     spec = oracle.UNetSpec(nb_filters_base=4)
-    w = {k[2:]: z[k] for k in z.files if k.startswith('w:')}
+    w = golden_weights(z)
     o = oracle.unet_forward(w, z['x'], spec)
     assert np.allclose(o['logit'].numpy(), z['logit'], atol=1e-10)
     mask, act = oracle.tta_predict(w, z['s'], spec, window=32, dtype=torch.float64)
     assert np.array_equal(mask, z['tta_mask']) and np.allclose(act, z['tta_act'], atol=1e-9)
     L, nw, st, g, _ = oracle.train_step(w, z['x'], z['y'], spec=spec, loss='dice_loss')
     assert abs(L - float(z['dice_loss:loss'])) < 1e-10
-    assert np.allclose(g['botb/kernel'], z['dice_loss:grad:botb/kernel'], atol=1e-12)
+    assert np.allclose(as_stored(z, 'botb/kernel', g['botb/kernel']), z['dice_loss:grad:botb/kernel'], atol=1e-12)
     assert np.allclose(nw['head/kernel'], z['dice_loss:new:head/kernel'], atol=1e-7)
 
 
