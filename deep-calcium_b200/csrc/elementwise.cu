@@ -722,49 +722,72 @@ __device__ __forceinline__ void tta_dst(int k, int S, int i, int j, int& a, int&
     default: tta_src(k, S, i, j, a, b); break;        // the other six are involutions
   }
 }
-__device__ __forceinline__ int reflect_index(int i, int n) {   // np.pad(mode='reflect')
+__device__ __forceinline__ int reflect_index(int i, int n) {   // np.pad(mode='reflect'), extended to negative i
   if (n == 1) return 0;
   const int period = 2 * (n - 1);
-  int r = i % period;
+  int r = (i < 0 ? -i : i) % period;
   return r < n ? r : period - r;
 }
 
-// s [hs][ws] f32 -> out [count][S][S]: reflect-pad bottom/right to S x S (unet_2d_summary.py:569-571)
-// then apply transforms first..first+count-1
+// Overlap-tile TTA.  The canvas is s [hs][ws] reflect-padded at the bottom and right (unet_2d_summary.py:569-571); a plan
+// cuts it into S x S tiles with origins (oy[ty], ox[tx]) over an n_ty x n_tx grid, numbered row-major.  A group is the
+// tiles tile_first..tile_first+n_tiles-1.  oy == ox == nullptr is the one-tile plan of the 512^2 window (origin 0).
+//
+// make_batch: out [n_tiles][count][S][S] = each tile of the group under transforms first..first+count-1.  The canvas is
+// never materialised: every pixel is read from s through reflect_index in canvas coordinates.
 template <typename T>
-__global__ void tta_make_batch_kernel(const float* __restrict__ s, int hs, int ws, int S, int first, int count,
-                                      T* __restrict__ out) {
-  const long long n = (long long)count * S * S;
+__global__ void tile_make_batch_kernel(const float* __restrict__ s, int hs, int ws, int S, const int* __restrict__ oy,
+                                       const int* __restrict__ ox, int n_tx, int tile_first, int n_tiles, int first,
+                                       int count, T* __restrict__ out) {
+  const long long per = (long long)S * S;
+  const long long n = (long long)n_tiles * count * per;
   if (threadIdx.x == 0) pdl_trigger();
   pdl_wait();
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long long)gridDim.x * blockDim.x) {
-    const int j = (int)(idx % S), i = (int)((idx / S) % S), kk = (int)(idx / ((long long)S * S));
+    const int j = (int)(idx % S), i = (int)((idx / S) % S);
+    const long long b = idx / per;
+    const int kk = (int)(b % count), t = tile_first + (int)(b / count);
+    const int y0 = oy ? oy[t / n_tx] : 0, x0 = ox ? ox[t % n_tx] : 0;
     int si, sj;
     tta_src(first + kk, S, i, j, si, sj);
-    out[idx] = from_f32<T>(s[(long long)reflect_index(si, hs) * ws + reflect_index(sj, ws)]);
+    out[idx] = from_f32<T>(s[(long long)reflect_index(y0 + si, hs) * ws + reflect_index(x0 + sj, ws)]);
   }
 }
 
-// probs [n_aug][S][S] -> act[hs][ws] (float64: sum_k float32(p_k / n_aug)), mask = act > threshold
-__global__ void tta_combine_kernel(const float* __restrict__ probs, int S, int hs, int ws, float threshold, int n_aug,
-                                   double* __restrict__ act, uint8_t* __restrict__ mask) {
-  const long long n = (long long)hs * ws;
+// combine: probs [n_tiles][n_aug][S][S] -> act / mask [hs][ws] at the image pixels the group's tiles own.  Tile (ty, tx)
+// owns canvas rows [cy[ty-1], cy[ty]) and columns [cx[tx-1], cx[tx]) (the first / last tile of a row or column from / to
+// the canvas edge; cy == cx == nullptr: the one tile owns everything).  act = sum_k float32(inv_k(p_k) / n_aug) in
+// float64, in transform order; mask = act > threshold.  Every pixel has exactly one owner and is written once, so the
+// result does not depend on how the tiles are grouped.
+__global__ void tile_combine_kernel(const float* __restrict__ probs, int S, int hs, int ws, const int* __restrict__ oy,
+                                    const int* __restrict__ ox, const int* __restrict__ cy, const int* __restrict__ cx,
+                                    int n_ty, int n_tx, int tile_first, int n_tiles, float threshold, int n_aug,
+                                    double* __restrict__ act, uint8_t* __restrict__ mask) {
+  const long long per = (long long)S * S;
+  const long long n = (long long)n_tiles * per;
   if (threadIdx.x == 0) pdl_trigger();
   pdl_wait();
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long long)gridDim.x * blockDim.x) {
-    const int j = (int)(idx % ws), i = (int)(idx / ws);
+    const int j = (int)(idx % S), i = (int)((idx / S) % S), lt = (int)(idx / per);
+    const int t = tile_first + lt, ty = t / n_tx, tx = t % n_tx;
+    const int y = (oy ? oy[ty] : 0) + i, x = (ox ? ox[tx] : 0) + j;
+    if (y < 0 || y >= hs || x < 0 || x >= ws) continue;
+    if (cy && ((ty > 0 && y < cy[ty - 1]) || (ty < n_ty - 1 && y >= cy[ty]))) continue;
+    if (cx && ((tx > 0 && x < cx[tx - 1]) || (tx < n_tx - 1 && x >= cx[tx]))) continue;
+    const float* p = probs + (long long)lt * n_aug * per;
     double acc = 0.0;
     if (n_aug == 1) {
-      acc = (double)probs[(long long)i * S + j];
+      acc = (double)p[(long long)i * S + j];
     } else {
       for (int k = 0; k < n_aug; ++k) {
         int a, b;
         tta_dst(k, S, i, j, a, b);
-        acc += (double)(probs[((long long)k * S + a) * S + b] / (float)n_aug);
+        acc += (double)(p[((long long)k * S + a) * S + b] / (float)n_aug);
       }
     }
-    if (act) act[idx] = acc;
-    mask[idx] = acc > (double)threshold ? 1 : 0;
+    const long long o = (long long)y * ws + x;
+    if (act) act[o] = acc;
+    mask[o] = acc > (double)threshold ? 1 : 0;
   }
 }
 
@@ -1077,31 +1100,66 @@ extern "C" int dcb_head_loss_bwd_rank1(int dtype, const void* x, long long M, in
   return DCB_OK;
 }
 
+static int launch_make_batch(int dtype, const float* s, int hs, int ws, int S, const int* oy, const int* ox, int n_tx,
+                             int tile_first, int n_tiles, int first, int count, void* out, dcb_stream_t stream) {
+  const bool pdl = policy(DCB_POLICY_PDL) != 0;
+  DISPATCH_T(dtype, {
+    const cudaError_t le = launch_k(tile_make_batch_kernel<T>, ew_grid((long long)n_tiles * count * S * S, 256), 256, 0,
+                                    (cudaStream_t)stream, pdl, s, hs, ws, S, oy, ox, n_tx, tile_first, n_tiles, first, count,
+                                    (T*)out);
+    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tile_make_batch_kernel failed: %s", cudaGetErrorString(le));
+  })
+  g_launches += 1;
+  return DCB_OK;
+}
+
+static int launch_combine(const float* probs, int S, int hs, int ws, const int* oy, const int* ox, const int* cy,
+                          const int* cx, int n_ty, int n_tx, int tile_first, int n_tiles, float threshold, int n_aug,
+                          double* act, uint8_t* mask, dcb_stream_t stream) {
+  const cudaError_t le = launch_k(tile_combine_kernel, ew_grid((long long)n_tiles * S * S, 256), 256, 0, (cudaStream_t)stream,
+                                  policy(DCB_POLICY_PDL) != 0, probs, S, hs, ws, oy, ox, cy, cx, n_ty, n_tx, tile_first,
+                                  n_tiles, threshold, n_aug, act, mask);
+  if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tile_combine_kernel failed: %s", cudaGetErrorString(le));
+  g_launches += 1;
+  return DCB_OK;
+}
+
 extern "C" int dcb_tta_make_batch(int dtype, const float* s, int hs, int ws, int S, int first, int count, void* out,
                                   dcb_stream_t stream) {
   DCB_CHECK_ARG(s && out && hs > 0 && ws > 0 && hs <= S && ws <= S, "dcb_tta_make_batch: image %dx%d does not fit window %d", hs, ws, S);
   DCB_CHECK_ARG(first >= 0 && count > 0 && first + count <= 8, "dcb_tta_make_batch: transforms [%d,%d) out of range", first, first + count);
-  const bool pdl = policy(DCB_POLICY_PDL) != 0;
-  DISPATCH_T(dtype, {
-    const cudaError_t le = launch_k(tta_make_batch_kernel<T>, ew_grid((long long)count * S * S, 256), 256, 0, (cudaStream_t)stream, pdl,
-                                    s, hs, ws, S, first, count, (T*)out);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tta_make_batch_kernel failed: %s", cudaGetErrorString(le));
-  })
-  g_launches += 1;
-  return DCB_OK;
+  return launch_make_batch(dtype, s, hs, ws, S, nullptr, nullptr, 1, 0, 1, first, count, out, stream);
 }
 
 extern "C" int dcb_tta_combine(const float* probs, int S, int hs, int ws, float threshold, int n_aug, double* act,
                                uint8_t* mask, dcb_stream_t stream) {
   DCB_CHECK_ARG(probs && mask && hs > 0 && ws > 0 && hs <= S && ws <= S, "dcb_tta_combine: bad arguments");
   DCB_CHECK_ARG(n_aug == 1 || n_aug == 8, "dcb_tta_combine: n_aug must be 1 or 8 (got %d)", n_aug);
-  {
-    const cudaError_t le = launch_k(tta_combine_kernel, ew_grid((long long)hs * ws, 256), 256, 0, (cudaStream_t)stream,
-                                    policy(DCB_POLICY_PDL) != 0, probs, S, hs, ws, threshold, n_aug, act, mask);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tta_combine_kernel failed: %s", cudaGetErrorString(le));
-  }
-  g_launches += 1;
-  return DCB_OK;
+  return launch_combine(probs, S, hs, ws, nullptr, nullptr, nullptr, nullptr, 1, 1, 0, 1, threshold, n_aug, act, mask, stream);
+}
+
+extern "C" int dcb_tile_make_batch(int dtype, const float* s, int hs, int ws, int T, const int* origins_y,
+                                   const int* origins_x, int n_ty, int n_tx, int tile_first, int n_tiles, int first, int count,
+                                   void* out, dcb_stream_t stream) {
+  DCB_CHECK_ARG(s && out && origins_y && origins_x && hs > 0 && ws > 0 && T > 0 && n_ty > 0 && n_tx > 0,
+                "dcb_tile_make_batch: bad arguments");
+  DCB_CHECK_ARG(tile_first >= 0 && n_tiles > 0 && (long long)tile_first + n_tiles <= (long long)n_ty * n_tx,
+                "dcb_tile_make_batch: tiles [%d,%d) outside the %dx%d plan", tile_first, tile_first + n_tiles, n_ty, n_tx);
+  DCB_CHECK_ARG(first >= 0 && count > 0 && first + count <= 8, "dcb_tile_make_batch: transforms [%d,%d) out of range", first, first + count);
+  return launch_make_batch(dtype, s, hs, ws, T, origins_y, origins_x, n_tx, tile_first, n_tiles, first, count, out, stream);
+}
+
+extern "C" int dcb_tile_combine(const float* probs, int T, int hs, int ws, const int* origins_y, const int* origins_x,
+                                const int* cuts_y, const int* cuts_x, int n_ty, int n_tx, int tile_first, int n_tiles,
+                                float threshold, int n_aug, double* act, uint8_t* mask, dcb_stream_t stream) {
+  DCB_CHECK_ARG(probs && mask && origins_y && origins_x && hs > 0 && ws > 0 && T > 0 && n_ty > 0 && n_tx > 0,
+                "dcb_tile_combine: bad arguments");
+  DCB_CHECK_ARG((cuts_y || n_ty == 1) && (cuts_x || n_tx == 1), "dcb_tile_combine: a plan with several tiles needs its cuts");
+  DCB_CHECK_ARG(tile_first >= 0 && n_tiles > 0 && (long long)tile_first + n_tiles <= (long long)n_ty * n_tx,
+                "dcb_tile_combine: tiles [%d,%d) outside the %dx%d plan", tile_first, tile_first + n_tiles, n_ty, n_tx);
+  DCB_CHECK_ARG(n_aug == 1 || n_aug == 8, "dcb_tile_combine: n_aug must be 1 or 8 (got %d)", n_aug);
+  return launch_combine(probs, T, hs, ws, origins_y, origins_x, cuts_y, cuts_x, n_ty, n_tx, tile_first, n_tiles, threshold,
+                        n_aug, act, mask, stream);
 }
 
 extern "C" int dcb_adam_step(float* p, const float* g, float* m, float* v, long long n, float lr_t,

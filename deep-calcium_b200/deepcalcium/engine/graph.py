@@ -160,3 +160,121 @@ def list_to_weights(spec, lst):
             raise ValueError('weight %s: expected shape %s, got %s' % (k, shapes[k], a.shape))
         out[k] = a
     return out
+
+
+# ------------------------------------------------------------------ overlap-tile inference for images larger than the window
+MAX_TILE = 2048          # largest tile edge: a 2048^2 canvas is one tile; a batch holds at most 8 * MAX_TILE^2 pixels
+
+
+def receptive_reach(spec, block=16):
+    """How far (in input pixels, on either side) the outputs of a ``block``-aligned run of ``block`` output pixels reach
+    into the input: a 1-D dependency pass over the graph (conv 3x3 widens by one position at its level, max-pool and
+    convT 2x2 / nearest upsampling are 2x index maps, the skip paths join by union).  Returns (left, right)."""
+    def memo(fn):
+        cache = {}
+
+        def g(p):
+            r = cache.get(p)
+            if r is None:
+                r = cache[p] = fn(p)
+            return r
+        return g
+
+    # each tensor is a map: position at its level -> [lo, hi] interval of input positions it depends on; all maps are
+    # non-decreasing in both ends, so a window's interval is (lo of its first position, hi of its last)
+    def conv(f):
+        return memo(lambda p: (f(p - 1)[0], f(p + 1)[1]))
+
+    def pool(f):
+        return memo(lambda p: (f(2 * p)[0], f(2 * p + 1)[1]))
+
+    def up(f):
+        return memo(lambda p: f(p // 2))
+
+    def cat(f, g):
+        return memo(lambda p: (min(f(p)[0], g(p)[0]), max(f(p)[1], g(p)[1])))
+
+    t, skips = (lambda p: (p, p)), {}
+    for blk in spec.blocks:
+        if blk.kind == 'up':
+            t = up(t)
+        elif blk.kind == 'conv':
+            if blk.name.startswith('dec') and blk.name.endswith('a'):
+                t = cat(up(t) if spec.up_mode == 'upsampling' else t, skips[blk.level])
+            t = conv(t)
+            if blk.name.startswith('enc') and blk.name.endswith('b'):
+                skips[blk.level] = t
+                t = pool(t)
+    return -t(0)[0], t(block - 1)[1] - (block - 1)
+
+
+def tile_halo(spec):
+    """h: the smallest multiple of 16 that covers the receptive reach.  A pixel at least h from every tile edge that is
+    not a canvas edge gets the same prediction from the tile as from the whole canvas."""
+    return -(-max(receptive_reach(spec)) // 16) * 16
+
+
+def _round16(n):
+    return -(-n // 16) * 16
+
+
+def _plan_1d(C, T, h):
+    """tile origins and ownership cuts along one canvas dimension of C pixels"""
+    if C == T:
+        return [0], []
+    n = -(-(C - 2 * h) // (T - 2 * h))
+    while True:
+        # o_k = 16 * round(k (C - T) / (16 (n - 1))), halves rounded up
+        o = [16 * ((2 * k * (C - T) + 16 * (n - 1)) // (32 * (n - 1))) for k in range(n)]
+        if all(o[k + 1] - o[k] <= T - 2 * h for k in range(n - 1)):
+            break
+        n += 1
+    return o, [(o[k] + o[k + 1] + T) // 2 for k in range(n - 1)]
+
+
+class TilePlan(object):
+    """Square T x T tiles over the canvas (the image reflect-padded at the bottom and right to C_h x C_w,
+    C_d = max(T, roundup16(size_d))).  Tile (ty, tx) has its origin at (origins[0][ty], origins[1][tx]) and owns canvas
+    rows [cuts[0][ty-1], cuts[0][ty]) and columns [cuts[1][tx-1], cuts[1][tx]) (up to the canvas edge at either end)."""
+    __slots__ = ('shape', 'tile', 'halo', 'canvas', 'origins', 'cuts')
+
+    def __init__(self, shape, tile, halo, canvas, origins, cuts):
+        self.shape, self.tile, self.halo, self.canvas, self.origins, self.cuts = shape, tile, halo, canvas, origins, cuts
+
+    @property
+    def grid(self):
+        return len(self.origins[0]), len(self.origins[1])
+
+    @property
+    def n_tiles(self):
+        return len(self.origins[0]) * len(self.origins[1])
+
+    def computed_pixels(self):
+        return self.n_tiles * self.tile * self.tile
+
+    def key(self):
+        return (self.shape, self.tile, tuple(map(tuple, self.origins)), tuple(map(tuple, self.cuts)))
+
+
+def plan_tiles(shape, halo, tile=None, max_tile=MAX_TILE):
+    """Tile plan for an image of ``shape`` = (hs, ws).  Origins are multiples of 16 (the four max-pools see the canvas'
+    phase), every tile lies inside the canvas (per-layer zero padding happens at the real canvas edge), and every pixel is
+    owned by one tile and lies at least ``halo`` from each of its tile's edges that is not a canvas edge.
+    ``tile=None`` picks T among the multiples of 128 in [512, max_tile] that minimise the computed pixels (ties: fewer
+    tiles); an explicit ``tile`` must be a multiple of 16 greater than 2 * halo."""
+    hs, ws = int(shape[0]), int(shape[1])
+    if hs <= 0 or ws <= 0:
+        raise ValueError('empty image %s' % (shape,))
+    if tile is None:
+        best = None
+        for T in range(512, max_tile + 1, 128):
+            p = plan_tiles((hs, ws), halo, T)
+            if best is None or (p.computed_pixels(), p.n_tiles) < (best.computed_pixels(), best.n_tiles):
+                best = p
+        return best
+    T = int(tile)
+    if T % 16 or T <= 2 * halo:
+        raise ValueError('tile %d must be a multiple of 16 greater than twice the halo (%d)' % (T, halo))
+    canvas = (max(T, _round16(hs)), max(T, _round16(ws)))
+    per_dim = [_plan_1d(C, T, halo) for C in canvas]
+    return TilePlan((hs, ws), T, halo, canvas, [o for o, _ in per_dim], [c for _, c in per_dim])

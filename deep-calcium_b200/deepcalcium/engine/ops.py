@@ -446,6 +446,28 @@ def tta_combine(probs, S, hs, ws, threshold, n_aug, act, mask):
          ptr(mask), stream_ptr())
 
 
+def tile_make_batch(s, T, origins_y, origins_x, tile_first, n_tiles, first, count, out):
+    """the tiles tile_first.. of a plan (device int32 origins per dimension) under transforms first..first+count-1 ->
+    out [n_tiles * count, T, T]"""
+    _chk(s, torch.float32); _chk(origins_y, torch.int32); _chk(origins_x, torch.int32)
+    hs, ws = s.shape
+    call('dcb_tile_make_batch', _dt(out), ptr(s), c_int(hs), c_int(ws), c_int(T), ptr(origins_y), ptr(origins_x),
+         c_int(origins_y.numel()), c_int(origins_x.numel()), c_int(tile_first), c_int(n_tiles), c_int(first), c_int(count),
+         ptr(out), stream_ptr())
+
+
+def tile_combine(probs, T, origins_y, origins_x, cuts_y, cuts_x, tile_first, n_tiles, threshold, n_aug, act, mask):
+    """act / mask [hs, ws] at the pixels owned by the tiles tile_first..tile_first+n_tiles-1 of the plan"""
+    _chk(probs, torch.float32); _chk(mask, torch.uint8)
+    for t in (origins_y, origins_x, cuts_y, cuts_x):
+        _chk(t, torch.int32)
+    hs, ws = mask.shape
+    call('dcb_tile_combine', ptr(probs), c_int(T), c_int(hs), c_int(ws), ptr(origins_y), ptr(origins_x),
+         ptr(cuts_y if cuts_y.numel() else None), ptr(cuts_x if cuts_x.numel() else None), c_int(origins_y.numel()),
+         c_int(origins_x.numel()), c_int(tile_first), c_int(n_tiles), c_f(threshold), c_int(n_aug), ptr(act), ptr(mask),
+         stream_ptr())
+
+
 # ---------------------------------------------------------------- optimiser
 def adam_step(p, g, m, v, lr_t=0., lr_t_dev=None, beta1=0.9, beta2=0.999, eps=1e-8):
     call('dcb_adam_step', ptr(p), ptr(g), ptr(m), ptr(v), c_ll(p.numel()), c_f(lr_t), ptr(lr_t_dev), c_f(beta1),

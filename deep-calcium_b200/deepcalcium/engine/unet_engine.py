@@ -16,7 +16,8 @@ import torch
 
 from .. import _native as nat
 from . import ops
-from .graph import GraphSpec, BN_EPS, BN_MOMENTUM_CONV, BN_MOMENTUM_UP, TRAINABLE, he_normal_weights
+from .graph import (GraphSpec, BN_EPS, BN_MOMENTUM_CONV, BN_MOMENTUM_UP, TRAINABLE, MAX_TILE, he_normal_weights, plan_tiles,
+                    tile_halo)
 
 _PRECISIONS = {'bf16': torch.bfloat16, 'fp16': torch.float16, 'f16': torch.float16, 'fp32': torch.float32, 'f32': torch.float32}
 
@@ -68,6 +69,9 @@ class UNetEngine(object):
         # CTAs of the next main-chain kernel take the SM slots in which the weight-gradient side stream overlapped
         self.pdl_train = os.environ.get('DCB_PDL_TRAIN', '0') != '0'
         self._side = None
+        self.halo = tile_halo(self.spec)
+        # predict_tiled runs its tiles in groups of at most this many batch pixels (8 transforms of one MAX_TILE^2 tile)
+        self.tile_batch_pixels = 8 * MAX_TILE * MAX_TILE
         self.set_weights_dict(he_normal_weights(self.spec, seed=0))
 
     # ------------------------------------------------------------------ parameter storage
@@ -408,6 +412,56 @@ class UNetEngine(object):
         self._run_graphed(s['tta_graphs'], key, run)
         if transforms is not None:
             return s['prob']
+        return st['mask'], st['act']
+
+    def _batch_prefix(self, s, nb):
+        """session s restricted to its first nb images (views of its buffers): the last, smaller group of a tile plan"""
+        if nb == s['NB']:
+            return s
+        v = s.setdefault('prefixes', {}).get(nb)
+        if v is None:
+            v = dict(NB=nb, H=s['H'], W=s['W'], training=False, x=s['x'][:nb], logit=s['logit'][:nb], prob=s['prob'][:nb],
+                     act={k: a[:nb] for k, a in s['act'].items()})
+            s['prefixes'][nb] = v
+        return v
+
+    @_on_engine_device
+    def predict_tiled(self, summ_dev, augmentation=True, threshold=0.5, tile=None):
+        """predict_tta for a summary image of any size (fp32 [hs,ws] on the device): the reference's TTA computed on the
+        canvas (the image reflect-padded at the bottom and right to C_h x C_w, C_d = max(T, roundup16(size_d))) and cropped
+        to hs x ws.  The canvas runs as square T x T tiles (graph.plan_tiles; ``tile=None`` picks T) that overlap by the
+        network's receptive reach, so every pixel gets exactly the whole-canvas prediction from the one tile that owns
+        it.  Tiles go through the 8-transform batch in groups of at most tile_batch_pixels batch pixels; one CUDA graph
+        holds every group.  Returns (mask uint8 [hs,ws], act float64 [hs,ws]) as device tensors (static buffers)."""
+        hs, ws = summ_dev.shape
+        plan = plan_tiles((hs, ws), self.halo, tile)
+        T, n_aug = plan.tile, (8 if augmentation else 1)
+        per_group = min(plan.n_tiles, max(1, self.tile_batch_pixels // (n_aug * T * T)))
+        s = self._session(per_group * n_aug, T, T, False)
+        key = ('tiled', n_aug, float(threshold), plan.key())
+        st = s['tta_graphs'].get(('bufs',) + key)
+        if st is None:
+            i32 = dict(dtype=torch.int32, device=self.dev)
+            st = dict(summ=torch.zeros(hs, ws, dtype=torch.float32, device=self.dev),
+                      mask=torch.zeros(hs, ws, dtype=torch.uint8, device=self.dev),
+                      act=torch.zeros(hs, ws, dtype=torch.float64, device=self.dev),
+                      oy=torch.tensor(plan.origins[0], **i32), ox=torch.tensor(plan.origins[1], **i32),
+                      cy=torch.tensor(plan.cuts[0], **i32), cx=torch.tensor(plan.cuts[1], **i32))
+            s['tta_graphs'][('bufs',) + key] = st
+        self._ensure_inference_ready()
+        st['summ'].copy_(summ_dev)
+
+        def run():
+            with nat.policy(pdl=1 if self.pdl else 0):
+                for t0 in range(0, plan.n_tiles, per_group):
+                    nt = min(per_group, plan.n_tiles - t0)
+                    g = self._batch_prefix(s, nt * n_aug)
+                    ops.tile_make_batch(st['summ'], T, st['oy'], st['ox'], t0, nt, 0, n_aug, g['x'])
+                    self._forward_inference(g)
+                    ops.tile_combine(g['prob'], T, st['oy'], st['ox'], st['cy'], st['cx'], t0, nt, threshold, n_aug,
+                                     st['act'], st['mask'])
+
+        self._run_graphed(s['tta_graphs'], key + (per_group,), run)
         return st['mask'], st['act']
 
     # ------------------------------------------------------------------ training

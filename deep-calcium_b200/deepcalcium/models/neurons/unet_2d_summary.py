@@ -347,6 +347,14 @@ class UNet2DSummary(object):
         def pad(x):
             return np.pad(x, ((0, hw - x.shape[0]), (0, ww - x.shape[1])), 'reflect')
 
+        def predict(x):
+            if x.shape[0] <= hw and x.shape[1] <= ww:
+                return self._predict_window(model, pad(x), hw)[:x.shape[0], :x.shape[1]]
+            # larger than the validation window: the identity transform over overlapping tiles (probabilities)
+            import torch
+            xd = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float32)).to(model.engine.dev)
+            return model.engine.predict_tiled(xd, augmentation=False)[1].cpu().numpy()
+
         fwd = [lambda x: x, np.fliplr, np.flipud, lambda x: np.rot90(x, 1), lambda x: np.rot90(x, 2),
                lambda x: np.rot90(x, 3)]
         pp, rr, ff = [], [], []
@@ -357,7 +365,7 @@ class UNet2DSummary(object):
                 fs, fm = f(s), f(m)
                 yy, xx = np.where(f(vm) == 1)
                 a0, a1, b0, b1 = min(yy), max(yy), min(xx), max(xx)
-                mp = self._predict_window(model, pad(fs), hw)[:fs.shape[0], :fs.shape[1]]
+                mp = predict(fs)
                 p, r, _, _, f1 = nf_mask_metrics(fm[a0:a1, b0:b1], mp[a0:a1, b0:b1].round())
                 pp.append(p); rr.append(r); ff.append(f1)
         eps = 1e-4 * epoch if epoch else 0
@@ -497,9 +505,13 @@ class UNet2DSummary(object):
         def stage(i):
             dsp = dataset_paths[i]
             summ = np.ascontiguousarray(np.asarray(self.series_summary_func(dsp), dtype=np.float32))
-            if summ.shape[0] > window_shape[0] or summ.shape[1] > window_shape[1]:
-                raise ValueError('summary image %s larger than the window %s' % (summ.shape, window_shape))
             sl = slots[i % 2]
+            # an image larger than the window is predicted from overlapping tiles (engine.predict_tiled), outside the
+            # pipeline: its own compute dwarfs the staging this pipeline hides
+            sl['large'] = summ.shape[0] > window_shape[0] or summ.shape[1] > window_shape[1]
+            if sl['large']:
+                sl['summ'] = summ
+                return
             cfg = (summ.shape, bool(augmentation), float(threshold))
             if sl.get('cfg') != cfg:
                 bufs = model.engine.tta_buffers(summ.shape, window=window_shape[0], augmentation=augmentation,
@@ -529,8 +541,11 @@ class UNet2DSummary(object):
             dsp = dataset_paths[i]
             name = self.dataset_name_func(dsp)
             sl = slots[i % 2]
-            sl['done'].synchronize()
-            mp = sl['hout'].numpy().copy()
+            if sl['large']:
+                mp = sl.pop('mp')
+            else:
+                sl['done'].synchronize()
+                mp = sl['hout'].numpy().copy()
             Mp.append(mp)
             names.append(name)
             if print_scores:
@@ -554,15 +569,21 @@ class UNet2DSummary(object):
             stage(0)
         for i, dsp in enumerate(dataset_paths):
             sl = slots[i % 2]
-            main = torch.cuda.current_stream(dev)
-            main.wait_event(sl['ready'])
-            model.engine.predict_tta(sl['din'], window=window_shape[0], augmentation=augmentation, threshold=threshold,
-                                     slot=i % 2)
-            sl['computed'].record(main)
-            with torch.cuda.stream(down_stream):           # this slot's mask buffer is not touched again before finalize(i)
-                down_stream.wait_event(sl['computed'])
-                sl['hout'].copy_(sl['dmask'], non_blocking=True)
-                sl['done'].record(down_stream)
+            if sl['large']:
+                # the mask leaves before the next image runs: a later image of the same shape reuses its buffers
+                mask, _ = model.engine.predict_tiled(torch.from_numpy(sl['summ']).to(dev), augmentation=augmentation,
+                                                     threshold=threshold)
+                sl['mp'] = mask.cpu().numpy()
+            else:
+                main = torch.cuda.current_stream(dev)
+                main.wait_event(sl['ready'])
+                model.engine.predict_tta(sl['din'], window=window_shape[0], augmentation=augmentation, threshold=threshold,
+                                         slot=i % 2)
+                sl['computed'].record(main)
+                with torch.cuda.stream(down_stream):       # this slot's mask buffer is not touched again before finalize(i)
+                    down_stream.wait_event(sl['computed'])
+                    sl['hout'].copy_(sl['dmask'], non_blocking=True)
+                    sl['done'].record(down_stream)
             # image i is now queued on the GPU; meanwhile collect image i-1 (frees its slot) and stage image i+1 into it
             if i >= 1:
                 finalize(i - 1)

@@ -117,6 +117,53 @@ def tta_source_index(k, S, i, j):
             (S - 1 - j, i), (j, i), (S - 1 - j, S - 1 - i)][k]
 
 
+def _reflect(i, n):
+    """np.pad(mode='reflect') index map, extended to negative indices (reflect_index in csrc/elementwise.cu)"""
+    if n == 1:
+        return np.zeros_like(i)
+    r = np.abs(i) % (2 * (n - 1))
+    return np.where(r < n, r, 2 * (n - 1) - r)
+
+
+def tile_make_batch_host(s, T, origins_y, origins_x, tile_first, n_tiles, first, count):
+    """Host statement of dcb_tile_make_batch: [n_tiles * count, T, T] float32, the tiles tile_first.. of the plan (row-major
+    over the origin grid) cut from the bottom / right reflect-padded canvas, each under transforms first..first+count-1."""
+    s = np.asarray(s, np.float32)
+    hs, ws = s.shape
+    out = np.empty((n_tiles * count, T, T), np.float32)
+    for lt in range(n_tiles):
+        t = tile_first + lt
+        y0, x0 = origins_y[t // len(origins_x)], origins_x[t % len(origins_x)]
+        tile = s[np.ix_(_reflect(np.arange(y0, y0 + T), hs), _reflect(np.arange(x0, x0 + T), ws))][None]
+        for kk in range(count):
+            out[lt * count + kk] = INVERTIBLE_2D_AUGMENTATIONS[first + kk][1](tile)[0]
+    return out
+
+
+def tile_combine_host(probs, T, hs, ws, origins_y, origins_x, cuts_y, cuts_x, tile_first, n_tiles, n_aug, act=None):
+    """Host statement of dcb_tile_combine: writes act [hs, ws] (float64) at the pixels owned by the group's tiles, the sum
+    over the transforms in order of inv_k(p_k) / n_aug taken in the dtype of ``probs`` (float32 on the device).  Returns
+    act; the mask is act > threshold."""
+    act = np.zeros((hs, ws)) if act is None else act
+    n_ty, n_tx = len(origins_y), len(origins_x)
+    for lt in range(n_tiles):
+        t = tile_first + lt
+        ty, tx = t // n_tx, t % n_tx
+        y0, x0 = origins_y[ty], origins_x[tx]
+        p = probs[lt * n_aug:(lt + 1) * n_aug]
+        acc = np.zeros((T, T))
+        if n_aug == 1:
+            acc += p[0]
+        else:
+            for k, (_, _, inv) in enumerate(INVERTIBLE_2D_AUGMENTATIONS):
+                acc += inv(p[k:k + 1])[0] / n_aug
+        r0, r1 = max(y0, cuts_y[ty - 1] if ty > 0 else 0), min(y0 + T, cuts_y[ty] if ty < n_ty - 1 else y0 + T, hs)
+        c0, c1 = max(x0, cuts_x[tx - 1] if tx > 0 else 0), min(x0 + T, cuts_x[tx] if tx < n_tx - 1 else x0 + T, ws)
+        if r0 < r1 and c0 < c1:
+            act[r0:r1, c0:c1] = acc[r0 - y0:r1 - y0, c0 - x0:c1 - x0]
+    return act
+
+
 # ---------------------------------------------------------------------------------------------- outlined figures
 _COLORS = {'red': (1., 0., 0.), 'blue': (0., 0., 1.), 'green': (0., 0.5, 0.), 'white': (1., 1., 1.), 'yellow': (1., 1., 0.)}
 

@@ -342,6 +342,20 @@ int dcb_tta_make_batch(int dtype, const float* s, int hs, int ws, int S, int fir
                        dcb_stream_t stream);
 int dcb_tta_combine(const float* probs, int S, int hs, int ws, float threshold, int n_aug, double* act,
                     uint8_t* mask, dcb_stream_t stream);
+/* Overlap-tile TTA for images larger than the window.  The canvas is s[hs][ws] reflect-padded at the bottom and right; a
+ * plan cuts it into T x T tiles with origins (origins_y[ty], origins_x[tx]) on an n_ty x n_tx grid, numbered row-major,
+ * and tile (ty, tx) owns canvas rows [cuts_y[ty-1], cuts_y[ty]) and columns [cuts_x[tx-1], cuts_x[tx]) (n_ty - 1 and
+ * n_tx - 1 cuts; the first and last tile own up to the canvas edge).  The plan arrays are caller-owned device int32 arrays,
+ * so a captured CUDA graph keeps reading the same plan.  A call handles the group of tiles tile_first..tile_first+n_tiles-1.
+ * make_batch: out [n_tiles][count][T][T] = each tile of the group under transforms first..first+count-1;
+ * combine: probs [n_tiles][n_aug][T][T] -> act / mask at the image pixels the group owns (act = sum_k float32(inv_k(p_k) /
+ * n_aug) in float64, mask = act > threshold); every pixel is written by exactly one group. */
+int dcb_tile_make_batch(int dtype, const float* s, int hs, int ws, int T, const int* origins_y, const int* origins_x,
+                        int n_ty, int n_tx, int tile_first, int n_tiles, int first, int count, void* out,
+                        dcb_stream_t stream);
+int dcb_tile_combine(const float* probs, int T, int hs, int ws, const int* origins_y, const int* origins_x,
+                     const int* cuts_y, const int* cuts_x, int n_ty, int n_tx, int tile_first, int n_tiles, float threshold,
+                     int n_aug, double* act, uint8_t* mask, dcb_stream_t stream);
 
 /* ---- a9: keras.optimizers.Adam (2.0.6) over one flat fp32 parameter buffer;
  * lr_t = lr*sqrt(1-b2^t)/(1-b1^t) is computed by the caller (unet_2d_summary.py:335) ---- */
