@@ -187,8 +187,8 @@ def attach_peers(engine, comm, group=None):
         engine.peers = None
         return None
     group = group or PeerGroup(comm)
-    cmax = max(b.cout for b in engine.spec.blocks)
-    n_slots = 2 * (len(engine.spec.blocks) + 8) + 2
+    cmax = max(b.cout for b in engine.dspec.blocks)
+    n_slots = 2 * (len(engine.dspec.blocks) + 8) + 2
     slot_doubles = comm.world * 2 * cmax
     xchg = group.alloc(n_slots * slot_doubles * 8)
     flags = group.alloc(n_slots * 8 * 8)

@@ -41,33 +41,65 @@ class Block(object):
         return shp
 
 
-class GraphSpec(object):
-    """Arguments of the reference's ``unet()`` (unet_2d_summary.py:123-124)."""
+# ------------------------------------------------------------------ device channel layout of the 16-bit precisions
+MAX_NFB_16BIT = 64       # padded_width is defined up to 1024 channels: the bottleneck of nb_filters_base 64
 
-    def __init__(self, nb_filters_base=32, prop_dropout_base=0.25, upsampling_or_transpose='transpose'):
+
+def padded_width(c):
+    """Channel width a c-channel tensor takes on the device in the 16-bit precisions: max(32, next power of two >= c).
+    It is the smallest width that the tensor-core convolutions (multiples of 32), the first-layer conv (Cout in
+    {8, 16, 32, 64}) and the single-launch BatchNorm kernels (a power of two <= 1024) all accept.  Powers of two from
+    32 up map to themselves."""
+    c = int(c)
+    if not 1 <= c <= 1024:
+        raise ValueError('no 16-bit device layout for %d channels (1 ... 1024)' % c)
+    return max(32, 1 << (c - 1).bit_length())
+
+
+class GraphSpec(object):
+    """Arguments of the reference's ``unet()`` (unet_2d_summary.py:123-124).
+
+    ``padded=True`` gives the device spec of the 16-bit precisions (see device_spec): the same graph with every tensor
+    width c stored as padded_width(c) channels, so the concat input of a dec<l>a block is padded_width(up) +
+    padded_width(skip) channels.  The network input (1 channel) and the head output (2 channels) keep their widths."""
+
+    def __init__(self, nb_filters_base=32, prop_dropout_base=0.25, upsampling_or_transpose='transpose', padded=False):
         assert upsampling_or_transpose in ('transpose', 'upsampling')
         self.nfb = int(nb_filters_base)
         self.drp = float(prop_dropout_base)
         self.up_mode = upsampling_or_transpose
-        n = self.nfb
-        b = [Block('enc0a', 'conv', 1, n, 0), Block('enc0b', 'conv', n, n, 0)]
+        self.padded = bool(padded)
+        n, P = self.nfb, (padded_width if padded else int)
+        b = [Block('enc0a', 'conv', 1, P(n), 0), Block('enc0b', 'conv', P(n), P(n), 0)]
         for lvl in (1, 2, 3):
             w = n << lvl
-            b += [Block('enc%da' % lvl, 'conv', w // 2, w, lvl), Block('enc%db' % lvl, 'conv', w, w, lvl)]
-        b += [Block('bota', 'conv', 8 * n, 16 * n, 4), Block('botb', 'conv', 16 * n, 16 * n, 4)]
+            b += [Block('enc%da' % lvl, 'conv', P(w // 2), P(w), lvl), Block('enc%db' % lvl, 'conv', P(w), P(w), lvl)]
+        b += [Block('bota', 'conv', P(8 * n), P(16 * n), 4), Block('botb', 'conv', P(16 * n), P(16 * n), 4)]
+        self.cat_split = OrderedDict()     # dec<l>a -> how many of its input channels come from the up path (the rest: skip)
         c = 16 * n
         for lvl in (3, 2, 1, 0):
             w = n << lvl
             if self.up_mode == 'transpose':
-                b.append(Block('up%d' % lvl, 'up', c, w, lvl))
-                cat = 2 * w
+                b.append(Block('up%d' % lvl, 'up', P(c), P(w), lvl))
+                up = P(w)
             else:
-                cat = c + w
-            b += [Block('dec%da' % lvl, 'conv', cat, w, lvl), Block('dec%db' % lvl, 'conv', w, w, lvl)]
+                up = P(c)
+            self.cat_split['dec%da' % lvl] = up
+            b += [Block('dec%da' % lvl, 'conv', up + P(w), P(w), lvl), Block('dec%db' % lvl, 'conv', P(w), P(w), lvl)]
             c = w
-        b.append(Block('head', 'head', n, 2, 0))
+        b.append(Block('head', 'head', P(n), 2, 0))
         self.blocks = b
         self.by_name = OrderedDict((x.name, x) for x in b)
+
+    def device_spec(self, precision):
+        """The spec the engine allocates and launches with: padded for 'bf16' / 'fp16', this spec for the fp32 check
+        mode, whose kernels take any width.  nb_filters_base 32 and 64 pad to themselves."""
+        if precision == 'fp32' or self.padded:
+            return self
+        if not 1 <= self.nfb <= MAX_NFB_16BIT:
+            raise ValueError("precision %r supports nb_filters_base 1 ... %d (got %d); use precision='fp32'"
+                             % (precision, MAX_NFB_16BIT, self.nfb))
+        return GraphSpec(self.nfb, self.drp, self.up_mode, padded=True)
 
     def dropout_after(self):
         """{tensor name: drop probability}, unet_2d_summary.py:179,185,191,198,204,210,216."""
@@ -162,8 +194,127 @@ def list_to_weights(spec, lst):
     return out
 
 
+def _channel_index(spec, dspec, name):
+    """(device position of every input channel, of every output channel) of block ``name``: a concat input's up-path
+    channels [0, up) stay in place, its skip channels [up, up + skip) move to [P(up), P(up) + skip)"""
+    blk = spec.by_name[name]
+    cin = np.arange(blk.cin)
+    if name in spec.cat_split:
+        up = spec.cat_split[name]
+        cin = np.concatenate([cin[:up], dspec.cat_split[name] + np.arange(blk.cin - up)])
+    return cin, np.arange(blk.cout)
+
+
+def _index(spec, dspec, key):
+    """index of the real entries of Keras array ``key`` inside its device array"""
+    name, p = key.split('/')
+    cin, cout = _channel_index(spec, dspec, name)
+    if p != 'kernel':
+        return cout
+    if spec.by_name[name].kind == 'up':      # (2, 2, Cout, Cin)
+        return slice(None), slice(None), cout[:, None], cin[None, :]
+    return slice(None), slice(None), cin[:, None], cout[None, :]
+
+
+def pack(spec, dspec, w):
+    """Keras-shaped arrays of ``spec`` (any subset of its weight keys) -> arrays of the device spec ``dspec``.  Padded
+    entries are 0 (kernel, bias, gamma, beta, moving_mean) or 1 (moving_var): a padded channel's convolution output is
+    then exactly 0, its batch mean and variance are 0, and everything downstream of it, gradients included, stays 0."""
+    if dspec is spec:
+        return OrderedDict((k, np.asarray(a, dtype=np.float32)) for k, a in w.items())
+    shapes, out = dspec.weight_shapes(), OrderedDict()
+    for k, a in w.items():
+        d = (np.ones if k.endswith('/moving_var') else np.zeros)(shapes[k], np.float32)
+        d[_index(spec, dspec, k)] = a
+        out[k] = d
+    return out
+
+
+def unpack(spec, dspec, w):
+    """inverse of pack: device arrays -> Keras-shaped arrays of ``spec``"""
+    if dspec is spec:
+        return OrderedDict((k, np.asarray(a, dtype=np.float32)) for k, a in w.items())
+    return OrderedDict((k, np.ascontiguousarray(np.asarray(a, dtype=np.float32)[_index(spec, dspec, k)]))
+                       for k, a in w.items())
+
+
+def _align4(n):
+    return (n + 3) // 4 * 4
+
+
+def flat_layout(spec):
+    """The engine's flat parameter buffers: (OrderedDict key -> (trainable?, offset, shape), trainable floats,
+    non-trainable floats).  Trainable arrays (kernel, bias, gamma, beta) share one buffer, the moving statistics
+    another; every array starts at a multiple of 4 floats."""
+    slots, off_t, off_n = OrderedDict(), 0, 0
+    for blk in spec.blocks:
+        for p, shp in blk.param_shapes().items():
+            n = int(np.prod(shp))
+            if p in TRAINABLE:
+                slots['%s/%s' % (blk.name, p)] = (True, off_t, shp)
+                off_t += _align4(n)
+            else:
+                slots['%s/%s' % (blk.name, p)] = (False, off_n, shp)
+                off_n += _align4(n)
+    return slots, off_t, off_n
+
+
+def _convert_flat(src, dst, flat, fn):
+    slots, n = flat_layout(src)[:2]
+    flat = np.asarray(flat, dtype=np.float32)
+    if flat.shape != (n,):
+        raise ValueError('expected a flat trainable-parameter vector of %d floats, got shape %s' % (n, flat.shape))
+    arrays = fn(OrderedDict((k, flat[off:off + int(np.prod(shp))].reshape(shp)) for k, (tr, off, shp) in slots.items() if tr))
+    slots, n = flat_layout(dst)[:2]
+    out = np.zeros(n, np.float32)
+    for k, a in arrays.items():
+        off = slots[k][1]
+        out[off:off + a.size] = a.ravel()
+    return out
+
+
+def pack_flat(spec, dspec, flat):
+    """a vector over the trainable parameters (Adam's m or v) in flat_layout(spec) -> the same in flat_layout(dspec)"""
+    return _convert_flat(spec, dspec, flat, lambda w: pack(spec, dspec, w))
+
+
+def unpack_flat(spec, dspec, flat):
+    """inverse of pack_flat"""
+    return _convert_flat(dspec, spec, flat, lambda w: unpack(spec, dspec, w))
+
+
 # ------------------------------------------------------------------ overlap-tile inference for images larger than the window
 MAX_TILE = 2048          # largest tile edge: a 2048^2 canvas is one tile; a batch holds at most 8 * MAX_TILE^2 pixels
+
+
+def inference_bytes_per_pixel(spec, elem_bytes):
+    """device bytes of the inference activation buffers per batch pixel for the device spec ``spec``: every block's
+    output, the max-pooled encoder outputs and the upsampled tensors of the 'upsampling' graph at ``elem_bytes`` per
+    value, plus the fp32 input, logit and probability"""
+    b = 12.
+    for blk in spec.blocks:
+        if blk.kind == 'head':
+            continue
+        b += blk.cout * elem_bytes / 4. ** blk.level
+        if blk.name.startswith('enc') and blk.name.endswith('b'):
+            b += blk.cout * elem_bytes / 4. ** (blk.level + 1)
+    if spec.up_mode == 'upsampling':
+        b += sum(spec.cat_split['dec%da' % l] * elem_bytes / 4. ** l for l in range(4))
+    return b
+
+
+def tile_limits(spec, elem_bytes):
+    """(batch pixels per tile group, largest tile edge) of predict_tiled for the device spec ``spec``: the activation
+    bytes of 8 transforms of a MAX_TILE^2 tile at nb_filters_base 32 (29.4 GiB peak in fp16), which every narrower
+    network keeps; a wider one gets proportionally fewer pixels and the largest multiple of 128 that still fits 8 of
+    its tiles"""
+    ref = GraphSpec(32, upsampling_or_transpose=spec.up_mode)
+    px = 8 * MAX_TILE * MAX_TILE
+    px = min(px, int(px * inference_bytes_per_pixel(ref, elem_bytes) // inference_bytes_per_pixel(spec, elem_bytes)))
+    T = MAX_TILE
+    while 8 * T * T > px and T > 512:
+        T -= 128
+    return px, T
 
 
 def receptive_reach(spec, block=16):

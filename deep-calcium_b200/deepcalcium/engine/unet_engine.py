@@ -16,14 +16,10 @@ import torch
 
 from .. import _native as nat
 from . import ops
-from .graph import (GraphSpec, BN_EPS, BN_MOMENTUM_CONV, BN_MOMENTUM_UP, TRAINABLE, MAX_TILE, he_normal_weights, plan_tiles,
-                    tile_halo)
+from .graph import (GraphSpec, BN_EPS, BN_MOMENTUM_CONV, BN_MOMENTUM_UP, flat_layout, he_normal_weights, pack, pack_flat,
+                    plan_tiles, tile_halo, tile_limits, unpack, unpack_flat)
 
 _PRECISIONS = {'bf16': torch.bfloat16, 'fp16': torch.float16, 'f16': torch.float16, 'fp32': torch.float32, 'f32': torch.float32}
-
-
-def _align4(n):
-    return (n + 3) // 4 * 4
 
 
 def _on_engine_device(fn):
@@ -47,6 +43,10 @@ class UNetEngine(object):
         # north star's 1e-2 logit tolerance where bf16 storage cannot); 'fp32': CUDA-core check mode
         self.precision = {torch.bfloat16: 'bf16', torch.float16: 'fp16', torch.float32: 'fp32'}[self.dtype]
         self.tc = self.dtype != torch.float32
+        # what the kernels run: the 16-bit precisions pad every channel width (graph.padded_width), the fp32 check mode
+        # runs the spec as it is.  Weights and optimiser state cross the engine's boundary in the layout of self.spec.
+        self.dspec = self.spec.device_spec(self.precision)
+        self.head_c = self.dspec.by_name['head'].cin
         self.dev = torch.device(device if device is not None else 'cuda:%d' % torch.cuda.current_device())
         self.use_graphs = use_graphs
         self._build_param_storage()
@@ -63,30 +63,21 @@ class UNetEngine(object):
         self.comm = None          # engine.dist.Comm for data-parallel training (None = single GPU)
         self.overlap_wgrad = True  # weight-gradient launches on a side stream (see _train_step_enqueue)
         self.rank1_head_grad = True   # the softmax head's input gradient stays factored (see _train_step_enqueue)
-        self.head_wd = torch.zeros(self.spec.nfb, dtype=torch.float32, device=self.dev)
+        self.head_wd = torch.zeros(self.head_c, dtype=torch.float32, device=self.dev)
         self.pdl = os.environ.get('DCB_PDL', '1') != '0'   # programmatic dependent launch in the inference forward
         # ... along the main chain of the training step it LOSES (2.81 -> 3.14 ms, scripts/train_time.py): the early-resident
         # CTAs of the next main-chain kernel take the SM slots in which the weight-gradient side stream overlapped
         self.pdl_train = os.environ.get('DCB_PDL_TRAIN', '0') != '0'
         self._side = None
         self.halo = tile_halo(self.spec)
-        # predict_tiled runs its tiles in groups of at most this many batch pixels (8 transforms of one MAX_TILE^2 tile)
-        self.tile_batch_pixels = 8 * MAX_TILE * MAX_TILE
+        # predict_tiled runs its tiles in groups of at most this many batch pixels, tiles of at most max_tile pixels a side
+        # (8 transforms of one 2048^2 tile up to nb_filters_base 32; the same activation bytes for wider networks)
+        self.tile_batch_pixels, self.max_tile = tile_limits(self.dspec, self.dtype.itemsize)
         self.set_weights_dict(he_normal_weights(self.spec, seed=0))
 
     # ------------------------------------------------------------------ parameter storage
     def _build_param_storage(self):
-        off_t, off_n = 0, 0
-        self._slots = OrderedDict()        # key -> (trainable?, offset, shape)
-        for blk in self.spec.blocks:
-            for p, shp in blk.param_shapes().items():
-                n = int(np.prod(shp))
-                if p in TRAINABLE:
-                    self._slots['%s/%s' % (blk.name, p)] = (True, off_t, shp)
-                    off_t += _align4(n)
-                else:
-                    self._slots['%s/%s' % (blk.name, p)] = (False, off_n, shp)
-                    off_n += _align4(n)
+        self._slots, off_t, off_n = flat_layout(self.dspec)        # key -> (trainable?, offset, device shape)
         f32 = dict(dtype=torch.float32, device=self.dev)
         self.params = torch.zeros(off_t, **f32)
         self.grads = torch.zeros(off_t, **f32)
@@ -111,7 +102,7 @@ class UNetEngine(object):
         self.inf_scale, self.inf_shift = {}, {}
         self.bn = {}
         n_dbl = 0
-        for blk in self.spec.blocks:
+        for blk in self.dspec.blocks:
             if blk.kind == 'head':
                 continue
             nk = int(np.prod(blk.kernel_shape()))
@@ -141,13 +132,13 @@ class UNetEngine(object):
             n_dbl += 4 * blk.cout
         self._off_head_sums = n_dbl
         self._off_head_dwb = n_dbl + 8
-        n_dbl += 8 + 2 * self.spec.nfb + 2
+        n_dbl += 8 + 2 * self.head_c + 2
         self.dbl = torch.zeros(n_dbl, dtype=torch.float64, device=self.dev)
         # single-launch BatchNorm kernels (dcb_bn_train_fwd / _bwd): 4 barrier words per (layer, direction), zeroed at the
         # start of every step, and one shared workspace for the fixed-point per-channel totals (zeroed once; the kernels
         # leave it zeroed)
-        self.bn_sync = torch.zeros(8 * len(self.spec.blocks), dtype=torch.int32, device=self.dev)
-        self.bn_ws = torch.zeros(ops.bn_train_workspace_bytes(max(b.cout for b in self.spec.blocks)), dtype=torch.uint8,
+        self.bn_sync = torch.zeros(8 * len(self.dspec.blocks), dtype=torch.int32, device=self.dev)
+        self.bn_ws = torch.zeros(ops.bn_train_workspace_bytes(max(b.cout for b in self.dspec.blocks)), dtype=torch.uint8,
                                  device=self.dev)
         self.peers = None         # dcb_peer_exchange description for in-kernel SyncBN (engine.dist.attach_peers)
         self.metrics = torch.zeros(8, **f32)
@@ -173,16 +164,33 @@ class UNetEngine(object):
 
     # ------------------------------------------------------------------ weights in / out (Keras layouts)
     def set_weights_dict(self, w):
-        for key, (tr, off, shp) in self._slots.items():
-            a = np.ascontiguousarray(np.asarray(w[key], dtype=np.float32))
-            if tuple(a.shape) != tuple(shp):
-                raise ValueError('weight %s: expected shape %s, got %s' % (key, shp, a.shape))
-            self.P[key].copy_(torch.from_numpy(a))
+        shapes = self.spec.weight_shapes()
+        real = OrderedDict()
+        for key, shp in shapes.items():
+            real[key] = np.asarray(w[key], dtype=np.float32)
+            if tuple(real[key].shape) != tuple(shp):
+                raise ValueError('weight %s: expected shape %s, got %s' % (key, shp, real[key].shape))
+        for key, a in pack(self.spec, self.dspec, real).items():
+            self.P[key].copy_(torch.from_numpy(np.ascontiguousarray(a)))
         self._weights_dirty = True
 
     def get_weights_dict(self):
         torch.cuda.synchronize(self.dev)
-        return OrderedDict((key, self.P[key].detach().cpu().numpy().copy()) for key in self._slots)
+        return unpack(self.spec, self.dspec, OrderedDict((key, self.P[key].detach().cpu().numpy().copy()) for key in self._slots))
+
+    def get_optimizer_state(self):
+        """Adam's m and v over the trainable parameters in flat_layout(self.spec) - the layout of an unpadded engine,
+        so the state moves between precisions - and the step state {iteration, dropout seed}."""
+        torch.cuda.synchronize(self.dev)
+        m, v = (unpack_flat(self.spec, self.dspec, t.cpu().numpy()) for t in (self.adam_m, self.adam_v))
+        return OrderedDict(adam_m=m, adam_v=v, step_state=self.step_state.cpu().numpy())
+
+    def set_optimizer_state(self, adam_m, adam_v, step_state):
+        """inverse of get_optimizer_state"""
+        self.adam_m.copy_(torch.from_numpy(pack_flat(self.spec, self.dspec, adam_m)))
+        self.adam_v.copy_(torch.from_numpy(pack_flat(self.spec, self.dspec, adam_v)))
+        self.step_state.copy_(torch.from_numpy(np.asarray(step_state, dtype=np.int64)))
+        self.iteration = int(step_state[0])
 
     def reset_optimizer(self):
         self.adam_m.zero_(); self.adam_v.zero_()
@@ -194,7 +202,7 @@ class UNetEngine(object):
         tab = self._prep_tables.get(for_training)
         if tab is None:
             rows = []
-            for blk in self.spec.blocks:
+            for blk in self.dspec.blocks:
                 if blk.kind == 'head':
                     continue
                 n = blk.name
@@ -221,7 +229,7 @@ class UNetEngine(object):
             ops.prep_weights_batch(tab, count, self.dtype)
         if for_training:
             return
-        for blk in self.spec.blocks:
+        for blk in self.dspec.blocks:
             if blk.kind == 'head':
                 continue
             n = blk.name
@@ -242,7 +250,7 @@ class UNetEngine(object):
         s['x'] = torch.zeros(NB, H, W, dtype=torch.float32, device=self.dev)
         if self.dtype == torch.float32:
             s['act']['x'] = s['x'].view(NB, H, W, 1)
-        for blk in self.spec.blocks:
+        for blk in self.dspec.blocks:
             if blk.kind == 'head':
                 continue
             h, w = H >> blk.level, W >> blk.level
@@ -257,12 +265,12 @@ class UNetEngine(object):
                         s['dx'][blk.name] = torch.empty(NB, h // 2, w // 2, blk.cin, dtype=torch.float32, device=self.dev)
         for un, prev in self._ups.items():
             l = int(un[2:])
-            c = self.spec.by_name[prev].cout
+            c = self.dspec.by_name[prev].cout
             s['act'][un] = torch.empty(NB, H >> l, W >> l, c, **T)
             if training:
                 s['dx'][un] = torch.empty(NB, H >> (l + 1), W >> (l + 1), c, dtype=torch.float32, device=self.dev)
         for l in range(4):
-            c = self.spec.nfb << l
+            c = self.dspec.by_name['enc%db' % l].cout
             s['act']['pool%d' % l] = torch.empty(NB, H >> (l + 1), W >> (l + 1), c, **T)
             if training:
                 s['dx']['skip%d' % l] = torch.empty(NB, H >> l, W >> l, c, dtype=torch.float32, device=self.dev)
@@ -270,10 +278,10 @@ class UNetEngine(object):
         s['prob'] = torch.empty(NB, H, W, dtype=torch.float32, device=self.dev)
         if training:
             s['y'] = torch.zeros(NB, H, W, dtype=torch.uint8, device=self.dev)
-            s['dhead'] = torch.empty(NB, H, W, self.spec.nfb, dtype=torch.float32, device=self.dev)
+            s['dhead'] = torch.empty(NB, H, W, self.head_c, dtype=torch.float32, device=self.dev)
             s['gpix'] = torch.empty(NB, H, W, dtype=torch.float32, device=self.dev)     # rank-1 head gradient: per-pixel factor
             need = 0
-            for blk in self.spec.blocks:
+            for blk in self.dspec.blocks:
                 h, w = H >> blk.level, W >> blk.level
                 if blk.kind == 'conv':
                     if blk.cin == 1 and self.tc:
@@ -301,7 +309,7 @@ class UNetEngine(object):
 
     def _forward_inference_enqueue(self, s, prob_out):
         act = s['act']
-        for blk in self.spec.blocks:
+        for blk in self.dspec.blocks:
             n = blk.name
             if blk.kind == 'head':
                 continue                                  # fused into dec0b below
@@ -434,7 +442,7 @@ class UNetEngine(object):
         it.  Tiles go through the 8-transform batch in groups of at most tile_batch_pixels batch pixels; one CUDA graph
         holds every group.  Returns (mask uint8 [hs,ws], act float64 [hs,ws]) as device tensors (static buffers)."""
         hs, ws = summ_dev.shape
-        plan = plan_tiles((hs, ws), self.halo, tile)
+        plan = plan_tiles((hs, ws), self.halo, tile, self.max_tile)
         T, n_aug = plan.tile, (8 if augmentation else 1)
         per_group = min(plan.n_tiles, max(1, self.tile_batch_pixels // (n_aug * T * T)))
         s = self._session(per_group * n_aug, T, T, False)
@@ -478,7 +486,7 @@ class UNetEngine(object):
             self.comm.allreduce_sum(t)
 
     def _train_step_enqueue(self, s, loss_id, lr, dropout, beta1, beta2, eps):
-        spec, act, raw, dxb = self.spec, s['act'], s['raw'], s['dx']
+        spec, act, raw, dxb = self.dspec, s['act'], s['raw'], s['dx']
         world = self.comm.world if self.comm is not None else 1
         # ranks draw different dropout masks for their own crops
         seed_base = (self.comm.rank if self.comm is not None else 0) * 0x9E3779B1
@@ -576,7 +584,8 @@ class UNetEngine(object):
                 ops.maxpool2x2(act[n], pooled)
         # ---------------- head + loss + its gradient
         hs = self.dbl[self._off_head_sums:self._off_head_sums + 8]
-        hd = self.dbl[self._off_head_dwb:self._off_head_dwb + 2 * spec.nfb + 2]
+        hc = self.head_c
+        hd = self.dbl[self._off_head_dwb:self._off_head_dwb + 2 * hc + 2]
         ops.head_loss_fwd(act['dec0b'], self.P['head/kernel'], self.P['head/bias'], s['y'], s['prob'], hs)
         if self.peers is not None:                      # loss / metric sums of the global batch: one-shot exchange over NVLink
             ops.peer_allreduce_f64(hs, self.peers, self.peers['n_slots'] - 1)
@@ -584,12 +593,12 @@ class UNetEngine(object):
             self._allreduce(hs)
         # head kernel [1,1,C,2] and bias [2] are adjacent in the flat gradient buffer
         off_k = self._slots['head/kernel'][1]
-        dw_out = self.grads[off_k:off_k + 2 * spec.nfb + 2]
-        assert self._slots['head/bias'][1] == off_k + 2 * spec.nfb
+        dw_out = self.grads[off_k:off_k + 2 * hc + 2]
+        assert self._slots['head/bias'][1] == off_k + 2 * hc
         # dL/d(dec0b) = gpix[pixel] * wd[channel] is never materialised when the single-launch BatchNorm backward follows: the
         # head kernel writes the two factors, dec0b's BatchNorm backward rebuilds the product while it reads (134 MB less to
         # write and 2 x 67 MB less to read for a 32 x 128^2 batch)
-        rank1 = fused_bn and self.rank1_head_grad and spec.nfb == 32
+        rank1 = fused_bn and self.rank1_head_grad and hc == 32
         if rank1:
             ops.head_loss_bwd_rank1(act['dec0b'], self.P['head/kernel'], s['y'], s['prob'], hs, loss_id, s['gpix'], self.head_wd,
                                     hd, dw_out, self.metrics, M_total=s['prob'].numel() * world)
@@ -613,7 +622,7 @@ class UNetEngine(object):
             with torch.cuda.stream(side):
                 fn(*args)
 
-        grad_of = {'dec0b': ((s['gpix'], self.head_wd) if rank1 else s['dhead'], spec.nfb, 0)}
+        grad_of = {'dec0b': ((s['gpix'], self.head_wd) if rank1 else s['dhead'], hc, 0)}
         skip_grad = {}
         for blk in reversed(spec.blocks):
             n = blk.name

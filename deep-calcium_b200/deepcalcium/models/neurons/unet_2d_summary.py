@@ -17,7 +17,7 @@ from time import time
 
 import numpy as np
 
-from ...engine.graph import GraphSpec, weights_to_list, list_to_weights, he_normal_weights
+from ...engine.graph import GraphSpec, MAX_NFB_16BIT, flat_layout, weights_to_list, list_to_weights, he_normal_weights
 from ...utils.runtime import funcname
 from ...utils import neurons as _un
 from ...utils.neurons import (F1, prec, reca, dice, dicesq, dice_loss, dicesq_loss, posyt, posyp,
@@ -48,7 +48,7 @@ class UNetModel(object):
         assert len(window_shape) == 2
         self.window_shape = tuple(int(v) for v in window_shape)
         self.spec = spec
-        precision = precision or 'bf16'          # trainable default; inference-only loads use 'fp16' (see load_model_...)
+        precision = precision or _default_precision(spec, True)   # inference-only loads use 'fp16' (see load_model_...)
         self.engine = UNetEngine(spec, precision=precision)
         self.engine.set_weights_dict(he_normal_weights(spec, seed))
         self.optimizer = Adam(0.002)
@@ -101,13 +101,11 @@ class UNetModel(object):
     # ---- persistence.  *.hdf5 / *.h5: the Keras-2.0.6 model layout the reference writes (utils/keras_hdf5.py: readable by
     # Keras' load_weights and by this package); anything else: an .npz container with the same arrays
     def save(self, filepath, include_optimizer=True):
-        import torch
         e = self.engine
         w = e.get_weights_dict()
         extra = {}
-        if include_optimizer:
-            torch.cuda.synchronize()
-            extra = dict(adam_m=e.adam_m.cpu().numpy(), adam_v=e.adam_v.cpu().numpy(), step_state=e.step_state.cpu().numpy())
+        if include_optimizer:         # the unpadded layout of every precision: a checkpoint loads into any of them
+            extra = dict(e.get_optimizer_state())
         if filepath.endswith(('.hdf5', '.h5')):
             from ...utils.keras_hdf5 import write_keras_model
             write_keras_model(filepath, self.spec, w, self.window_shape, optimizer=self.optimizer.get_config(), loss=self.loss,
@@ -135,16 +133,15 @@ class UNetModel(object):
 
 def _default_precision(spec, trainable):
     # predict() loads with trainable=False: inference only -> fp16 activations (same tensor-core rate as bf16, 8x smaller
-    # logit error: meets the 1e-2 tolerance); a model that will be trained is bf16.  Widths that are not multiples of 32
-    # have no tensor-core path: fp32 check mode.
-    return 'fp32' if spec.nfb % 32 else ('bf16' if trainable else 'fp16')
+    # logit error: meets the 1e-2 tolerance); a model that will be trained is bf16.  The 16-bit modes run every
+    # nb_filters_base up to 64 (narrower ones on zero-padded channels); wider networks run in the fp32 check mode.
+    return 'fp32' if spec.nfb > MAX_NFB_16BIT else ('bf16' if trainable else 'fp16')
 
 
 def load_model_with_new_input_shape(model_path, input_shape, compile=True, precision=None, trainable=True, **kwargs):
     """Counterpart of deepcalcium/utils/keras_helpers.py:24-68: the graph is fully convolutional, so the same weights
     simply run at another window size (no file rewriting).  Reads Keras-2.x HDF5 model files (the reference's
     checkpoints, the released unet2ds_model.hdf5) and this package's .npz containers."""
-    import torch
     from ...utils.keras_hdf5 import is_hdf5, read_keras_weights, read_extra
     if is_hdf5(model_path):
         spec, w, info = read_keras_weights(model_path)
@@ -159,11 +156,8 @@ def load_model_with_new_input_shape(model_path, input_shape, compile=True, preci
             model.loss = tc['loss']
         if compile:
             ex = read_extra(model_path, ('adam_m', 'adam_v', 'step_state'))
-            if len(ex) == 3 and ex['adam_m'].shape == tuple(model.engine.adam_m.shape):
-                model.engine.adam_m.copy_(torch.from_numpy(ex['adam_m']))
-                model.engine.adam_v.copy_(torch.from_numpy(ex['adam_v']))
-                model.engine.step_state.copy_(torch.from_numpy(ex['step_state']))
-                model.engine.iteration = int(ex['step_state'][0])
+            if len(ex) == 3 and ex['adam_m'].shape == (flat_layout(spec)[1],):
+                model.engine.set_optimizer_state(ex['adam_m'], ex['adam_v'], ex['step_state'])
         return model
     with np.load(model_path, allow_pickle=False) as z:
         cfg = json.loads(str(z['config']))
@@ -175,9 +169,7 @@ def load_model_with_new_input_shape(model_path, input_shape, compile=True, preci
         model.optimizer = Adam(**cfg['optimizer'])
         model.loss = cfg['loss']
         if compile and 'adam_m' in z.files:
-            model.engine.adam_m.copy_(torch.from_numpy(z['adam_m']))
-            model.engine.adam_v.copy_(torch.from_numpy(z['adam_v']))
-            model.engine.step_state.copy_(torch.from_numpy(z['step_state']))
+            model.engine.set_optimizer_state(z['adam_m'], z['adam_v'], z['step_state'])
             model.engine.iteration = int(cfg['iteration'])
     return model
 
@@ -185,7 +177,8 @@ def load_model_with_new_input_shape(model_path, input_shape, compile=True, preci
 def unet(window_shape=(128, 128), nb_filters_base=32, conv_kernel_init='he_normal',
          prop_dropout_base=0.25, upsampling_or_transpose='transpose', precision=None, seed=None):
     """Same arguments as the reference's unet() (unet_2d_summary.py:123-124).  ``precision`` selects 'bf16' (tcgen05
-    kernels, default: trainable), 'fp16' (same kernels with fp16 storage, inference only) or 'fp32' (CUDA-core check mode)."""
+    kernels, default: trainable), 'fp16' (same kernels with fp16 storage, inference only) or 'fp32' (CUDA-core check mode).
+    The 16-bit modes take nb_filters_base up to 64 (ValueError above that); wider networks default to 'fp32'."""
     assert len(window_shape) == 2 and window_shape[0] == window_shape[1]
     if conv_kernel_init != 'he_normal':
         raise NotImplementedError("only conv_kernel_init='he_normal' (the reference default) is built")
