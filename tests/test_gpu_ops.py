@@ -1,6 +1,7 @@
 """Per-kernel parity on the GPU through the C ABI (deepcalcium.engine.ops) against float64 CPU
 references built from the oracle's layer arithmetic (torch CPU + autograd).
-fp32 = CUDA-core check kernels (tolerance 1e-4 class), bf16 = tcgen05 kernels (bf16 tolerance)."""
+fp32 = CUDA-core check kernels (tolerance 1e-4 class); bf16 / fp16 = tcgen05 kernels, whose contractions are held to the
+float64 rounding bound of tests/rounding_bound.py."""
 import os
 
 import numpy as np
@@ -9,11 +10,12 @@ import torch
 import torch.nn.functional as F
 
 import oracle
+import rounding_bound as rb
 from oracle import losses as ol
 
 pytestmark = pytest.mark.gpu
 
-DT = {'fp32': torch.float32, 'bf16': torch.bfloat16}
+DT = {'fp32': torch.float32, 'bf16': torch.bfloat16, 'fp16': torch.float16}
 
 
 def dev(a, dtype=torch.float32):
@@ -27,11 +29,27 @@ def q(a, precision):
 
 
 def tol(precision, scale=1.0):
-    return dict(fp32=2e-4, bf16=3e-2)[precision] * scale
+    return dict(fp32=2e-4, bf16=3e-2, fp16=3e-2)[precision] * scale
 
 
 def nhwc_to_nchw(a):
     return torch.as_tensor(a).permute(0, 3, 1, 2).contiguous()
+
+
+def assert_bound(got_nchw, A, B, scale, shift, precision, what, c_acc=rb.C_ACC_TC, relu=True):
+    """16-bit forward output (NCHW, stored dtype) within its float64 rounding bound (tests/rounding_bound.py)"""
+    s = None if scale is None else torch.as_tensor(np.asarray(scale, np.float64))[None, :, None, None]
+    t = None if shift is None else torch.as_tensor(np.asarray(shift, np.float64))[None, :, None, None]
+    r = rb.check(got_nchw, A.detach(), B.detach(), s, t, c_acc=c_acc, relu=relu, fmt=precision)
+    rb.assert_ok(r, what)
+    return r
+
+
+def assert_acc(got, A, B, c_acc, what):
+    """fp32 output of a 16-bit contraction (dgrad / wgrad): |y - A| <= c_acc * 2^-24 * B"""
+    r = rb.acc_ratio(got, A.detach(), B.detach())
+    assert r <= c_acc, '%s: |y - A| = %.3g x 2^-24 B, above c_acc %g' % (what, r, c_acc)
+    return r
 
 
 # Dispatch variants of the bf16 contraction kernels, pinned per call with dcb_set_policy (deepcalcium._native.policy):
@@ -88,10 +106,25 @@ CONV_CASES = [
     # enough 256-pixel tiles for the swapped (weights-as-A) orientation of the generic kernel
     (8, 64, 64, 64, 0, 128),
     (5, 48, 80, 64, 64, 64),
+    # the padded networks (nb_filters_base 48 / 64): more than 512 output channels (slices of 512 through the generic
+    # kernel, with offsets into weights, scale, shift and output), concat inputs of 1536 and 768 channels
+    (2, 4, 4, 512, 0, 768),
+    (1, 4, 6, 512, 0, 1024),
+    (2, 2, 2, 1024, 0, 1024),
+    (1, 8, 8, 1024, 512, 512),
+    (2, 8, 8, 512, 256, 256),
+    # tiled inference: level widths of a 640 and a 192 tile at batch 8 (no W % 128 strip rows below 640)
+    (8, 4, 640, 32, 0, 32),
+    (8, 4, 320, 64, 0, 64),
+    (8, 4, 160, 128, 128, 128),
+    (8, 4, 80, 256, 0, 256),
+    (8, 4, 192, 64, 0, 64),
+    (8, 4, 96, 128, 0, 128),
+    (3, 6, 640, 64, 64, 64),          # odd N
 ]
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 @pytest.mark.parametrize('case', CONV_CASES)
 def test_conv3x3_fwd_dgrad_wgrad(cuda, precision, case):
     from deepcalcium.engine import ops
@@ -108,6 +141,10 @@ def test_conv3x3_fwd_dgrad_wgrad(cuda, precision, case):
     conv = F.conv2d(xt, wt.permute(3, 2, 0, 1), padding=1)
     ref = torch.relu(conv * torch.tensor(scale, dtype=torch.float64)[None, :, None, None]
                      + torch.tensor(shift, dtype=torch.float64)[None, :, None, None])
+    # the same contraction on absolute values: B of the rounding bound, forward / dgrad / wgrad
+    xa = nhwc_to_nchw(np.abs(x)).requires_grad_(True)
+    wa = torch.tensor(np.abs(w), requires_grad=True)
+    conv_abs = F.conv2d(xa, wa.permute(3, 2, 0, 1), padding=1)
     from deepcalcium import _native as nat
     x0 = dev(x[..., :C0], dt)
     x1 = dev(x[..., C0:], dt) if C1 else None
@@ -117,33 +154,51 @@ def test_conv3x3_fwd_dgrad_wgrad(cuda, precision, case):
     ops.prep_conv3x3_weights(wm, wf, wd, dt)
     dy = q(rng.standard_normal((N, H, W, Cout)), precision)
     conv.backward(nhwc_to_nchw(dy))
+    conv_abs.backward(nhwc_to_nchw(np.abs(dy)))
     dyd = dev(dy, dt)
     seen = {}
-    for vname, pol in (FWD_VARIANTS if precision == 'bf16' else FWD_VARIANTS[:1]):
+    tc = precision != 'fp32'
+    for vname, pol in (FWD_VARIANTS if tc else FWD_VARIANTS[:1]):
         with nat.policy(**pol):
             # forward (+ concat + epilogue)
             out = torch.empty(N, H, W, Cout, dtype=dt, device='cuda')
             ops.conv3x3_fwd(x0, x1, wf, out, dev(scale), dev(shift), True)
             kf = nat.last_kernel()
-            got = out.float().cpu().permute(0, 3, 1, 2).double()
-            assert torch.max(torch.abs(got - ref)).item() < tol(precision, 1 + ref.abs().max().item()), (vname, kf)
-            # plain conv (no epilogue): dgrad against autograd; gradients are fp32 in both modes
+            if tc:
+                got = out.cpu().permute(0, 3, 1, 2)
+                r = assert_bound(got, conv, conv_abs, scale, shift, precision, (case, precision, vname, kf), c_acc=rb.c_acc_tc(9 * Cin))
+            else:
+                got = out.float().cpu().permute(0, 3, 1, 2).double()
+                assert torch.max(torch.abs(got - ref)).item() < tol(precision, 1 + ref.abs().max().item()), (vname, kf)
+            # plain conv (no epilogue): dgrad against autograd; gradients are fp32 in every mode
             dx = torch.empty(N, H, W, Cin, dtype=torch.float32, device='cuda')
             ops.conv3x3_dgrad(dyd, wd, dx)
             kd = nat.last_kernel()
             gx = dx.float().cpu().permute(0, 3, 1, 2).double()
-            assert torch.max(torch.abs(gx - xt.grad)).item() < tol(precision, 1 + xt.grad.abs().max().item()), (vname, kd)
-            seen[vname] = (kf, kd)
-    if precision == 'bf16':
+            if tc:
+                ra = assert_acc(gx, xt.grad, xa.grad, rb.c_acc_tc(9 * Cout), (case, precision, vname, kd))
+                seen[vname] = (kf, kd, 'exact %.4f / %.4f sharp %.4f dgrad c %.2f' % (r['exact'], r['exact_nz'], r['sharp'], ra))
+            else:
+                assert torch.max(torch.abs(gx - xt.grad)).item() < tol(precision, 1 + xt.grad.abs().max().item()), (vname, kd)
+    if tc:
         assert seen['generic'][0] == 'generic' and seen['generic_swap'][0] in ('generic', 'generic_swap')
-        print('conv %s kernels: %s' % (case, seen))
-    for vname, pol in (WGRAD_VARIANTS if precision == 'bf16' else WGRAD_VARIANTS[:1]):
+        print('conv %s %s kernels: %s' % (case, precision, seen))
+    if precision == 'fp16':           # fp16 is inference only: the library rejects fp16 gradients
+        dW = torch.empty(3, 3, Cin, Cout, dtype=torch.float32, device='cuda')
+        ws = torch.empty(max(16, ops.conv3x3_wgrad_workspace_bytes(torch.bfloat16, N, H, W, Cin, Cout)), dtype=torch.uint8, device='cuda')
+        with pytest.raises(nat.DcbError):
+            ops.conv3x3_wgrad(x0, x1, dyd, dW, ws)
+        return
+    for vname, pol in (WGRAD_VARIANTS if tc else WGRAD_VARIANTS[:1]):
         with nat.policy(**pol):
             dW = torch.empty(3, 3, Cin, Cout, dtype=torch.float32, device='cuda')
             ws = torch.empty(max(16, ops.conv3x3_wgrad_workspace_bytes(dt, N, H, W, Cin, Cout)), dtype=torch.uint8, device='cuda')
             ops.conv3x3_wgrad(x0, x1, dyd, dW, ws)
             gw = dW.cpu().double()
-            assert torch.max(torch.abs(gw - wt.grad)).item() < tol(precision, 1 + wt.grad.abs().max().item()), (vname, nat.last_kernel())
+            if tc:
+                assert_acc(gw, wt.grad, wa.grad, rb.C_ACC_WGRAD, (case, vname, nat.last_kernel()))
+            else:
+                assert torch.max(torch.abs(gw - wt.grad)).item() < tol(precision, 1 + wt.grad.abs().max().item()), (vname, nat.last_kernel())
 
 
 def test_policy_roundtrip_and_kernel_names(cuda):
@@ -176,9 +231,11 @@ def test_policy_roundtrip_and_kernel_names(cuda):
     assert run(2, 32, 32, 64, 64) in ('generic', 'generic_swap')          # too few work items for the flat kernel
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 @pytest.mark.parametrize('case', [(1, 8, 8, 64, 32), (2, 4, 4, 512, 256), (1, 16, 16, 128, 64), (3, 2, 2, 256, 128),
-                                  (4, 64, 64, 128, 64), (8, 64, 64, 64, 32)])
+                                  (4, 64, 64, 128, 64), (8, 64, 64, 64, 32),
+                                  (2, 4, 4, 1024, 512),          # up3 of nb_filters_base 64
+                                  (8, 10, 10, 256, 128)])        # a 640 tile's 80^2 level
 def test_convT2x2_fwd_dgrad_wgrad(cuda, precision, case):
     from deepcalcium.engine import ops
     N, h, w_, Cin, Cout = case
@@ -190,6 +247,10 @@ def test_convT2x2_fwd_dgrad_wgrad(cuda, precision, case):
     xt = nhwc_to_nchw(x).requires_grad_(True)
     kt = torch.tensor(k, requires_grad=True)
     ref = F.conv_transpose2d(xt, kt.permute(3, 2, 0, 1), torch.tensor(bias, dtype=torch.float64), stride=2)
+    xa = nhwc_to_nchw(np.abs(x)).requires_grad_(True)
+    ka = torch.tensor(np.abs(k), requires_grad=True)
+    ref_abs = F.conv_transpose2d(xa, ka.permute(3, 2, 0, 1), stride=2)
+    tc = precision != 'fp32'
     wf = torch.empty(4 * Cin * Cout, dtype=dt, device='cuda')
     wd = torch.empty(4 * Cin * Cout, dtype=dt, device='cuda')
     ops.prep_convT2x2_weights(dev(k), wf, wd, dt)
@@ -198,22 +259,39 @@ def test_convT2x2_fwd_dgrad_wgrad(cuda, precision, case):
         with nat.policy(tma_store=tma_store):
             out = torch.zeros(N, 2 * h, 2 * w_, Cout, dtype=dt, device='cuda')
             ops.convT2x2_fwd(dev(x, dt), wf, out, None, dev(bias), False)
-            got = out.float().cpu().permute(0, 3, 1, 2).double()
-            assert torch.max(torch.abs(got - ref)).item() < tol(precision, 1 + ref.abs().max().item()), tma_store
+            if tc:        # bias as the epilogue shift with scale 1: y = A + bias, no ReLU
+                assert_bound(out.cpu().permute(0, 3, 1, 2), ref - torch.tensor(bias, dtype=torch.float64)[None, :, None, None],
+                             ref_abs, np.ones(Cout), bias, precision, (case, precision, tma_store), c_acc=rb.c_acc_tc(Cin), relu=False)
+            else:
+                got = out.float().cpu().permute(0, 3, 1, 2).double()
+                assert torch.max(torch.abs(got - ref)).item() < tol(precision, 1 + ref.abs().max().item()), tma_store
     dy = q(rng.standard_normal((N, 2 * h, 2 * w_, Cout)), precision)
     ref.backward(nhwc_to_nchw(dy))
+    ref_abs.backward(nhwc_to_nchw(np.abs(dy)))
     dx = torch.empty(N, h, w_, Cin, dtype=torch.float32, device='cuda')
     ops.convT2x2_dgrad(dev(dy, dt), wd, dx)
-    assert torch.max(torch.abs(dx.float().cpu().permute(0, 3, 1, 2).double() - xt.grad)).item() < \
-        tol(precision, 1 + xt.grad.abs().max().item())
+    if tc:
+        assert_acc(dx.cpu().permute(0, 3, 1, 2).double(), xt.grad, xa.grad, rb.c_acc_tc(4 * Cout), (case, precision, 'dgrad'))
+    else:
+        assert torch.max(torch.abs(dx.float().cpu().permute(0, 3, 1, 2).double() - xt.grad)).item() < \
+            tol(precision, 1 + xt.grad.abs().max().item())
     dW = torch.empty(2, 2, Cout, Cin, dtype=torch.float32, device='cuda')
-    ws = torch.empty(max(16, ops.convT2x2_wgrad_workspace_bytes(dt, N, h, w_, Cin, Cout)), dtype=torch.uint8, device='cuda')
+    ws = torch.empty(max(16, ops.convT2x2_wgrad_workspace_bytes(torch.bfloat16 if tc else dt, N, h, w_, Cin, Cout)),
+                     dtype=torch.uint8, device='cuda')
+    if precision == 'fp16':           # inference only: no fp16 gradients
+        with pytest.raises(nat.DcbError):
+            ops.convT2x2_wgrad(dev(x, dt), dev(dy, dt), dW, ws)
+        return
     ops.convT2x2_wgrad(dev(x, dt), dev(dy, dt), dW, ws)
-    assert torch.max(torch.abs(dW.cpu().double() - kt.grad)).item() < tol(precision, 1 + kt.grad.abs().max().item())
+    if tc:
+        assert_acc(dW.cpu().double(), kt.grad, ka.grad, rb.C_ACC_WGRAD, (case, precision, 'wgrad'))
+    else:
+        assert torch.max(torch.abs(dW.cpu().double() - kt.grad)).item() < tol(precision, 1 + kt.grad.abs().max().item())
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 @pytest.mark.parametrize('shape', [(2, 16, 128, 32, 32), (1, 6, 256, 64, 64), (1, 8, 24, 32, 32), (2, 40, 256, 32, 32), (1, 44, 512, 64, 32),
+                                   (2, 8, 512, 64, 64), (8, 4, 640, 64, 64),        # full-resolution 64 -> 64 (nfb 64)
                                    # pooled epilogue of the generic kernel: pixels-as-M tiles (several tile shapes, an N tile
                                    # narrower than Cout), weights-as-M tiles of 128x2 and 64x4 pixels
                                    (2, 32, 32, 128, 128), (3, 8, 8, 256, 256), (8, 64, 64, 128, 256),
@@ -245,10 +323,56 @@ def test_conv3x3_fused_pool_and_head_equal_the_unfused_composition(cuda, precisi
             _check_fused(ops, nat, precision, shape, x, wf, scale, shift, hk, hb, y, pool, logit, prob)
 
 
+OVERFLOW_VARIANTS = [('plain', {}, False), ('generic', dict(strip=0, flat=0, swap_min_cout=0), False),
+                     ('generic_swap', dict(strip=0, flat=0), False),
+                     ('generic_tma_store', dict(strip=0, flat=0, swap_min_cout=0, tma_store=2), False),
+                     ('strip_pool', {}, True), ('generic_pool', dict(strip=0, flat=0), True)]
+
+
+@pytest.mark.parametrize('variant', OVERFLOW_VARIANTS, ids=[v[0] for v in OVERFLOW_VARIANTS])
+def test_fp16_outputs_past_65504_are_stored_as_inf(cuda, variant):
+    """fp16 range: a scale that pushes outputs past the largest fp16 value.  Every stored value is RN16 of the result -
+    +inf from 65520 up, 0 for the negative ones after ReLU - in the plain, TMA-store and pooled epilogues, and no other bit
+    pattern (NaN, 65504, bf16 bits) appears.  This characterises the kernels; nothing clamps on purpose."""
+    from deepcalcium import _native as nat
+    from deepcalcium.engine import ops
+    name, pol, pooled = variant
+    N, H, W, Cin, Cout = 2, 8, 128, 64, 64
+    dt = torch.float16
+    rng = np.random.default_rng(65504)
+    x = q(rng.standard_normal((N, H, W, Cin)), 'fp16')
+    w = q(rng.standard_normal((3, 3, Cin, Cout)) * np.sqrt(2. / (9 * Cin)), 'fp16')
+    scale = np.where(np.arange(Cout) % 2 == 0, 6e4, 0.7).astype(np.float32)      # even channels overflow where A > ~1.1
+    shift = rng.standard_normal(Cout).astype(np.float32)
+    xt, wt = nhwc_to_nchw(x), torch.tensor(w).permute(3, 2, 0, 1)
+    A = F.conv2d(xt, wt, padding=1)
+    B = F.conv2d(xt.abs(), wt.abs(), padding=1)
+    wf = torch.empty(9 * Cin * Cout, dtype=dt, device='cuda')
+    ops.prep_conv3x3_weights(dev(w), wf, None, dt)
+    out = torch.empty(N, H, W, Cout, dtype=dt, device='cuda')
+    pool = torch.empty(N, H // 2, W // 2, Cout, dtype=dt, device='cuda')
+    with nat.policy(**pol):
+        if pooled:
+            ops.conv3x3_fwd_fused(dev(x, dt), None, wf, out, dev(scale), dev(shift), True, pool_out=pool)
+        else:
+            ops.conv3x3_fwd(dev(x, dt), None, wf, out, dev(scale), dev(shift), True)
+        kern = nat.last_kernel()
+    got = out.cpu().permute(0, 3, 1, 2)
+    assert not bool(torch.isnan(got).any()) and not bool((got == -np.inf).any()), kern
+    n_inf = int(torch.isinf(got).sum())
+    assert n_inf > 1000, (kern, n_inf)
+    # the bound admits exactly +inf where RN16(v - d) is +inf and only finite values where RN16(v + d) is finite
+    r = assert_bound(got, A, B, scale, shift, 'fp16', (name, kern), c_acc=rb.c_acc_tc(9 * Cin))
+    if pooled:                        # the pooled copy: bit for bit the 2x2 max of what was stored (either zero of a +-0 tie)
+        want = F.max_pool2d(out.permute(0, 3, 1, 2).float(), 2).permute(0, 2, 3, 1).to(dt).contiguous()
+        assert bool(((pool.view(torch.int16) == want.view(torch.int16)) | ((pool == 0) & (want == 0))).all()), kern
+    print('fp16 overflow %s -> %s: %d inf, exact %.5f' % (name, kern, n_inf, r['exact']))
+
+
 def _check_fused(ops, nat, precision, shape, x, wf, scale, shift, hk, hb, y, pool, logit, prob):
     y2 = torch.empty_like(y); pool2 = torch.empty_like(pool)
     ops.conv3x3_fwd_fused(x, None, wf, y2, scale, shift, True, pool_out=pool2)
-    print('fused pool %s %s -> %s' % (precision, shape, nat.last_kernel() if precision == 'bf16' else 'fp32 composition'))
+    print('fused pool %s %s -> %s' % (precision, shape, nat.last_kernel() if precision != 'fp32' else 'fp32 composition'))
     def same(a, b):
         if precision == 'fp32':
             return torch.equal(a, b)
@@ -264,8 +388,9 @@ def _check_fused(ops, nat, precision, shape, x, wf, scale, shift, hk, hb, y, poo
     assert torch.allclose(logit3, logit, atol=atol, rtol=1e-5) and torch.allclose(prob3, prob, atol=atol / 4)
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
-@pytest.mark.parametrize('shape', [(2, 24, 40, 32), (3, 7, 33, 32), (1, 5, 130, 32), (4, 128, 128, 32), (2, 9, 21, 16), (1, 16, 16, 64)])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
+@pytest.mark.parametrize('shape', [(2, 24, 40, 32), (3, 7, 33, 32), (1, 5, 130, 32), (4, 128, 128, 32), (2, 9, 21, 16), (1, 16, 16, 64),
+                                   (8, 8, 640, 64)])
 def test_conv3x3_first_layer_c1(cuda, precision, shape):
     """Cin = 1 layer (enc0a): CUDA-core forward; weight gradient = row-staged kernel for Cout == 32 (odd widths, one-row
     CTAs, more CTAs than rows), pixel-range kernel otherwise."""
@@ -281,7 +406,14 @@ def test_conv3x3_first_layer_c1(cuda, precision, shape):
     ref = F.conv2d(xt, wt.permute(3, 2, 0, 1), torch.tensor(b, dtype=torch.float64), padding=1)
     out = torch.empty(N, H, W, Cout, dtype=dt, device='cuda')
     ops.conv3x3_c1_fwd(dev(x), dev(w), out, None, dev(b), False)
+    if precision != 'fp32':
+        A = F.conv2d(xt, wt.detach().permute(3, 2, 0, 1), padding=1)
+        B = F.conv2d(xt.abs(), wt.detach().abs().permute(3, 2, 0, 1), padding=1)
+        assert_bound(out.cpu().permute(0, 3, 1, 2), A, B, np.ones(Cout), b, precision, (shape, precision), c_acc=rb.C_ACC_C1,
+                     relu=False)
     assert torch.max(torch.abs(out.float().cpu().permute(0, 3, 1, 2).double() - ref)).item() < tol(precision, 4)
+    if precision == 'fp16':           # inference only: the weight gradient is not built for fp16
+        return
     dy = q(rng.standard_normal((N, H, W, Cout)), precision)
     ref.backward(nhwc_to_nchw(dy))
     dW = torch.empty(3, 3, 1, Cout, dtype=torch.float32, device='cuda')
@@ -446,7 +578,7 @@ def test_dropout_is_consistent_between_forward_and_backward(cuda, precision):
     assert torch.allclose(sums[:C], 2.0 * keep.view(M, C).double().sum(0))
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 def test_maxpool_forward_and_backward_routing(cuda, precision):
     from deepcalcium.engine import ops
     dt = DT[precision]
@@ -459,6 +591,8 @@ def test_maxpool_forward_and_backward_routing(cuda, precision):
     yd = torch.empty(N, H // 2, W // 2, C, dtype=dt, device='cuda')
     ops.maxpool2x2(xd, yd)
     assert torch.equal(yd.float().cpu().permute(0, 3, 1, 2).double(), ref.detach())
+    if precision == 'fp16':           # inference only: forward
+        return
     dp = q(rng.standard_normal((N, H // 2, W // 2, C)), precision)
     skip_wide = q(rng.standard_normal((N, H, W, 2 * C)), precision)
     ref.backward(nhwc_to_nchw(dp))
@@ -469,7 +603,7 @@ def test_maxpool_forward_and_backward_routing(cuda, precision):
     assert torch.max(torch.abs(out.float().cpu().permute(0, 3, 1, 2).double() - exp)).item() < tol(precision, 4)
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 @pytest.mark.parametrize('loss', ['dice_loss', 'binary_crossentropy', 'dicesq_loss', 'weighted_binary_crossentropy'])
 def test_head_loss_metrics_and_gradient(cuda, precision, loss):
     from deepcalcium.engine import ops
@@ -489,6 +623,8 @@ def test_head_loss_metrics_and_gradient(cuda, precision, loss):
     prob = torch.empty(M, device='cuda'); logit = torch.empty(M, device='cuda')
     ops.head_fwd(xd, dev(w), dev(b), logit, prob)
     assert np.allclose(prob.cpu().numpy(), p.detach().numpy(), atol=1e-5)
+    if precision == 'fp16':           # inference only: head_fwd
+        return
     sums = torch.zeros(8, dtype=torch.float64, device='cuda'); dwb = torch.zeros(2 * C + 2, dtype=torch.float64, device='cuda')
     ops.head_loss_fwd(xd, dev(w), dev(b), dev(yt, torch.uint8), prob, sums)
     dx = torch.empty(1, 1, M, C, device='cuda'); dw = torch.empty(2 * C + 2, device='cuda'); met = torch.empty(8, device='cuda')
@@ -574,12 +710,12 @@ def test_bn_finalize_apply_equals_the_two_separate_calls(cuda, precision):
             assert torch.equal(a, b)
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
+@pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 def test_prep_weights_batch_equals_per_layer_calls(cuda, precision):
     from deepcalcium.engine import ops
     dt = DT[precision]
     rng = np.random.default_rng(4)
-    layers = [('conv', 32, 64), ('convT', 64, 32), ('conv', 1, 32), ('conv', 96, 32)]
+    layers = [('conv', 32, 64), ('convT', 64, 32), ('conv', 1, 32), ('conv', 96, 32), ('conv', 1536, 512), ('convT', 1024, 512)]
     rows, ref, got = [], [], []
     for kind, cin, cout in layers:
         if kind == 'conv':
@@ -595,7 +731,12 @@ def test_prep_weights_batch_equals_per_layer_calls(cuda, precision):
     tab = torch.tensor([r[:5] for r in rows], dtype=torch.int64, device='cuda')
     ops.prep_weights_batch(tab, len(rows), dt)
     for a, b in zip(ref, got):
-        assert torch.equal(a, b)
+        assert torch.equal(a.view(torch.int16) if dt != torch.float32 else a, b.view(torch.int16) if dt != torch.float32 else b)
+    if dt != torch.float32:           # both are round-to-nearest of the fp32 master: [Cout][9][Cin] / [4][Cout][Cin]
+        w0 = rows[0][5]
+        assert torch.equal(ref[0].view(torch.int16), w0.permute(3, 0, 1, 2).reshape(-1).to(dt).view(torch.int16))
+        w1 = rows[1][5]
+        assert torch.equal(ref[2].view(torch.int16), w1.reshape(-1).to(dt).view(torch.int16))
 
 
 STATS_CASES = [
