@@ -722,13 +722,6 @@ __device__ __forceinline__ void tta_dst(int k, int S, int i, int j, int& a, int&
     default: tta_src(k, S, i, j, a, b); break;        // the other six are involutions
   }
 }
-__device__ __forceinline__ int reflect_index(int i, int n) {   // np.pad(mode='reflect'), extended to negative i
-  if (n == 1) return 0;
-  const int period = 2 * (n - 1);
-  int r = (i < 0 ? -i : i) % period;
-  return r < n ? r : period - r;
-}
-
 // Overlap-tile TTA.  The canvas is s [hs][ws] reflect-padded at the bottom and right (unet_2d_summary.py:569-571); a plan
 // cuts it into S x S tiles with origins (oy[ty], ox[tx]) over an n_ty x n_tx grid, numbered row-major.  A group is the
 // tiles tile_first..tile_first+n_tiles-1.  oy == ox == nullptr is the one-tile plan of the 512^2 window (origin 0).

@@ -101,6 +101,15 @@ template <typename T, int VEC> __device__ __forceinline__ void loadv(const T* p,
   }
 }
 
+// np.pad(mode='reflect'), extended to negative i.  For pads longer than the axis np.pad reflects repeatedly, which is
+// this periodic map.
+__device__ __forceinline__ int reflect_index(int i, int n) {
+  if (n == 1) return 0;
+  const int period = 2 * (n - 1);
+  int r = (i < 0 ? -i : i) % period;
+  return r < n ? r : period - r;
+}
+
 // packed fp32x2 FMA (sm_100): d = a * b + c on two values at once, one issue slot
 __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
   uint64_t ua, ub, uc, ud;

@@ -286,31 +286,57 @@ def _match_regions(a, b, threshold):
     return out
 
 
+def _overlaps(a, b, match):
+    """|s_a & s_b| of every truth region and its matched prediction region (0 without a match)"""
+    out = []
+    for ra, ib in zip(a, match):
+        if ib < 0:
+            out.append(0)
+            continue
+        sa = set(map(tuple, ra.tolist()))
+        out.append(sum(1 for xy in map(tuple, b[ib].tolist()) if xy in sa))
+    return out
+
+
+def _match_stats(a, b, threshold):
+    """(match index or -1 per truth region, truth sizes, prediction sizes, overlaps) of two region lists"""
+    match = [-1 if ib is None else ib for ib in _match_regions(a, b, threshold)]
+    return match, [len(r) for r in a], [len(r) for r in b], _overlaps(a, b, match)
+
+
+def nf_scores_from_matches(na, nb, match, size_a, size_b, nhit):
+    """The float arithmetic of neurofinder.centers / shapes and the combined score, from a matching: na truth and nb
+    prediction regions, match[k] = index of the prediction region matched to truth region k or -1, size_a / size_b the
+    region pixel counts, nhit[k] the overlap of truth region k with its match.  -> (prec, reca, incl, excl, comb).
+    Every matched pair is closer than the threshold (the matching only takes such pairs), so it counts for centers.
+    Host and device scoring both end here, so their five numbers come from the same expressions."""
+    match = np.asarray(match, dtype=np.int64).reshape(-1)
+    hit = match >= 0
+    n = int(np.count_nonzero(hit))
+    with np.errstate(divide='ignore', invalid='ignore'):
+        r, p = np.float64(n) / np.float64(na), np.float64(n) / np.float64(nb)
+    if n:
+        nh = np.asarray(nhit, dtype=np.float64).reshape(-1)[hit]
+        sa = np.asarray(size_a, dtype=np.float64).reshape(-1)[hit]
+        sb = np.asarray(size_b, dtype=np.float64).reshape(-1)[match[hit]]
+        rates = np.stack([nh / sa, nh / sb], axis=1)
+        i, e = (float(v) for v in rates.mean(axis=0))
+    else:
+        i, e = 0.0, 0.0
+    with np.errstate(divide='ignore', invalid='ignore'):
+        f1 = np.float64(2.) * (r * p) / (r + p)
+    return (float(p), float(r), float(i), float(e), float(f1))
+
+
 def nf_centers(a, b, threshold=5):
     """neurofinder.centers on two region lists -> (recall, precision)."""
-    inds = _match_regions(a, b, threshold)
-    n = 0
-    for ra, ib in zip(a, inds):
-        if ib is not None and np.sqrt(((ra.mean(axis=0) - b[ib].mean(axis=0)) ** 2).sum()) < threshold:
-            n += 1
-    with np.errstate(divide='ignore', invalid='ignore'):
-        return np.float64(n) / np.float64(len(a)), np.float64(n) / np.float64(len(b))
+    p, r = nf_scores_from_matches(len(a), len(b), *_match_stats(a, b, threshold))[:2]
+    return np.float64(r), np.float64(p)
 
 
 def nf_shapes(a, b, threshold=5):
     """neurofinder.shapes on two region lists -> (inclusion, exclusion)."""
-    inds = _match_regions(a, b, threshold)
-    rates = []
-    for ra, ib in zip(a, inds):
-        if ib is None:
-            continue
-        sa = set(map(tuple, ra.tolist()))
-        nhit = float(sum(1 for xy in map(tuple, b[ib].tolist()) if xy in sa))
-        rates.append((nhit / len(ra), nhit / len(b[ib])))
-    if not rates:
-        return 0.0, 0.0
-    r = np.asarray(rates, dtype=np.float64).mean(axis=0)
-    return float(r[0]), float(r[1])
+    return nf_scores_from_matches(len(a), len(b), *_match_stats(a, b, threshold))[2:4]
 
 
 def nf_mask_metrics(m, mp):
@@ -320,11 +346,63 @@ def nf_mask_metrics(m, mp):
     if np.sum(mp.round()) == 0:
         return 0., 0., 0., 0., 0.
     a, b = _label_regions(m), _label_regions(mp)
-    r, p = nf_centers(a, b)
-    i, e = nf_shapes(a, b)
-    with np.errstate(divide='ignore', invalid='ignore'):
-        f1 = np.float64(2.) * (r * p) / (r + p)
-    return (float(p), float(r), float(i), float(e), float(f1))
+    return nf_scores_from_matches(len(a), len(b), *_match_stats(a, b, 5))
+
+
+# device scoring: one table row per image (ops.nf_score); kind 0 = uint8 nonzero, 1 / 2 = fp32 / fp64 round(p) != 0
+_SCORE_KINDS = {'torch.uint8': 0, 'torch.bool': 0, 'torch.float32': 1, 'torch.float64': 2}
+
+
+def _tensor_row(t):
+    kind = _SCORE_KINDS.get(str(t.dtype))
+    if not t.is_cuda or t.dim() != 2 or kind is None:
+        raise TypeError('nf_mask_metrics_device takes 2-D CUDA masks of dtype uint8, bool, float32 or float64, got %s %s %s'
+                        % (t.device, t.dtype, tuple(t.shape)))
+    return [t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), t.stride(1), kind, 0, 0]
+
+
+def nf_metrics_from_table(h_desc, device):
+    """Score the (truth, prediction) image pairs of an int64 table [2 n, 8] (rows as in ops.nf_score; the images must stay
+    alive until this returns) -> n tuples (prec, reca, incl, excl, comb)."""
+    import torch
+    from ..engine import ops
+    h_desc = np.ascontiguousarray(h_desc, dtype=np.int64)
+    n = h_desc.shape[0] // 2
+    if n == 0:
+        return []
+    nbytes, cap = ops.nf_score_workspace_bytes(h_desc)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    info = torch.empty(max(cap, 1), 3, dtype=torch.int32, device=device)
+    base = torch.empty(2 * n + 1, dtype=torch.int32, device=device)
+    ops.nf_score(torch.from_numpy(h_desc).to(device), h_desc, base, info, ws)
+    hbase = base.cpu().numpy().astype(np.int64)
+    hinfo = info[:int(hbase[-1])].cpu().numpy()
+    out = []
+    for i in range(n):
+        a0, a1, b1 = hbase[2 * i], hbase[2 * i + 1], hbase[2 * i + 2]
+        if b1 == a1:                     # no predicted region: nf_mask_metrics' early exit
+            out.append((0., 0., 0., 0., 0.))
+            continue
+        ta = hinfo[a0:a1]
+        out.append(nf_scores_from_matches(a1 - a0, b1 - a1, ta[:, 1], ta[:, 0], hinfo[a1:b1, 0], ta[:, 2]))
+    return out
+
+
+def nf_mask_metrics_device(pairs):
+    """nf_mask_metrics for a batch of (truth, prediction) masks that are already on the GPU: 2-D CUDA tensors with values
+    in {0, 1} (uint8, bool, float32 or float64; any strides, shapes may differ between pairs but not within one).
+    Labelling, region statistics, the centre matching and the overlaps run in one device call (ops.nf_score); only the
+    per-region integers come back.  Returns one (prec, reca, incl, excl, comb) tuple per pair, equal bit for bit to
+    nf_mask_metrics(truth.cpu(), pred.cpu()), NaN included."""
+    pairs = list(pairs)
+    if not pairs:
+        return []
+    rows = []
+    for t, p in pairs:
+        if tuple(t.shape) != tuple(p.shape):
+            raise ValueError('truth %s and prediction %s differ in shape' % (tuple(t.shape), tuple(p.shape)))
+        rows += [_tensor_row(t), _tensor_row(p)]
+    return nf_metrics_from_table(np.asarray(rows, dtype=np.int64), pairs[0][0].device)
 
 
 def nf_submit(Mp, names, json_path):

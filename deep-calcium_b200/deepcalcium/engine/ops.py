@@ -6,6 +6,7 @@ or numpy arithmetic.
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from .. import _native as nat
@@ -466,6 +467,43 @@ def tile_combine(probs, T, origins_y, origins_x, cuts_y, cuts_x, tile_first, n_t
          ptr(cuts_y if cuts_y.numel() else None), ptr(cuts_x if cuts_x.numel() else None), c_int(origins_y.numel()),
          c_int(origins_x.numel()), c_int(tile_first), c_int(n_tiles), c_f(threshold), c_int(n_aug), ptr(act), ptr(mask),
          stream_ptr())
+
+
+# ---------------------------------------------------------------- region scoring (csrc/regions.cu)
+# An image table is an int64 numpy array [n, 8] of {data pointer, H, W, row stride, column stride, kind, 0, 0} (strides in
+# elements; kind 0 uint8 nonzero, 1 fp32 / 2 fp64 round(p) != 0); the calls take it on the host and on the device.
+def _h_desc(h_desc):
+    assert h_desc.dtype == np.int64 and h_desc.ndim == 2 and h_desc.shape[1] == 8 and h_desc.flags.c_contiguous
+    return h_desc.ctypes.data_as(c_p)
+
+
+def nf_score_workspace_bytes(h_desc):
+    """-> (workspace bytes of label_regions / nf_score for this table, capacity of region_info in rows)"""
+    nbytes, cap = c_sz(0), c_ll(0)
+    call('dcb_nf_score_workspace_bytes', _h_desc(h_desc), c_int(h_desc.shape[0]), ctypes.byref(nbytes), ctypes.byref(cap))
+    return nbytes.value, cap.value
+
+
+def label_regions(desc, h_desc, labels, region_base, workspace):
+    """labels int32 [sum H*W] (scipy.ndimage.label numbering, 8-connected), region_base int32 [n + 1]"""
+    _chk(desc, torch.int64); _chk(labels, torch.int32); _chk(region_base, torch.int32); _chk(workspace, torch.uint8)
+    call('dcb_label_regions', ptr(desc), _h_desc(h_desc), c_int(h_desc.shape[0]), ptr(labels), ptr(region_base),
+         ptr(workspace), c_sz(workspace.numel()), stream_ptr())
+
+
+def nf_score(desc, h_desc, region_base, region_info, workspace):
+    """(truth, prediction) pairs as rows 2p, 2p+1 of the table -> region_base int32 [n + 1], region_info int32 [cap, 3]
+    = {pixel count, matched prediction region of the pair or -1, overlap pixels}"""
+    _chk(desc, torch.int64); _chk(region_base, torch.int32); _chk(region_info, torch.int32); _chk(workspace, torch.uint8)
+    call('dcb_nf_score', ptr(desc), _h_desc(h_desc), c_int(h_desc.shape[0] // 2), ptr(region_base), ptr(region_info),
+         ptr(workspace), c_sz(workspace.numel()), stream_ptr())
+
+
+def orient_pad(s, k, out):
+    """out [H, W] = np.pad(f_k(s), ((0, H - hf), (0, W - wf)), 'reflect'), f_k = (identity, fliplr, flipud, rot90 1/2/3)[k]"""
+    _chk(s, torch.float32); _chk(out, torch.float32)
+    call('dcb_orient_pad_f32', ptr(s), c_int(s.shape[0]), c_int(s.shape[1]), c_int(k), c_int(out.shape[0]),
+         c_int(out.shape[1]), ptr(out), stream_ptr())
 
 
 # ---------------------------------------------------------------- optimiser

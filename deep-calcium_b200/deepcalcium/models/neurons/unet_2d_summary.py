@@ -22,7 +22,7 @@ from ...utils.runtime import funcname
 from ...utils import neurons as _un
 from ...utils.neurons import (F1, prec, reca, dice, dicesq, dice_loss, dicesq_loss, posyt, posyp,
                               weighted_binary_crossentropy, binary_crossentropy)
-from ...datasets.nf import open_dataset, nf_mask_metrics
+from ...datasets.nf import open_dataset, nf_mask_metrics_device
 
 MODEL_URL_LATEST = 'https://github.com/alexklibisz/deep-calcium/releases/download/v0.0.1-weights/unet2ds_model.hdf5'
 METRIC_NAMES = ['loss', 'F1', 'prec', 'reca', 'dice', 'dicesq', 'posyt', 'posyp']   # unet_2d_summary.py:398-399
@@ -286,6 +286,7 @@ class UNet2DSummary(object):
         # (slice, zero fill, flips / rot90s) runs on the GPU and the batch never visits the host
         gen_trn = self._batch_gen(S_summ, M_summ, names, yctrn, batch_size_trn, nb_steps_trn, shape_trn, 15,
                                   device=model.engine.dev)
+        val = self._validation_data(S_summ, M_summ, model.engine.dev)
 
         for cb in keras_callbacks:               # Keras calls these before the first epoch
             if hasattr(cb, 'set_model'):
@@ -302,7 +303,7 @@ class UNet2DSummary(object):
                 xb, yb = next(gen_trn)
                 acc += np.asarray(model.train_on_batch(xb, yb))
             logs = dict(zip(METRIC_NAMES, (acc / nb_steps_trn).tolist()))
-            logs.update(self._validate(model, S_summ, M_summ, names, ycval, shape_val, epoch))
+            logs.update(self._validate(model, S_summ, M_summ, names, ycval, shape_val, epoch, val))
             logs['lr'] = model.optimizer.lr
             # ModelCheckpoint every epoch (:423-424)
             last_path = '%s/%d_model_%02d_%.3f.hdf5' % (self.cpdir, tic, epoch, logs['val_nf_f1_mean'])
@@ -331,44 +332,78 @@ class UNet2DSummary(object):
             logger.info('epoch %d: %s' % (epoch, ' '.join('%s=%.4f' % kv for kv in sorted(logs.items()))))
         return history, last_path
 
-    def _validate(self, model, S_summ, M_summ, names, y_coords, shape_val, epoch):
-        """_ValidationMetricsCB.on_epoch_end (:62-120): six orientations of every dataset at the
-        validation window, scored inside the validation rows with nf_mask_metrics (region matching of the
-        `neurofinder` package, restated in deepcalcium.datasets.nf)."""
+    # The six orientations of _ValidationMetricsCB (:62-120): f_k = identity, np.fliplr, np.flipud, np.rot90 k = 1, 2, 3.
+    # _VAL_SRC[k](H, W, a, b) = the pixel (i, j) of an H x W image that f_k puts at (a, b); _VAL_DST is its inverse.
+    _VAL_SRC = (lambda H, W, a, b: (a, b), lambda H, W, a, b: (a, W - 1 - b), lambda H, W, a, b: (H - 1 - a, b),
+                lambda H, W, a, b: (b, W - 1 - a), lambda H, W, a, b: (H - 1 - a, W - 1 - b),
+                lambda H, W, a, b: (H - 1 - b, a))
+    _VAL_DST = (lambda H, W, y, x: (y, x), lambda H, W, y, x: (y, W - 1 - x), lambda H, W, y, x: (H - 1 - y, x),
+                lambda H, W, y, x: (W - 1 - x, y), lambda H, W, y, x: (H - 1 - y, W - 1 - x),
+                lambda H, W, y, x: (x, H - 1 - y))
+
+    @classmethod
+    def _val_box(cls, shape, y0, y1, k):
+        """(a0, a1, b0, b1): the smallest and largest row and column that the validation rows [y0, y1) of an image of
+        `shape` occupy after orientation k - the reference's np.where(f(vm) == 1) box (scored as [a0:a1, b0:b1], the
+        exclusive max() end kept), taken from the corners of the band"""
+        H, W = shape
+        if not (0 <= y0 < y1 <= H) or W == 0:
+            raise ValueError('validation rows [%d, %d) are empty in a %d x %d image' % (y0, y1, H, W))
+        pts = [cls._VAL_DST[k](H, W, y, x) for y in (y0, y1 - 1) for x in (0, W - 1)]
+        return min(p[0] for p in pts), max(p[0] for p in pts), min(p[1] for p in pts), max(p[1] for p in pts)
+
+    @staticmethod
+    def _validation_data(S_summ, M_summ, dev):
+        """the summary images (fp32) and truth masks (m != 0 as uint8) on the device, uploaded once per fit"""
+        import torch
+        return [(torch.from_numpy(np.ascontiguousarray(s, dtype=np.float32)).to(dev),
+                 torch.from_numpy(np.ascontiguousarray(np.asarray(m) != 0, dtype=np.uint8)).to(dev))
+                for s, m in zip(S_summ, M_summ)]
+
+    def _validate(self, model, S_summ, M_summ, names, y_coords, shape_val, epoch, val=None):
+        """_ValidationMetricsCB.on_epoch_end (:62-120): six orientations of every dataset at the validation window, scored
+        inside the validation rows with the Neurofinder region matching (nf_mask_metrics).  Runs on the device: each
+        orientation is reflect-padded to the window by ops.orient_pad and predicted at batch 1 as the reference does
+        (images larger than the window: the identity transform over overlapping tiles); the truth masks are strided views
+        of the uploaded masks, and all datasets x orientations are scored in one nf_metrics_from_table call.  `val`:
+        _validation_data(S_summ, M_summ) (built here when not given)."""
+        import torch
+        from ...engine import ops
+        from ...datasets.nf import nf_metrics_from_table
+        dev = model.engine.dev
+        if val is None:
+            val = self._validation_data(S_summ, M_summ, dev)
         hw, ww = shape_val
-
-        def pad(x):
-            return np.pad(x, ((0, hw - x.shape[0]), (0, ww - x.shape[1])), 'reflect')
-
-        def predict(x):
-            if x.shape[0] <= hw and x.shape[1] <= ww:
-                return self._predict_window(model, pad(x), hw)[:x.shape[0], :x.shape[1]]
-            # larger than the validation window: the identity transform over overlapping tiles (probabilities)
-            import torch
-            xd = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float32)).to(model.engine.dev)
-            return model.engine.predict_tiled(xd, augmentation=False)[1].cpu().numpy()
-
-        fwd = [lambda x: x, np.fliplr, np.flipud, lambda x: np.rot90(x, 1), lambda x: np.rot90(x, 2),
-               lambda x: np.rot90(x, 3)]
-        pp, rr, ff = [], [], []
-        for s, m, (y0, y1) in zip(S_summ, M_summ, y_coords):
-            vm = np.zeros(s.shape, dtype=np.uint8)
-            vm[y0:y1, :] = 1
-            for f in fwd:
-                fs, fm = f(s), f(m)
-                yy, xx = np.where(f(vm) == 1)
-                a0, a1, b0, b1 = min(yy), max(yy), min(xx), max(xx)
-                mp = predict(fs)
-                p, r, _, _, f1 = nf_mask_metrics(fm[a0:a1, b0:b1], mp[a0:a1, b0:b1].round())
-                pp.append(p); rr.append(r); ff.append(f1)
+        win = torch.empty(hw, ww, dtype=torch.float32, device=dev)
+        preds, rows = [], []
+        with torch.cuda.device(dev):
+            for (s, m), (y0, y1) in zip(val, y_coords):
+                H, W = s.shape
+                for k in range(6):
+                    hf, wf = (W, H) if k in (3, 5) else (H, W)
+                    a0, a1, b0, b1 = self._val_box((H, W), y0, y1, k)
+                    if hf <= hw and wf <= ww:
+                        ops.orient_pad(s, k, win)
+                        mp, kind = model.engine.infer(win[None])[0][0].clone(), 1
+                    else:
+                        fs = torch.empty(hf, wf, dtype=torch.float32, device=dev)
+                        ops.orient_pad(s, k, fs)
+                        mp, kind = model.engine.predict_tiled(fs, augmentation=False)[1].clone(), 2
+                    preds.append(mp)
+                    # truth: f_k(m)[a0:a1, b0:b1] as a signed-stride view of m (uint8, row-major H x W)
+                    src = self._VAL_SRC[k]
+                    off = [i * W + j for i, j in (src(H, W, a0, b0), src(H, W, a0 + 1, b0), src(H, W, a0, b0 + 1))]
+                    rows.append([m.data_ptr() + off[0], a1 - a0, b1 - b0, off[1] - off[0], off[2] - off[0], 0, 0, 0])
+                    rows.append([mp.data_ptr() + (a0 * mp.stride(0) + b0) * mp.element_size(), a1 - a0, b1 - b0,
+                                 mp.stride(0), 1, kind, 0, 0])
+            scores = nf_metrics_from_table(np.asarray(rows, dtype=np.int64), dev)
+        pp = [sc[0] for sc in scores]
+        rr = [sc[1] for sc in scores]
+        ff = [sc[4] for sc in scores]
         eps = 1e-4 * epoch if epoch else 0
         return {'val_nf_f1_mean': float(np.mean(ff) + eps), 'val_nf_f1_median': float(np.median(ff) + eps),
                 'val_nf_f1_min': float(np.min(ff) + eps), 'val_nf_f1_adj': float(np.mean(ff) * np.min(ff) + eps),
                 'val_nf_prec': float(np.mean(pp)), 'val_nf_reca': float(np.mean(rr))}
-
-    @staticmethod
-    def _predict_window(model, x, hw):
-        return model.predict(x[np.newaxis, :, :])[0]
 
     # D4 elements of the sampler's augment_funcs as index maps on an n x n window: out[i, j] = a[M @ (i, j) + t]
     @staticmethod
@@ -493,7 +528,8 @@ class UNet2DSummary(object):
             cache['up'] = torch.cuda.Stream(device=dev)
             cache['down'] = torch.cuda.Stream(device=dev)
             cache['slots'] = [{}, {}]
-        up_stream, down_stream, slots = cache['up'], cache['down'], cache['slots']
+            cache['score'] = torch.cuda.Stream(device=dev)
+        up_stream, down_stream, slots, score_stream = cache['up'], cache['down'], cache['slots'], cache['score']
 
         def stage(i):
             dsp = dataset_paths[i]
@@ -542,8 +578,11 @@ class UNet2DSummary(object):
             Mp.append(mp)
             names.append(name)
             if print_scores:
+                # scored on a stream of its own: waiting for the scores must not wait for image i, already queued
                 m = self.mask_summary_func(dsp)
-                p, r, incl, excl, comb = nf_mask_metrics(m, mp.round())
+                with torch.cuda.stream(score_stream):
+                    truth = torch.from_numpy(np.ascontiguousarray(np.asarray(m) != 0, dtype=np.uint8)).to(dev)
+                    p, r, incl, excl, comb = nf_mask_metrics_device([(truth, torch.from_numpy(mp).to(dev))])[0]
                 logger.info('%s: prec=%.3lf, reca=%.3lf, incl=%.3lf, excl=%.3lf, comb=%.3lf' % (name, p, r, incl, excl, comb))
                 for k, v in enumerate((p, r, comb)):
                     scores[k] += v / len(dataset_paths)

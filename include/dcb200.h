@@ -357,6 +357,33 @@ int dcb_tile_combine(const float* probs, int T, int hs, int ws, const int* origi
                      const int* cuts_y, const int* cuts_x, int n_ty, int n_tx, int tile_first, int n_tiles, float threshold,
                      int n_aug, double* act, uint8_t* mask, dcb_stream_t stream);
 
+/* ---- N3: Neurofinder scoring of predicted masks (datasets/nf.py:153-174: skimage.measure.label, neurofinder.centers /
+ * shapes, threshold 5) and the validation windows of fit (unet_2d_summary.py:62-120); csrc/regions.cu ----
+ * Images are given by a table of n_images records of 8 x int64 {data pointer, H, W, row stride, column stride, kind, 0, 0}:
+ * pixel (y, x) is element y * row_stride + x * column_stride (signed, in elements), so flips, rotations and crops are views.
+ * kind 0: uint8, foreground = nonzero; 1: fp32 and 2: fp64, foreground = round(p) != 0, i.e. !(|p| <= 0.5) (NaN is
+ * foreground).  `desc` is the table on the device (read by the kernels), `h_desc` the same table on the host (shapes only,
+ * read during the call).  H and W < 2^24, at most 2^31 - 1 pixels per call.
+ * Regions are the 8-connected components numbered like scipy.ndimage.label(m != 0, structure=ones((3, 3))): in raster
+ * order of their first pixel.  Regions get global numbers in table order: image i holds regions
+ * [region_base[i], region_base[i+1]), region_base[n_images] = total.
+ * workspace_bytes: the workspace of both calls below; region_capacity bounds the total number of regions (the rows
+ * region_info must have). */
+int dcb_nf_score_workspace_bytes(const long long* h_desc, int n_images, size_t* bytes, long long* region_capacity);
+/* labels int32 [sum of H*W]: image i row-major at the sum of the earlier images' H*W, 1..n_i per region, 0 background */
+int dcb_label_regions(const long long* desc, const long long* h_desc, int n_images, int* labels, int* region_base,
+                      void* workspace, size_t workspace_bytes, dcb_stream_t stream);
+/* n_pairs (truth, prediction) pairs of equal shape, as images 2p and 2p+1 of the table.  region_info int32
+ * [region_capacity][3] per region = {pixel count, match, overlap}: for a truth region, match is the index (from 0) of the
+ * prediction region of its pair that neurofinder.match(truth, prediction, 5) assigns to it (nearest remaining centre by
+ * correctly rounded float64 distance < 5, ties to the smaller index, truth regions in label order) or -1, and overlap
+ * is the number of its pixels inside that region; prediction regions carry {count, -1, 0}. */
+int dcb_nf_score(const long long* desc, const long long* h_desc, int n_pairs, int* region_base, int* region_info,
+                 void* workspace, size_t workspace_bytes, dcb_stream_t stream);
+/* out [H][W] = np.pad(f(s), ((0, H - hf), (0, W - wf)), 'reflect') for s [hs][ws] and f = (identity, np.fliplr, np.flipud,
+ * np.rot90 k=1, 2, 3)[k] (hf x wf = shape of f(s); H >= hf, W >= wf) */
+int dcb_orient_pad_f32(const float* s, int hs, int ws, int k, int H, int W, float* out, dcb_stream_t stream);
+
 /* ---- a9: keras.optimizers.Adam (2.0.6) over one flat fp32 parameter buffer;
  * lr_t = lr*sqrt(1-b2^t)/(1-b1^t) is computed by the caller (unet_2d_summary.py:335) ---- */
 int dcb_adam_step(float* p, const float* g, float* m, float* v, long long n, float lr_t, const float* lr_t_dev,
