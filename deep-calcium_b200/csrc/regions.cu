@@ -1,7 +1,8 @@
 // Neurofinder scoring on the device (datasets/nf.py:153-174 of the reference, restated in deepcalcium/datasets/nf.py):
 // 8-connected region labelling numbered like scipy.ndimage.label(m != 0, structure=ones((3, 3))), per-region pixel
 // counts and coordinate sums, the greedy centre matching of neurofinder.match(a, b, threshold=5) and the matched
-// overlaps.  Plus the orientation + reflect pad of the fit validation windows (unet_2d_summary.py:62-120).
+// overlaps.  Plus the orientation + reflect pad of the fit validation windows (unet_2d_summary.py:62-120) and the truth
+// mask summary of a dataset's per-neuron planes (unet_2d_summary.py:244-291), whose clusters the labelling finds.
 //
 // Images come in through a device table of 8 x int64 records {ptr, H, W, row stride, col stride, kind, 0, 0}: pixel
 // (y, x) is element y * row_stride + x * col_stride of ptr (signed, in elements, so flips / rotations / crops are
@@ -13,6 +14,9 @@
 // borders are merged in global memory, the forest is flattened, and an exclusive scan of the root flags over
 // 1024-pixel chunks numbers the components in raster order of their first pixel - scipy's numbering.  Every count
 // and coordinate sum is an integer, so nothing depends on the order of the atomics.
+#include <algorithm>
+#include <climits>
+
 #include "elementwise.cuh"
 
 namespace dcb {
@@ -434,6 +438,226 @@ __global__ void orient_pad_kernel(const float* __restrict__ s, int hs, int ws, i
   }
 }
 
+// ---- mask summary (unet_2d_summary.py:244-291, _summarize_mask): masks [n][H][W] (one byte, "== 1" counts) -> [H][W]
+// Only a candidate centre - an alive pixel whose alive 3 x 3 window holds two owners - ever deletes, and deletions only
+// shrink windows.  Candidates in different 8-connected components of the 3 x 3 dilation of the candidate map are >= 4 px
+// apart, so their windows are disjoint: each component (cluster) is walked on its own, in (owner, y, x) order.
+constexpr int kZChunk = 64;      // planes per thread of the owner pass
+constexpr int kSortCap = 2048;   // largest cluster sorted in shared memory
+
+// packed[p] += {planes == 1 in this thread's chunk} << 32 | {that plane, when it is the only one}: the high word counts the
+// planes (carries from the low word only ever raise a count that is already >= 2); count 1 leaves the owner in the low word.
+// Thread = 16 consecutive pixels x kZChunk planes; block 0 also writes the labelling table record of the dilated map.
+__global__ void __launch_bounds__(256) mask_owner_kernel(const uint8_t* __restrict__ masks, int n, long long HW, bool vec,
+                                                         unsigned long long* __restrict__ packed, long long* __restrict__ desc,
+                                                         const uint8_t* dil, int H, int W) {
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    desc[0] = (long long)dil; desc[1] = H; desc[2] = W; desc[3] = W; desc[4] = 1;
+    desc[5] = desc[6] = desc[7] = 0;
+  }
+  const long long groups = (HW + 15) / 16;
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= groups * ((n + kZChunk - 1) / kZChunk)) return;
+  const long long g = t % groups, p0 = g * 16;
+  const int z0 = (int)(t / groups) * kZChunk, z1 = min(n, z0 + kZChunk);
+  uint32_t cnt[4] = {0, 0, 0, 0};                    // per-byte saturating counts of 16 pixels
+  int own[16];
+#pragma unroll
+  for (int j = 0; j < 16; ++j) own[j] = 0;
+#pragma unroll 4
+  for (int z = z0; z < z1; ++z) {
+    const uint8_t* src = masks + (size_t)z * HW + p0;
+    uint32_t w[4];
+    if (vec) {
+      const uint4 v = __ldg(reinterpret_cast<const uint4*>(src));
+      w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
+    } else {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        w[k] = 0;
+#pragma unroll
+        for (int b = 0; b < 4; ++b)
+          if (p0 + 4 * k + b < HW) w[k] |= (uint32_t)src[4 * k + b] << (8 * b);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const uint32_t eq = __vcmpeq4(w[k], 0x01010101u);
+      if (eq) {
+        cnt[k] = __vaddus4(cnt[k], eq & 0x01010101u);
+#pragma unroll
+        for (int b = 0; b < 4; ++b)
+          if ((eq >> (8 * b)) & 1u) own[4 * k + b] = z;
+      }
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 16; ++j) {
+    const unsigned c = (cnt[j >> 2] >> (8 * (j & 3))) & 0xffu;
+    if (c) atomicAdd(packed + p0 + j, ((unsigned long long)c << 32) | (c == 1 ? (unsigned)own[j] : 0u));
+  }
+}
+
+__device__ __forceinline__ int owner_at(const unsigned long long* __restrict__ packed, int H, int W, int y, int x) {
+  if (y < 0 || y >= H || x < 0 || x >= W) return -1;
+  const unsigned long long v = packed[(long long)y * W + x];
+  return (v >> 32) == 1 ? (int)(unsigned)v : -1;
+}
+
+// per pixel: own (owner or -1 when no plane or several planes claim it), out = alive, dil = 3 candidate, 1 within one
+// pixel of a candidate, 0 otherwise.  A pixel's flag needs the owners of its 5 x 5 neighbourhood.
+__global__ void __launch_bounds__(256) mask_candidates_kernel(const unsigned long long* __restrict__ packed, int H, int W,
+                                                              int* __restrict__ own, uint8_t* __restrict__ out,
+                                                              uint8_t* __restrict__ dil) {
+  const long long HW = (long long)H * W;
+  for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < HW; p += (long long)gridDim.x * blockDim.x) {
+    const int y = (int)(p / W), x = (int)(p % W);
+    int o[5][5];
+#pragma unroll
+    for (int i = 0; i < 5; ++i)
+#pragma unroll
+      for (int j = 0; j < 5; ++j) o[i][j] = owner_at(packed, H, W, y + i - 2, x + j - 2);
+    bool near = false, self = false;
+#pragma unroll
+    for (int ci = 1; ci < 4; ++ci)
+#pragma unroll
+      for (int cj = 1; cj < 4; ++cj) {
+        int mn = INT_MAX, mx = -1;
+#pragma unroll
+        for (int i = -1; i <= 1; ++i)
+#pragma unroll
+          for (int j = -1; j <= 1; ++j) {
+            const int v = o[ci + i][cj + j];
+            if (v >= 0) { mn = min(mn, v); mx = max(mx, v); }
+          }
+        const bool cand = o[ci][cj] >= 0 && mn < mx;
+        near |= cand;
+        if (ci == 2 && cj == 2) self = cand;
+      }
+    own[p] = o[2][2];
+    out[p] = o[2][2] >= 0;
+    dil[p] = self ? 3 : (near ? 1 : 0);
+  }
+}
+
+// cluster of a candidate pixel = the region number of its dilated component
+__global__ void __launch_bounds__(kChunk) mask_cluster_count_kernel(const uint8_t* __restrict__ dil, long long HW,
+                                                                    const int* __restrict__ L, const int* __restrict__ R,
+                                                                    int* __restrict__ ccount) {
+  const long long p = (long long)blockIdx.x * kChunk + threadIdx.x;
+  if (p < HW && dil[p] == 3) atomicAdd(ccount + R[L[p]], 1);
+}
+
+// coff[c] = first key of cluster c (exclusive scan over the clusters the labelling found); coff[nclus] = candidates
+__global__ void __launch_bounds__(1024) mask_cluster_scan_kernel(const int* __restrict__ region_base,
+                                                                 const int* __restrict__ ccount, int* __restrict__ coff) {
+  __shared__ int warp_tot[32];
+  const int nclus = region_base[1];
+  int carry = 0;
+  for (int base = 0; base < nclus; base += blockDim.x) {
+    const int i = base + threadIdx.x;
+    int tot;
+    const int e = block_exclusive_scan(i < nclus ? ccount[i] : 0, warp_tot, &tot);
+    if (i < nclus) coff[i] = carry + e;
+    carry += tot;
+  }
+  if (threadIdx.x == 0) coff[nclus] = carry;
+}
+
+// keys of cluster c in coff[c]..coff[c+1] (unordered; the walk sorts them): owner << 32 | linear index
+__global__ void __launch_bounds__(kChunk) mask_cluster_scatter_kernel(const uint8_t* __restrict__ dil, long long HW,
+                                                                      const int* __restrict__ L, const int* __restrict__ R,
+                                                                      const int* __restrict__ own, const int* __restrict__ coff,
+                                                                      int* __restrict__ ccount,
+                                                                      unsigned long long* __restrict__ keys) {
+  const long long p = (long long)blockIdx.x * kChunk + threadIdx.x;
+  if (p >= HW || dil[p] != 3) return;
+  const int c = R[L[p]];
+  const int slot = atomicSub(ccount + c, 1) - 1;
+  keys[coff[c] + slot] = ((unsigned long long)(unsigned)own[p] << 32) | (unsigned long long)p;
+}
+
+// block-wide merge sort of n distinct keys: in each pass every key moves to (its index in its run) + (keys of the partner
+// run that are smaller).  a and b are both shared or both global memory; returns the buffer that holds the result.
+__device__ unsigned long long* block_sort_keys(unsigned long long* a, unsigned long long* b, int n) {
+  for (int w = 1; w < n; w <<= 1) {
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      const unsigned long long k = a[i];
+      const int r = i / w, mine = r * w, other = (r ^ 1) * w, start = min(mine, other);
+      int lo = other, hi = min(other + w, n);
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (a[mid] < k) lo = mid + 1; else hi = mid;
+      }
+      b[start + (i - mine) + (lo - other)] = k;
+    }
+    __syncthreads();
+    unsigned long long* t = a; a = b; b = t;
+  }
+  return a;
+}
+
+// one block per cluster (grid-stride over the cluster count, read on the device): sort its keys - in shared memory when
+// they fit, else in place in global memory against the scratch copy tmp - then one thread walks them in order and
+// deletes every alive pixel of each window that still holds two owners
+__global__ void __launch_bounds__(256) mask_walk_kernel(const int* __restrict__ region_base, const int* __restrict__ coff,
+                                                        unsigned long long* keys, unsigned long long* tmp,
+                                                        const int* __restrict__ own, int H, int W, uint8_t* alive) {
+  __shared__ unsigned long long sa[kSortCap], sb[kSortCap];
+  const int nclus = region_base[1];
+  for (int c = blockIdx.x; c < nclus; c += gridDim.x) {
+    const int k0 = coff[c], n = coff[c + 1] - k0;
+    unsigned long long* sorted;
+    if (n <= kSortCap) {
+      for (int i = threadIdx.x; i < n; i += blockDim.x) sa[i] = keys[k0 + i];
+      __syncthreads();
+      sorted = block_sort_keys(sa, sb, n);
+    } else {
+      sorted = block_sort_keys(keys + k0, tmp + k0, n);
+    }
+    if (threadIdx.x == 0) {
+      for (int i = 0; i < n; ++i) {
+        const int p = (int)(unsigned)sorted[i], y = p / W, x = p % W;
+        const int y0 = max(y - 1, 0), y1 = min(y + 1, H - 1), x0 = max(x - 1, 0), x1 = min(x + 1, W - 1);
+        int mn = INT_MAX, mx = -1;
+        for (int yy = y0; yy <= y1; ++yy)
+          for (int xx = x0; xx <= x1; ++xx)
+            if (alive[yy * W + xx]) { const int o = own[yy * W + xx]; mn = min(mn, o); mx = max(mx, o); }
+        if (mn < mx)
+          for (int yy = y0; yy <= y1; ++yy)
+            for (int xx = x0; xx <= x1; ++xx) alive[yy * W + xx] = 0;
+      }
+    }
+    __syncthreads();
+  }
+}
+
+struct MaskLayout {
+  Layout lab;
+  long long HW = 0;
+  size_t o_desc, o_base, o_packed, o_own, o_dil, o_ccount, o_coff, o_tmp, bytes;
+};
+
+int make_mask_layout(int n, int H, int W, MaskLayout& ml) {
+  DCB_CHECK_ARG(n >= 0 && H >= 0 && W >= 0, "mask summary: bad shape %d x %d x %d", n, H, W);
+  ml.HW = (long long)H * W;
+  const long long h_desc[8] = {1, H, W, W, 1, 0, 0, 0};        // shapes only: the pointer is set on the device
+  const int st = make_layout(h_desc, 1, ml.lab);
+  if (st != DCB_OK) return st;
+  size_t o = align_up(ml.lab.bytes);
+  auto take = [&](size_t bytes) { const size_t at = o; o = align_up(o + bytes); return at; };
+  ml.o_desc = take(8 * sizeof(long long));
+  ml.o_base = take(2 * sizeof(int));
+  ml.o_packed = take(sizeof(unsigned long long) * ml.HW);      // after the candidate pass: the cluster keys
+  ml.o_own = take(sizeof(int) * ml.HW);
+  ml.o_dil = take(ml.HW);
+  ml.o_ccount = take(sizeof(int) * ml.lab.rcap);
+  ml.o_coff = take(sizeof(int) * (ml.lab.rcap + 1));
+  ml.o_tmp = take(sizeof(unsigned long long) * ml.HW);
+  ml.bytes = o;
+  return DCB_OK;
+}
+
 }  // namespace
 }  // namespace dcb
 
@@ -509,6 +733,64 @@ extern "C" int dcb_nf_score(const long long* desc, const long long* h_desc, int 
     DCB_LAUNCH_OK("overlap_kernel");
     g_launches += 2;
   }
+  return DCB_OK;
+}
+
+extern "C" int dcb_mask_summary_workspace_bytes(int n, int H, int W, size_t* bytes) {
+  DCB_CHECK_ARG(bytes, "dcb_mask_summary_workspace_bytes: null output");
+  MaskLayout ml;
+  const int st = make_mask_layout(n, H, W, ml);
+  if (st != DCB_OK) return st;
+  *bytes = n == 0 ? 0 : ml.bytes;
+  return DCB_OK;
+}
+
+extern "C" int dcb_mask_summary(const uint8_t* masks, int n, int H, int W, uint8_t* out, void* workspace,
+                                size_t workspace_bytes, dcb_stream_t stream) {
+  MaskLayout ml;
+  int st = make_mask_layout(n, H, W, ml);
+  if (st != DCB_OK) return st;
+  const cudaStream_t s = (cudaStream_t)stream;
+  if (ml.HW == 0) return DCB_OK;
+  DCB_CHECK_ARG(out && (n == 0 || masks), "dcb_mask_summary: null pointer");
+  if (n == 0) {
+    DCB_CUDA_OK(cudaMemsetAsync(out, 0, ml.HW, s));
+    return DCB_OK;
+  }
+  if (!workspace || workspace_bytes < ml.bytes)
+    return fail(DCB_ERR_WORKSPACE, "dcb_mask_summary: workspace of %zu bytes, %zu needed", workspace_bytes, ml.bytes);
+  void* ws = workspace;
+  long long* desc = at<long long>(ws, ml.o_desc);
+  int* base = at<int>(ws, ml.o_base);
+  auto* packed = at<unsigned long long>(ws, ml.o_packed);
+  int* own = at<int>(ws, ml.o_own);
+  uint8_t* dil = at<uint8_t>(ws, ml.o_dil);
+  int* ccount = at<int>(ws, ml.o_ccount);
+  int* coff = at<int>(ws, ml.o_coff);
+  DCB_CUDA_OK(cudaMemsetAsync(packed, 0, sizeof(unsigned long long) * ml.HW, s));
+  DCB_CUDA_OK(cudaMemsetAsync(ccount, 0, sizeof(int) * ml.lab.rcap, s));
+  const bool vec = ml.HW % 16 == 0 && reinterpret_cast<uintptr_t>(masks) % 16 == 0;
+  const long long threads = (ml.HW + 15) / 16 * cdiv(n, kZChunk);
+  DCB_CHECK_ARG(threads / 256 < (1ll << 31), "dcb_mask_summary: %d x %d x %d masks are too many for one call", n, H, W);
+  mask_owner_kernel<<<cdiv(threads, 256), 256, 0, s>>>(masks, n, ml.HW, vec, packed, desc, dil, H, W);
+  DCB_LAUNCH_OK("mask_owner_kernel");
+  const int cap = sm_count() * 8;
+  mask_candidates_kernel<<<std::min(cdiv(ml.HW, 256), cap), 256, 0, s>>>(packed, H, W, own, out, dil);
+  DCB_LAUNCH_OK("mask_candidates_kernel");
+  g_launches += 2;
+  st = label_core(desc, 1, ml.lab, ws, base, s);
+  if (st != DCB_OK) return st;
+  const int* L = at<int>(ws, ml.lab.o_L); const int* R = at<int>(ws, ml.lab.o_R);
+  mask_cluster_count_kernel<<<ml.lab.nchunks, kChunk, 0, s>>>(dil, ml.HW, L, R, ccount);
+  DCB_LAUNCH_OK("mask_cluster_count_kernel");
+  mask_cluster_scan_kernel<<<1, 1024, 0, s>>>(base, ccount, coff);
+  DCB_LAUNCH_OK("mask_cluster_scan_kernel");
+  mask_cluster_scatter_kernel<<<ml.lab.nchunks, kChunk, 0, s>>>(dil, ml.HW, L, R, own, coff, ccount, packed);
+  DCB_LAUNCH_OK("mask_cluster_scatter_kernel");
+  mask_walk_kernel<<<(int)std::min<long long>(ml.lab.rcap, cap), 256, 0, s>>>(base, coff, packed,
+                                                                      at<unsigned long long>(ws, ml.o_tmp), own, H, W, out);
+  DCB_LAUNCH_OK("mask_walk_kernel");
+  g_launches += 4;
   return DCB_OK;
 }
 

@@ -46,6 +46,26 @@ def summarize_movie_device(movie_dev, floor_max_at_zero=False, variant=-1, t_spl
     return out
 
 
+def summarize_masks_device(masks_dev):
+    """masks_dev: int8, uint8 or bool CUDA tensor [n,H,W], one plane per neuron (a neuron owns the pixels where its plane
+    == 1).  Returns the truth mask of _summarize_mask (unet_2d_summary.py:244-291) as a uint8 CUDA tensor [H,W]: pixels
+    owned by one neuron, minus every 3x3 neighbourhood the reference's walk finds touching two neurons."""
+    import torch
+    from ..engine import ops
+    if masks_dev.dim() != 3:
+        raise ValueError('masks must be [n,H,W], got shape %s' % (tuple(masks_dev.shape),))
+    if masks_dev.dtype not in (torch.int8, torch.uint8, torch.bool) or not masks_dev.is_cuda:
+        raise TypeError('summarize_masks_device needs an int8, uint8 or bool CUDA tensor, got %s on %s'
+                        % (masks_dev.dtype, masks_dev.device))
+    masks_dev = masks_dev.contiguous()
+    n, H, W = masks_dev.shape
+    with torch.cuda.device(masks_dev.device):
+        out = torch.empty(H, W, dtype=torch.uint8, device=masks_dev.device)
+        ws = torch.empty(ops.mask_summary_workspace_bytes(n, H, W), dtype=torch.uint8, device=masks_dev.device)
+        ops.mask_summary(masks_dev, out, ws)
+    return out
+
+
 def summarize_movie(movie, floor_max_at_zero=False):
     """Mean / max projection of a [T,H,W] movie given as a numpy array (any real dtype; the
     reference's TIFF frames are int16, nf.py:121) -> (mean float32 [H,W], max float32 [H,W]).
@@ -78,9 +98,11 @@ def _h5():
         return hdf5_lite
 
 
-def open_dataset(path):
+def open_dataset(path, keys=None):
     """Read a dataset file into a dict {'name', 'series/mean', 'series/max', 'masks/raw', ...}: the reference's HDF5
-    schema (datasets/nf.py:39-44; ``series/raw``, the movie itself, is not loaded) or the .npz container."""
+    schema (datasets/nf.py:39-44; ``series/raw``, the movie itself, is not loaded) or the .npz container.
+    ``keys``: read only these arrays (e.g. ``('masks/raw',)``; missing ones are left out); 'name' is always there."""
+    want = None if keys is None else set(keys)
     if _is_hdf5(path):
         out = {}
         with _h5().File(path, 'r') as fp:
@@ -89,11 +111,13 @@ def open_dataset(path):
             for grp in ('series', 'masks'):
                 if grp in fp:
                     for k in fp[grp].keys():
-                        if k != 'raw' or grp == 'masks':
-                            out['%s/%s' % (grp, k)] = np.asarray(fp[grp][k][...])
+                        key = '%s/%s' % (grp, k)
+                        if (k != 'raw' or grp == 'masks') and (want is None or key in want):
+                            out[key] = np.asarray(fp[grp][k][...])
         return out
     with np.load(path, allow_pickle=False) as z:
-        out = {k.replace('__', '/'): z[k] for k in z.files}
+        out = {k.replace('__', '/'): z[k] for k in z.files
+               if want is None or k == 'name' or k.replace('__', '/') in want}
     out['name'] = str(out['name'])
     return out
 

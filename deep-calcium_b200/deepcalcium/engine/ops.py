@@ -499,6 +499,21 @@ def nf_score(desc, h_desc, region_base, region_info, workspace):
          ptr(workspace), c_sz(workspace.numel()), stream_ptr())
 
 
+def mask_summary_workspace_bytes(n, H, W):
+    out = c_sz(0)
+    call('dcb_mask_summary_workspace_bytes', c_int(n), c_int(H), c_int(W), ctypes.byref(out))
+    return out.value
+
+
+def mask_summary(masks, out, workspace):
+    """masks [n, H, W] (int8, uint8 or bool) -> out uint8 [H, W]: the reference's _summarize_mask"""
+    _chk(masks); _chk(out, torch.uint8)
+    assert masks.element_size() == 1, masks.dtype
+    n, H, W = masks.shape
+    call('dcb_mask_summary', ptr(masks), c_int(n), c_int(H), c_int(W), ptr(out), ptr(workspace),
+         c_sz(workspace.numel() if workspace is not None else 0), stream_ptr())
+
+
 def orient_pad(s, k, out):
     """out [H, W] = np.pad(f_k(s), ((0, H - hf), (0, W - wf)), 'reflect'), f_k = (identity, fliplr, flipud, rot90 1/2/3)[k]"""
     _chk(s, torch.float32); _chk(out, torch.float32)

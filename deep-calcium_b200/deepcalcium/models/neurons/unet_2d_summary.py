@@ -22,7 +22,7 @@ from ...utils.runtime import funcname
 from ...utils import neurons as _un
 from ...utils.neurons import (F1, prec, reca, dice, dicesq, dice_loss, dicesq_loss, posyt, posyp,
                               weighted_binary_crossentropy, binary_crossentropy)
-from ...datasets.nf import open_dataset, nf_mask_metrics_device
+from ...datasets.nf import open_dataset, nf_mask_metrics_device, summarize_masks_device
 
 MODEL_URL_LATEST = 'https://github.com/alexklibisz/deep-calcium/releases/download/v0.0.1-weights/unet2ds_model.hdf5'
 METRIC_NAMES = ['loss', 'F1', 'prec', 'reca', 'dice', 'dicesq', 'posyt', 'posyp']   # unet_2d_summary.py:398-399
@@ -191,7 +191,7 @@ def _summarize_series(dspath):
     """unet_2d_summary.py:227-241: series/mean -> float32 -> (x - mean) / std, on the GPU."""
     import torch
     from ...engine import ops
-    ds = open_dataset(dspath)
+    ds = open_dataset(dspath, keys=('series/mean',))
     summ = torch.from_numpy(np.ascontiguousarray(ds['series/mean'].astype(np.float32))).cuda()
     out = torch.empty_like(summ)
     ops.standardize(summ, out)
@@ -201,30 +201,18 @@ def _summarize_series(dspath):
 def _summarize_mask(dspath):
     """unet_2d_summary.py:244-291: flatten the per-neuron masks; drop pixels claimed by more than one
     neuron, then drop any 3x3 neighbourhood that still touches two different neurons (same visiting
-    order as the reference: first-seen order of the (y,x) keys)."""
-    msks = open_dataset(dspath)['masks/raw']
-    zz, yy, xx = np.where(msks == 1)
-    owner = {}
-    for z, y, x in zip(zz.tolist(), yy.tolist(), xx.tolist()):
-        owner.setdefault((y, x), []).append(z)
-    for k in [k for k, v in owner.items() if len(v) > 1]:
-        del owner[k]
-    for (y, x) in list(owner.keys()):
-        nbrs = [(y - 1, x), (y + 1, x), (y, x - 1), (y, x + 1), (y + 1, x + 1), (y - 1, x - 1), (y + 1, x - 1),
-                (y - 1, x + 1), (y, x)]
-        nbrs = [k for k in nbrs if k in owner]
-        if len(set(owner[k][0] for k in nbrs)) > 1:
-            for k in nbrs:
-                del owner[k]
-    summ = np.zeros(msks.shape[1:])
-    if owner:
-        ys, xs = zip(*owner.keys())
-        summ[list(ys), list(xs)] = 1.
-    return summ
+    order as the reference: first-seen order of the (y,x) keys).  Runs on the GPU (summarize_masks_device);
+    returns float64 [H, W] like the reference."""
+    import torch
+    msks = open_dataset(dspath, keys=('masks/raw',))['masks/raw']
+    if msks.dtype.itemsize != 1 or msks.dtype.kind not in 'biu':
+        msks = msks == 1                       # the device takes one-byte planes; "== 1" is the only test applied
+    out = summarize_masks_device(torch.from_numpy(np.ascontiguousarray(msks)).cuda())
+    return out.cpu().numpy().astype(np.float64)
 
 
 def _name_dataset(dspath):
-    return open_dataset(dspath)['name']
+    return open_dataset(dspath, keys=())['name']
 
 
 def _pixel_scores(m, mp):
@@ -577,6 +565,7 @@ class UNet2DSummary(object):
                 mp = sl['hout'].numpy().copy()
             Mp.append(mp)
             names.append(name)
+            m = None
             if print_scores:
                 # scored on a stream of its own: waiting for the scores must not wait for image i, already queued
                 m = self.mask_summary_func(dsp)
@@ -588,9 +577,10 @@ class UNet2DSummary(object):
                     scores[k] += v / len(dataset_paths)
             if save:                                   # outlined figure (:610-619): truth in blue when the dataset has masks
                 from PIL import Image
-                ds = open_dataset(dsp) if isinstance(dsp, str) and path.exists(dsp) else {}
+                ds = open_dataset(dsp, keys=('masks/raw',)) if isinstance(dsp, str) and path.exists(dsp) else {}
                 if 'masks/raw' in ds:
-                    outlined = _un.mask_outlines(sl['summ'], [self.mask_summary_func(dsp), mp.round()], ['blue', 'red'])
+                    m = self.mask_summary_func(dsp) if m is None else m
+                    outlined = _un.mask_outlines(sl['summ'], [m, mp.round()], ['blue', 'red'])
                 else:
                     outlined = _un.mask_outlines(sl['summ'], [mp.round()], ['red'])
                 save_path = '%s/%s_mp.png' % (self.cpdir, name)

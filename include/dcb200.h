@@ -380,6 +380,16 @@ int dcb_label_regions(const long long* desc, const long long* h_desc, int n_imag
  * is the number of its pixels inside that region; prediction regions carry {count, -1, 0}. */
 int dcb_nf_score(const long long* desc, const long long* h_desc, int n_pairs, int* region_base, int* region_info,
                  void* workspace, size_t workspace_bytes, dcb_stream_t stream);
+/* Truth mask of a dataset (unet_2d_summary.py:244-291, _summarize_mask): masks [n][H][W], one byte per pixel (int8, uint8
+ * or bool; a neuron owns the pixels where its plane == 1) -> out [H][W] uint8, 1 where the reference's summary is 1.0.
+ * Pixels owned by several neurons are dropped; then the survivors are visited in (owner, y, x) order and every visited
+ * centre whose alive 3 x 3 window holds two owners drops that whole window.  The result is bit-identical to that
+ * sequential walk: only centres whose initial window holds two owners can drop anything, and those more than 3 px apart
+ * (in separate components of the dilated candidate map, labelled as in dcb_label_regions) never interact, so each
+ * component is sorted and walked on its own.  n == 0 writes zeros and needs no workspace.  H and W < 2^24, H * W < 2^31. */
+int dcb_mask_summary_workspace_bytes(int n, int H, int W, size_t* bytes);
+int dcb_mask_summary(const uint8_t* masks, int n, int H, int W, uint8_t* out, void* workspace, size_t workspace_bytes,
+                     dcb_stream_t stream);
 /* out [H][W] = np.pad(f(s), ((0, H - hf), (0, W - wf)), 'reflect') for s [hs][ws] and f = (identity, np.fliplr, np.flipud,
  * np.rot90 k=1, 2, 3)[k] (hf x wf = shape of f(s); H >= hf, W >= wf) */
 int dcb_orient_pad_f32(const float* s, int hs, int ws, int k, int H, int W, float* out, dcb_stream_t stream);
