@@ -824,6 +824,7 @@ static int launch_slab(K kernel, const P& p, const SlabGeom& gm, cudaStream_t st
   cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, p, gm);
   if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(e));
   g_launches += 1;
+  note_kernel(name);
   return DCB_OK;
 }
 
@@ -903,6 +904,7 @@ static int launch_bn_fwd(BnFwdParams& p, void* ws, size_t ws_bytes, cudaStream_t
     if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of bn_train_fwd_kernel failed: %s", cudaGetErrorString(le));
   }
   g_launches += 1;
+  note_kernel(VEC == 8 ? (POOL ? "bn_train_fwd_v8_pool" : "bn_train_fwd_v8") : (POOL ? "bn_train_fwd_v4_pool" : "bn_train_fwd_v4"));
   return DCB_OK;
 }
 
@@ -929,8 +931,8 @@ extern "C" int dcb_bn_train_fwd(int dtype, const void* x, long long M, int C, lo
     SlabGeom gm;
     if (p.pv.world == 1 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0 &&
         slab_geom(M, C, dtype == DCB_F32 ? 4 : 2, pool_out ? 2LL * W : 1, 5LL << 20, gm)) {
-      if (pool_out) { BN_DISPATCH(dtype, return launch_slab(bn_slab_fwd_kernel<T, true>, p, gm, st, "bn_slab_fwd_kernel");) }
-      else { BN_DISPATCH(dtype, return launch_slab(bn_slab_fwd_kernel<T, false>, p, gm, st, "bn_slab_fwd_kernel");) }
+      if (pool_out) { BN_DISPATCH(dtype, return launch_slab(bn_slab_fwd_kernel<T, true>, p, gm, st, "bn_slab_fwd_pool");) }
+      else { BN_DISPATCH(dtype, return launch_slab(bn_slab_fwd_kernel<T, false>, p, gm, st, "bn_slab_fwd");) }
     }
   }
   if (vec == 8) {
@@ -953,6 +955,8 @@ static int launch_bn_fwd_sums(BnFwdParams& p, cudaStream_t st) {
   const cudaError_t le = launch_k(bn_train_fwd_kernel<T, VEC, POOL, true>, (int)grid, 256, smem, st, policy(DCB_POLICY_PDL) != 0, p);
   if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of bn_train_fwd_kernel (sums) failed: %s", cudaGetErrorString(le));
   g_launches += 1;
+  note_kernel(VEC == 8 ? (POOL ? "bn_train_fwd_sums_v8_pool" : "bn_train_fwd_sums_v8")
+                       : (POOL ? "bn_train_fwd_sums_v4_pool" : "bn_train_fwd_sums_v4"));
   return DCB_OK;
 }
 
@@ -999,6 +1003,7 @@ static int launch_bn_bwd(BnBwdParams& p, void* ws, size_t ws_bytes, cudaStream_t
     if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of bn_train_bwd_kernel failed: %s", cudaGetErrorString(le));
   }
   g_launches += 1;
+  note_kernel(VEC == 8 ? (p.gpix ? "bn_train_bwd_v8_rank1" : "bn_train_bwd_v8") : (p.gpix ? "bn_train_bwd_v4_rank1" : "bn_train_bwd_v4"));
   return DCB_OK;
 }
 
@@ -1051,7 +1056,7 @@ static int bn_train_bwd_impl(int dtype, const float* dy, int ldy, int offy, cons
   {
     SlabGeom gm;
     if (!gpix && p.pv.world == 1 && (reinterpret_cast<uintptr_t>(draw) & 15) == 0 && slab_geom(M, C, dtype == DCB_F32 ? 4 : 2, 1, 5LL << 19, gm)) {
-      BN_DISPATCH(dtype, return launch_slab(bn_slab_bwd_kernel<T>, p, gm, st, "bn_slab_bwd_kernel");)
+      BN_DISPATCH(dtype, return launch_slab(bn_slab_bwd_kernel<T>, p, gm, st, "bn_slab_bwd");)
     }
   }
   if (vec == 8) { BN_DISPATCH(dtype, return (launch_bn_bwd<T, 8>(p, workspace, workspace_bytes, st));) }

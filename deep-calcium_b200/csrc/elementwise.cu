@@ -904,6 +904,7 @@ extern "C" int dcb_bn_apply(int dtype, const void* x, long long M, int C, const 
   }
   g_launches += 1;
   DCB_LAUNCH_OK("bn_apply_kernel");
+  note_kernel(C % 8 == 0 ? "bn_apply_v8" : "bn_apply_v4");
   return DCB_OK;
 }
 
@@ -928,6 +929,7 @@ extern "C" int dcb_bn_finalize_apply(int dtype, const void* x, long long M, int 
   }
   g_launches += 1;
   DCB_LAUNCH_OK("bn_finalize_apply_kernel");
+  note_kernel(C % 8 == 0 ? "bn_finalize_apply_v8" : "bn_finalize_apply_v4");
   return DCB_OK;
 }
 
@@ -949,6 +951,7 @@ extern "C" int dcb_bn_bwd_reduce(int dtype, const float* dy, int ldy, int offy, 
   }
   g_launches += 1;
   DCB_LAUNCH_OK("bn_bwd_reduce_kernel");
+  note_kernel(C % 8 == 0 && 256 % (C / 8) == 0 ? "bn_bwd_reduce_v8" : "bn_bwd_reduce_v4");
   return DCB_OK;
 }
 
@@ -970,6 +973,7 @@ extern "C" int dcb_bn_bwd_apply(int dtype, const float* dy, int ldy, int offy, c
   }
   g_launches += 1;
   DCB_LAUNCH_OK("bn_bwd_apply_kernel");
+  note_kernel(C % 8 == 0 ? "bn_bwd_apply_v8" : "bn_bwd_apply_v4");
   return DCB_OK;
 }
 

@@ -105,7 +105,7 @@ class policy(object):
 
 
 def last_kernel():
-    """name of the contraction-kernel variant the last dcb_conv* / dcb_*wgrad call of this thread dispatched to"""
+    """name of the kernel variant the last dcb_conv* / dcb_*wgrad / BatchNorm call of this thread dispatched to"""
     s = lib().dcb_last_kernel()
     return s.decode() if s else ''
 

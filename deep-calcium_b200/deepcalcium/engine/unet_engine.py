@@ -481,6 +481,25 @@ class UNetEngine(object):
     def _dropout_p(self, name, enabled):
         return float(self.spec.dropout_after().get(name, 0.)) if enabled else 0.
 
+    def _layer_ids(self):
+        """{tensor name: layer id} of a training step: a block's index in dspec.blocks, len(blocks) + i for the i-th
+        nearest-upsampled tensor of the 'upsampling' graph.  The id selects the block's BatchNorm barrier words and is
+        the layer word of its dropout mask's Philox counter (elementwise.cuh, dropout_scale8)."""
+        layer_id = {blk.name: i for i, blk in enumerate(self.dspec.blocks)}
+        for i, un in enumerate(self._ups):
+            layer_id[un] = len(self.dspec.blocks) + i
+        return layer_id
+
+    def dropout_seed_base(self):
+        """Host half of the dropout key: the kernels draw with seed_base ^ step_state[1], the device half that every
+        step advances before its kernels read it.  Ranks of a data-parallel run draw different masks for their crops."""
+        return (self.comm.rank if self.comm is not None else 0) * 0x9E3779B1
+
+    def dropout_layers(self):
+        """{tensor name: (layer id, drop probability)} of the tensors a training step with dropout drops out"""
+        layer_id = self._layer_ids()
+        return OrderedDict((n, (layer_id[n], float(p))) for n, p in self.spec.dropout_after().items())
+
     def _allreduce(self, t):
         if self.comm is not None and self.comm.world > 1:
             self.comm.allreduce_sum(t)
@@ -488,8 +507,7 @@ class UNetEngine(object):
     def _train_step_enqueue(self, s, loss_id, lr, dropout, beta1, beta2, eps):
         spec, act, raw, dxb = self.dspec, s['act'], s['raw'], s['dx']
         world = self.comm.world if self.comm is not None else 1
-        # ranks draw different dropout masks for their own crops
-        seed_base = (self.comm.rank if self.comm is not None else 0) * 0x9E3779B1
+        seed_base = self.dropout_seed_base()
         seed_dev = self.step_state[1:2]
         ops.step_advance(self.step_state, lr, beta1, beta2, self.lr_t)
         self.dbl.zero_()
@@ -514,9 +532,7 @@ class UNetEngine(object):
                 prep_done.record(side)
         else:
             self._prepare_weights(for_training=True)
-        layer_id = {blk.name: i for i, blk in enumerate(spec.blocks)}
-        for i, un in enumerate(self._ups):
-            layer_id[un] = len(spec.blocks) + i
+        layer_id = self._layer_ids()
         # ---------------- forward (batch-statistic BN)
         for blk in spec.blocks:
             n = blk.name

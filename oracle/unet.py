@@ -149,7 +149,7 @@ def _bn(x, g, be, mm, mv, training, stats_out, name):
 
 
 def unet_forward(w, x, spec=UNetSpec(), training=False, dropout_keep=None, dtype=torch.float64,
-                 return_intermediates=False, requires_grad=False, emulate_bf16=False):
+                 return_intermediates=False, requires_grad=False, emulate_bf16=False, relu_gate=None):
     """Forward pass.  ``x``: [N,H,W] array.  Returns dict with
       'logit' = z1 - z0 (so prob = sigmoid(logit) = softmax(z)[..., -1]),
       'prob', and (training) 'bn_stats' {layer: (batch_mean, batch_var)}.
@@ -162,6 +162,9 @@ def unet_forward(w, x, spec=UNetSpec(), training=False, dropout_keep=None, dtype
     training path is compared with: the fp64 gradient of this randomly initialised dice-loss network is
     ill-conditioned w.r.t. 2^-9 perturbations of the activations (tens of percent), so only a
     reference with the same storage rounding isolates implementation errors.
+    ``relu_gate``: {block name: 0/1 array [N,C,H,W]} - the block's ReLU keeps exactly the gated elements instead of
+    deciding by the sign of its own pre-activation.  A pre-activation within a rounding error of 0 has no sign that
+    every correct evaluation agrees on; a test can take those decisions from the implementation it checks.
     """
     rb = _RoundBF16.apply if emulate_bf16 else (lambda t: t)
     tw = OrderedDict((k, torch.tensor(np.asarray(v), dtype=dtype, requires_grad=(
@@ -185,7 +188,10 @@ def unet_forward(w, x, spec=UNetSpec(), training=False, dropout_keep=None, dtype
             inter[name + '/raw'] = t
         t = _bn(t, tw[name + '/gamma'], tw[name + '/beta'], tw[name + '/moving_mean'],
                 tw[name + '/moving_var'], training, stats, name)
-        t = torch.relu(t)
+        if relu_gate is not None and name in relu_gate:
+            t = t * torch.as_tensor(relu_gate[name], dtype=dtype)
+        else:
+            t = torch.relu(t)
         if name not in drops or not (training and dropout_keep is not None):
             t = rb(t)
         if return_intermediates:
@@ -260,12 +266,12 @@ def keras_adam_update(p, g, m, v, iteration, lr=0.002, beta_1=0.9, beta_2=0.999,
 
 
 def train_step(w, x, y, opt_state=None, spec=UNetSpec(), loss='dice_loss', lr=0.002,
-               dropout_keep=None, dtype=torch.float64, emulate_bf16=False):
+               dropout_keep=None, dtype=torch.float64, emulate_bf16=False, relu_gate=None):
     """One ``train_on_batch``: forward with batch-stat BN, loss, autograd,
     Keras-Adam on the trainable tensors, momentum update of the BN moving stats.
     Returns (loss, new_weights, new_opt_state, grads, forward_out)."""
     out = unet_forward(w, x, spec, training=True, dropout_keep=dropout_keep, dtype=dtype, requires_grad=True,
-                       emulate_bf16=emulate_bf16)
+                       emulate_bf16=emulate_bf16, relu_gate=relu_gate)
     yt = torch.as_tensor(np.asarray(y), dtype=dtype)
     L = LOSSES[loss](yt, out['prob'])
     params = {k: t for k, t in out['params'].items() if t.requires_grad}

@@ -556,28 +556,6 @@ def _check_single_launch_batchnorm(precision, shape):
     assert torch.equal(x2, draw)
 
 
-@pytest.mark.parametrize('precision', ['fp32', 'bf16'])
-def test_dropout_is_consistent_between_forward_and_backward(cuda, precision):
-    from deepcalcium.engine import ops
-    dt = DT[precision]
-    M, C = 4096, 64
-    x = torch.ones(1, 1, M, C, dtype=dt, device='cuda')
-    one, zero = torch.ones(C, device='cuda'), torch.zeros(C, device='cuda')
-    y = torch.empty_like(x)
-    seed_dev = torch.tensor([12345], dtype=torch.int64, device='cuda')
-    ops.bn_apply(x, one, zero, y, True, 0.5, 7, seed_dev, 3)
-    keep = (y.float() > 0)
-    frac = keep.float().mean().item()
-    assert 0.47 < frac < 0.53 and torch.all(y.float()[keep] == 2.0)
-    y2 = torch.empty_like(x)
-    ops.bn_apply(x, one, zero, y2, True, 0.5, 7, seed_dev, 4)       # another layer -> another mask
-    assert (y2 != y).float().mean().item() > 0.3
-    # backward sees the same mask: sum dz over rows == 2 * kept count per channel (dy = 1, xhat = 0)
-    sums = torch.zeros(2 * C, dtype=torch.float64, device='cuda')
-    ops.bn_bwd_reduce(x.float(), C, 0, x, one, zero, one, one, sums, 0.5, 7, seed_dev, 3)
-    assert torch.allclose(sums[:C], 2.0 * keep.view(M, C).double().sum(0))
-
-
 @pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
 def test_maxpool_forward_and_backward_routing(cuda, precision):
     from deepcalcium.engine import ops
