@@ -16,7 +16,6 @@
 #include "stats_epilogue.cuh"
 
 namespace dcb {
-extern unsigned long long g_launches;
 
 struct PeerView {
   int world, rank;
@@ -796,34 +795,9 @@ static bool slab_geom(long long M, int C, int esize, long long row_gran, long lo
   return false;
 }
 
-template <typename K, typename P>
-static int launch_slab(K kernel, const P& p, const SlabGeom& gm, cudaStream_t st, const char* name) {
-  // clusters of 16 CTAs are "non-portable": opt in once per kernel (the template instances share one function-pointer
-  // type, so the set of prepared kernels is keyed by address)
-  static const void* prepared[8];
-  static int n_prepared = 0;
-  bool done = false;
-  for (int i = 0; i < n_prepared; ++i) done = done || prepared[i] == reinterpret_cast<const void*>(kernel);
-  if (!done) {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cluster-size attribute for %s failed: %s", name, cudaGetErrorString(e));
-    if (n_prepared < 8) prepared[n_prepared++] = reinterpret_cast<const void*>(kernel);
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)((p.C / gm.CW) * gm.S), 1, 1);
-  cfg.blockDim = dim3(SLAB_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = st;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = (unsigned)gm.S; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = policy(DCB_POLICY_PDL) != 0 ? 2 : 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, p, gm);
-  if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(e));
-  g_launches += 1;
+template <typename P>
+static int launch_slab(void (*kernel)(P, SlabGeom), const P& p, const SlabGeom& gm, cudaStream_t st, const char* name) {
+  if (int e = launch(kernel, name, (p.C / gm.CW) * gm.S, SLAB_THREADS, 0, 0, st, policy(DCB_POLICY_PDL) != 0, gm.S, p, gm)) return e;
   note_kernel(name);
   return DCB_OK;
 }
@@ -899,11 +873,8 @@ static int launch_bn_fwd(BnFwdParams& p, void* ws, size_t ws_bytes, cudaStream_t
   const size_t need = 2 * (size_t)p.C * sizeof(long long);
   if (!ws || ws_bytes < need) return fail(DCB_ERR_WORKSPACE, "dcb_bn_train_fwd: workspace %zu B < required %zu B", ws_bytes, need);
   p.totals = reinterpret_cast<double*>(ws);      // 64-bit fixed-point totals, zero on entry (see release_totals)
-  {
-    const cudaError_t le = launch_k(bn_train_fwd_kernel<T, VEC, POOL>, grid, 256, smem, st, policy(DCB_POLICY_PDL) != 0, p);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of bn_train_fwd_kernel failed: %s", cudaGetErrorString(le));
-  }
-  g_launches += 1;
+  if (int e = launch(bn_train_fwd_kernel<T, VEC, POOL>, "bn_train_fwd_kernel", grid, 256, smem, 0, st, policy(DCB_POLICY_PDL) != 0, 0, p))
+    return e;
   note_kernel(VEC == 8 ? (POOL ? "bn_train_fwd_v8_pool" : "bn_train_fwd_v8") : (POOL ? "bn_train_fwd_v4_pool" : "bn_train_fwd_v4"));
   return DCB_OK;
 }
@@ -952,9 +923,9 @@ static int launch_bn_fwd_sums(BnFwdParams& p, cudaStream_t st) {
   long long grid = (p.M + 8LL * rows_par - 1) / (8LL * rows_par);
   if (grid > 8LL * sm_count()) grid = 8LL * sm_count();
   if (grid < 1) grid = 1;
-  const cudaError_t le = launch_k(bn_train_fwd_kernel<T, VEC, POOL, true>, (int)grid, 256, smem, st, policy(DCB_POLICY_PDL) != 0, p);
-  if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of bn_train_fwd_kernel (sums) failed: %s", cudaGetErrorString(le));
-  g_launches += 1;
+  if (int e = launch(bn_train_fwd_kernel<T, VEC, POOL, true>, "bn_train_fwd_kernel (sums)", (int)grid, 256, smem, 0, st,
+                     policy(DCB_POLICY_PDL) != 0, 0, p))
+    return e;
   note_kernel(VEC == 8 ? (POOL ? "bn_train_fwd_sums_v8_pool" : "bn_train_fwd_sums_v8")
                        : (POOL ? "bn_train_fwd_sums_v4_pool" : "bn_train_fwd_sums_v4"));
   return DCB_OK;
@@ -998,11 +969,8 @@ static int launch_bn_bwd(BnBwdParams& p, void* ws, size_t ws_bytes, cudaStream_t
   const size_t need = 2 * (size_t)p.C * sizeof(long long);
   if (!ws || ws_bytes < need) return fail(DCB_ERR_WORKSPACE, "dcb_bn_train_bwd: workspace %zu B < required %zu B", ws_bytes, need);
   p.totals = reinterpret_cast<double*>(ws);      // 64-bit fixed-point totals, zero on entry (see release_totals)
-  {
-    const cudaError_t le = launch_k(bn_train_bwd_kernel<T, VEC>, grid, 256, smem, st, policy(DCB_POLICY_PDL) != 0, p);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of bn_train_bwd_kernel failed: %s", cudaGetErrorString(le));
-  }
-  g_launches += 1;
+  if (int e = launch(bn_train_bwd_kernel<T, VEC>, "bn_train_bwd_kernel", grid, 256, smem, 0, st, policy(DCB_POLICY_PDL) != 0, 0, p))
+    return e;
   note_kernel(VEC == 8 ? (p.gpix ? "bn_train_bwd_v8_rank1" : "bn_train_bwd_v8") : (p.gpix ? "bn_train_bwd_v4_rank1" : "bn_train_bwd_v4"));
   return DCB_OK;
 }

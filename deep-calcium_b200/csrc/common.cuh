@@ -7,6 +7,8 @@
 #include <cstdio>
 #include <cstdarg>
 #include <cstring>
+#include <map>
+#include <mutex>
 
 #include "../../include/dcb200.h"
 
@@ -38,44 +40,61 @@ int sm_count();   // cached multiprocessor count of the current device
 int policy(int key);               // current value of a dcb_policy_key (dcb_set_policy)
 void note_kernel(const char* name); // records the contraction kernel a call dispatched to (dcb_last_kernel)
 
+extern unsigned long long g_launches;   // kernels launched by the library (dcb_launch_count)
+
+// Sets a kernel's function attributes once, before its first launch that needs them: the maximum dynamic shared memory
+// (smem_max > 0: above the default 48 KB) and, for clusters of more than the portable 8 CTAs, the non-portable size.
+inline cudaError_t prepare_kernel(const void* kernel, int smem_max, int cluster) {
+  static std::mutex mu;
+  static std::map<const void*, int> applied;     // per kernel: 1 = shared-memory limit set, 2 = non-portable clusters allowed
+  const int want = (smem_max > 0 ? 1 : 0) | (cluster > 8 ? 2 : 0);
+  std::lock_guard<std::mutex> lock(mu);
+  int& have = applied[kernel];
+  cudaError_t e = cudaSuccess;
+  if (want & ~have & 1) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
+  if (e == cudaSuccess && (want & ~have & 2)) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+  if (e == cudaSuccess) have |= want;
+  return e;
+}
+
 // Kernel launch with optional PROGRAMMATIC DEPENDENT LAUNCH (policy DCB_POLICY_PDL): the kernel may be scheduled while
 // its predecessor in the stream is still running, executes its prologue (barrier / TMEM set-up, tensor-map prefetch,
 // loads of STATIC data such as weights) and blocks in pdl_wait() until the predecessor has completed and its writes
 // are visible.  Only kernels that call pdl_wait() before touching anything an earlier kernel of the stream produces
-// may be launched through this helper with pdl = true.  Captured into CUDA graphs as programmatic dependency edges.
+// may be launched with pdl = true.  Captured into CUDA graphs as programmatic dependency edges.
+// cluster > 0: the kernel runs as thread-block clusters of `cluster` CTAs (grid must be a multiple of it).
+// Counts the launch in g_launches; a failure is reported through fail(DCB_ERR_CUDA) with the kernel's name.
 template <typename... ExpTypes, typename... ActTypes>
-static inline cudaError_t launch_k(void (*kernel)(ExpTypes...), int grid, int block, size_t smem, cudaStream_t st, bool pdl,
-                                   ActTypes&&... args) {
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)grid, 1, 1); cfg.blockDim = dim3((unsigned)block, 1, 1);
-  cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<ExpTypes>(args)...);
-}
-
-// the same for a kernel that runs as thread-block clusters of `cluster_x` CTAs (grid must be a multiple of it)
-template <typename... ExpTypes, typename... ActTypes>
-static inline cudaError_t launch_kc(void (*kernel)(ExpTypes...), int grid, int block, size_t smem, cudaStream_t st, bool pdl,
-                                    int cluster_x, ActTypes&&... args) {
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)grid, 1, 1); cfg.blockDim = dim3((unsigned)block, 1, 1);
-  cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = (unsigned)cluster_x; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = pdl ? 2 : 1;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<ExpTypes>(args)...);
+static inline int launch(void (*kernel)(ExpTypes...), const char* name, int grid, int block, size_t smem, int smem_max,
+                         cudaStream_t st, bool pdl, int cluster, ActTypes&&... args) {
+  cudaError_t e = prepare_kernel(reinterpret_cast<const void*>(kernel), smem_max, cluster);
+  if (e == cudaSuccess) {
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3((unsigned)grid, 1, 1); cfg.blockDim = dim3((unsigned)block, 1, 1);
+    cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cudaLaunchAttribute at[2];
+    unsigned n = 0;
+    if (cluster > 0) {
+      at[n].id = cudaLaunchAttributeClusterDimension;
+      at[n].val.clusterDim.x = (unsigned)cluster; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
+      ++n;
+    }
+    if (pdl) {
+      at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+      at[n].val.programmaticStreamSerializationAllowed = 1;
+      ++n;
+    }
+    cfg.attrs = at; cfg.numAttrs = n;
+    e = cudaLaunchKernelEx(&cfg, kernel, static_cast<ExpTypes>(args)...);
+  }
+  if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(e));
+  g_launches += 1;
+  return DCB_OK;
 }
 
 // ---- device helpers ----
-// programmatic dependent launch (see launch_k): let the next kernel of the stream start its prologue / wait for the
+// programmatic dependent launch (see launch): let the next kernel of the stream start its prologue / wait for the
 // previous kernel's completion.  Both are no-ops for a kernel launched without the attribute.
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }

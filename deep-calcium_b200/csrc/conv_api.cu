@@ -6,7 +6,6 @@
 #include <cuda_fp16.h>
 
 namespace dcb {
-extern unsigned long long g_launches;
 
 void geom_conv3x3(TapGeom& g, int N, int H, int W);
 void geom_convT_fwd(TapGeom& g, int N, int h, int w);

@@ -5,7 +5,6 @@
 #include "stats_epilogue.cuh"
 
 namespace dcb {
-extern unsigned long long g_launches;
 void launch_reduce_splits(const float* part, int splits, size_t n, float* out, cudaStream_t st);
 
 // v2 (round 2).  The first version kept the weights in shared memory and was bound by the shared-memory pipe (ncu: l1tex
@@ -266,26 +265,22 @@ static int launch_c1_fwd(const float* x, int N, int H, int W, const float* w, in
   auto tiles = [&](int tw) { return (long long)N * cdiv(H, 16) * cdiv(W, tw); };
   auto grid_for = [&](long long t) { const long long cap = 2LL * sm_count(); return (int)(t < cap ? t : cap); };
   const bool pdl = policy(DCB_POLICY_PDL) != 0;
-  cudaError_t le = cudaSuccess;
   if (stats_done) *stats_done = 0;
   if (stat_sums && Cout == 32) {
-    le = launch_k(conv3x3_c1_fwd_kernel<T, 32, true>, grid_for(tiles(64)), 256, 0, st, pdl, x, N, H, W, w, scale, shift, relu, out,
-                  stat_sums);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of conv3x3_c1_fwd_kernel (stats) failed: %s", cudaGetErrorString(le));
-    g_launches += 1;
+    if (int e = launch(conv3x3_c1_fwd_kernel<T, 32, true>, "conv3x3_c1_fwd_kernel (stats)", grid_for(tiles(64)), 256, 0, 0, st, pdl, 0,
+                       x, N, H, W, w, scale, shift, relu, out, stat_sums))
+      return e;
     if (stats_done) *stats_done = 1;
     return DCB_OK;
   }
+  const char* name = "conv3x3_c1_fwd_kernel";
   switch (Cout) {
-    case 8: le = launch_k(conv3x3_c1_fwd_kernel<T, 8>, grid_for(tiles(256)), 256, 0, st, pdl, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr); break;
-    case 16: le = launch_k(conv3x3_c1_fwd_kernel<T, 16>, grid_for(tiles(128)), 256, 0, st, pdl, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr); break;
-    case 32: le = launch_k(conv3x3_c1_fwd_kernel<T, 32>, grid_for(tiles(64)), 256, 0, st, pdl, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr); break;
-    case 64: le = launch_k(conv3x3_c1_fwd_kernel<T, 64>, grid_for(tiles(32)), 256, 0, st, pdl, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr); break;
+    case 8: return launch(conv3x3_c1_fwd_kernel<T, 8>, name, grid_for(tiles(256)), 256, 0, 0, st, pdl, 0, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr);
+    case 16: return launch(conv3x3_c1_fwd_kernel<T, 16>, name, grid_for(tiles(128)), 256, 0, 0, st, pdl, 0, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr);
+    case 32: return launch(conv3x3_c1_fwd_kernel<T, 32>, name, grid_for(tiles(64)), 256, 0, 0, st, pdl, 0, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr);
+    case 64: return launch(conv3x3_c1_fwd_kernel<T, 64>, name, grid_for(tiles(32)), 256, 0, 0, st, pdl, 0, x, N, H, W, w, scale, shift, relu, out, (long long*)nullptr);
     default: return fail(DCB_ERR_UNSUPPORTED, "dcb_conv3x3_c1_fwd: Cout=%d unsupported (8,16,32,64)", Cout);
   }
-  if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of conv3x3_c1_fwd_kernel failed: %s", cudaGetErrorString(le));
-  g_launches += 1;
-  return DCB_OK;
 }
 
 extern "C" int dcb_conv3x3_c1_fwd(int dtype, const float* x, int N, int H, int W, const float* w, int Cout,

@@ -7,7 +7,6 @@
 #include "elementwise.cuh"
 
 namespace dcb {
-extern unsigned long long g_launches;
 
 static inline int ew_grid(long long work_items, int block) {
   long long g = (work_items + block - 1) / block;
@@ -1032,13 +1031,10 @@ extern "C" int dcb_pool_bwd_add(int dtype, const float* skipgrad, int lds, int o
   DCB_CHECK_ARG(y && pooled && dpool && out && N > 0 && H % 2 == 0 && W % 2 == 0 && C % 4 == 0, "dcb_pool_bwd_add: bad arguments");
   DCB_CHECK_ARG(!skipgrad || (lds % 4 == 0 && offs % 4 == 0 && offs + C <= lds), "dcb_pool_bwd_add: bad skip-gradient view");
   DISPATCH_T(dtype, {
-    const cudaError_t le = launch_k(pool_bwd_add_kernel<T>, ew_grid((long long)N * (H / 2) * (W / 2) * (C / 4), 256), 256, 0,
-                                    (cudaStream_t)stream, policy(DCB_POLICY_PDL) != 0, (const float*)skipgrad, lds, offs, (const T*)y,
-                                    (const T*)pooled, (const float*)dpool, N, H, W, C, (float*)out);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of pool_bwd_add_kernel failed: %s", cudaGetErrorString(le));
+    return launch(pool_bwd_add_kernel<T>, "pool_bwd_add_kernel", ew_grid((long long)N * (H / 2) * (W / 2) * (C / 4), 256), 256, 0, 0,
+                  (cudaStream_t)stream, policy(DCB_POLICY_PDL) != 0, 0, (const float*)skipgrad, lds, offs, (const T*)y,
+                  (const T*)pooled, (const float*)dpool, N, H, W, C, (float*)out);
   })
-  g_launches += 1;
-  return DCB_OK;
 }
 
 extern "C" int dcb_head_fwd(int dtype, const void* x, long long M, int C, const float* w, const float* b, float* logit,
@@ -1101,24 +1097,17 @@ static int launch_make_batch(int dtype, const float* s, int hs, int ws, int S, c
                              int tile_first, int n_tiles, int first, int count, void* out, dcb_stream_t stream) {
   const bool pdl = policy(DCB_POLICY_PDL) != 0;
   DISPATCH_T(dtype, {
-    const cudaError_t le = launch_k(tile_make_batch_kernel<T>, ew_grid((long long)n_tiles * count * S * S, 256), 256, 0,
-                                    (cudaStream_t)stream, pdl, s, hs, ws, S, oy, ox, n_tx, tile_first, n_tiles, first, count,
-                                    (T*)out);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tile_make_batch_kernel failed: %s", cudaGetErrorString(le));
+    return launch(tile_make_batch_kernel<T>, "tile_make_batch_kernel", ew_grid((long long)n_tiles * count * S * S, 256), 256, 0, 0,
+                  (cudaStream_t)stream, pdl, 0, s, hs, ws, S, oy, ox, n_tx, tile_first, n_tiles, first, count, (T*)out);
   })
-  g_launches += 1;
-  return DCB_OK;
 }
 
 static int launch_combine(const float* probs, int S, int hs, int ws, const int* oy, const int* ox, const int* cy,
                           const int* cx, int n_ty, int n_tx, int tile_first, int n_tiles, float threshold, int n_aug,
                           double* act, uint8_t* mask, dcb_stream_t stream) {
-  const cudaError_t le = launch_k(tile_combine_kernel, ew_grid((long long)n_tiles * S * S, 256), 256, 0, (cudaStream_t)stream,
-                                  policy(DCB_POLICY_PDL) != 0, probs, S, hs, ws, oy, ox, cy, cx, n_ty, n_tx, tile_first,
-                                  n_tiles, threshold, n_aug, act, mask);
-  if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tile_combine_kernel failed: %s", cudaGetErrorString(le));
-  g_launches += 1;
-  return DCB_OK;
+  return launch(tile_combine_kernel, "tile_combine_kernel", ew_grid((long long)n_tiles * S * S, 256), 256, 0, 0, (cudaStream_t)stream,
+                policy(DCB_POLICY_PDL) != 0, 0, probs, S, hs, ws, oy, ox, cy, cx, n_ty, n_tx, tile_first, n_tiles, threshold,
+                n_aug, act, mask);
 }
 
 extern "C" int dcb_tta_make_batch(int dtype, const float* s, int hs, int ws, int S, int first, int count, void* out,

@@ -14,7 +14,6 @@
 #include "common.cuh"
 
 namespace dcb {
-extern unsigned long long g_launches;
 
 __device__ __forceinline__ unsigned long long peer_ld_acquire(const unsigned long long* p) {
   unsigned long long v;

@@ -335,7 +335,6 @@ static int default_splits(int T, long long P, int variant) {
   return (int)s;
 }
 
-extern unsigned long long g_launches;
 
 }  // namespace dcb
 

@@ -20,7 +20,6 @@
 #include "elementwise.cuh"
 
 namespace dcb {
-extern unsigned long long g_launches;
 
 namespace {
 

@@ -7,7 +7,6 @@
 #include "tapgeom.h"
 
 namespace dcb {
-extern unsigned long long g_launches;
 
 constexpr int FM = 64, FN = 64, FK = 16;
 

@@ -23,7 +23,6 @@
 #include "tapgeom.h"
 
 namespace dcb {
-extern unsigned long long g_launches;
 using namespace tc;
 
 constexpr int TC_BM = 128;          // pixels per tile (= UMMA M, one TMEM lane per pixel)
@@ -1964,17 +1963,14 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// bf16 tensor map; dims/strides innermost first; strides[i] is the byte stride of dim i+1
-static thread_local int t_map_f16 = 0;   // element format of the maps built by the current call (set by the run_tc_* entry points)
-static int make_map(CUtensorMap* out, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                    const uint32_t* box, int swizzle_bytes_in) {
-  const int swizzle_bytes = swizzle_bytes_in;
-  const int f16 = t_map_f16;
-  typedef std::tuple<const void*, int, std::vector<uint64_t>, std::vector<uint64_t>, std::vector<uint32_t>, int> Key;
+// 16-bit tensor map (f16: fp16 elements, else bf16); dims/strides innermost first; strides[i] is the byte stride of dim i+1
+static int make_map(CUtensorMap* out, int f16, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                    const uint32_t* box, int swizzle_bytes) {
+  typedef std::tuple<const void*, int, std::vector<uint64_t>, std::vector<uint64_t>, std::vector<uint32_t>, int, int> Key;
   static std::map<Key, CUtensorMap> cache;
   static std::mutex mu;
   Key key(ptr, rank, std::vector<uint64_t>(dims, dims + rank), std::vector<uint64_t>(strides_bytes, strides_bytes + rank - 1),
-          std::vector<uint32_t>(box, box + rank), swizzle_bytes + (f16 ? 100000 : 0));
+          std::vector<uint32_t>(box, box + rank), swizzle_bytes, f16);
   std::lock_guard<std::mutex> lock(mu);
   auto it = cache.find(key);
   if (it != cache.end()) { *out = it->second; return DCB_OK; }
@@ -1999,6 +1995,41 @@ static int make_map(CUtensorMap* out, const void* ptr, int rank, const uint64_t*
   return DCB_OK;
 }
 
+// The four views the kernels read and write.  `pitch` is the channel stride of a pixel (>= C: a channel slice of a
+// wider tensor).
+// NHWC tensor [N][H][W][C], boxes of {bc channels, bw columns, bh rows, bn images}
+static int map_nhwc(CUtensorMap* m, int f16, const void* ptr, int N, int H, int W, int C, int pitch, uint32_t bc, uint32_t bw,
+                    uint32_t bh, uint32_t bn, int swz) {
+  const uint64_t dims[4] = {(uint64_t)C, (uint64_t)W, (uint64_t)H, (uint64_t)N};
+  const uint64_t str[3] = {(uint64_t)pitch * 2, (uint64_t)W * pitch * 2, (uint64_t)H * W * pitch * 2};
+  const uint32_t box[4] = {bc, bw, bh, bn};
+  return make_map(m, f16, ptr, 4, dims, str, box, swz);
+}
+// NHWC tensor with the image and row axes merged: [rows = N*H][W][C], boxes of {bc, bw, bh rows}
+static int map_rows(CUtensorMap* m, int f16, const void* ptr, long long rows, int W, int C, uint32_t bc, uint32_t bw, uint32_t bh,
+                    int swz) {
+  const uint64_t dims[3] = {(uint64_t)C, (uint64_t)W, (uint64_t)rows};
+  const uint64_t str[2] = {(uint64_t)C * 2, (uint64_t)W * C * 2};
+  const uint32_t box[3] = {bc, bw, bh};
+  return make_map(m, f16, ptr, 3, dims, str, box, swz);
+}
+// sub-pixel view of a [N][2h][2w][C] tensor: [rows = N*h][a = 2][w][b = 2][C] -> innermost first {C, b, w, a, rows};
+// boxes of {bc, 1, bw, 1, bh}: bw pixels of one (a, b) sub-position in each of bh rows
+static int map_subpixel(CUtensorMap* m, int f16, const void* ptr, long long rows, int w, int C, int pitch, uint32_t bc, uint32_t bw,
+                        uint32_t bh, int swz) {
+  const uint64_t dims[5] = {(uint64_t)C, 2, (uint64_t)w, 2, (uint64_t)rows};
+  const uint64_t str[4] = {(uint64_t)pitch * 2, (uint64_t)2 * pitch * 2, (uint64_t)2 * w * pitch * 2, (uint64_t)4 * w * pitch * 2};
+  const uint32_t box[5] = {bc, 1, bw, 1, bh};
+  return make_map(m, f16, ptr, 5, dims, str, box, swz);
+}
+// weight matrix [rows][K], boxes of {bk, brows}
+static int map_weights(CUtensorMap* m, int f16, const void* ptr, int K, int rows, uint32_t bk, uint32_t brows, int swz) {
+  const uint64_t dims[2] = {(uint64_t)K, (uint64_t)rows};
+  const uint64_t str[1] = {(uint64_t)K * 2};
+  const uint32_t box[2] = {bk, brows};
+  return make_map(m, f16, ptr, 2, dims, str, box, swz);
+}
+
 static int pick_pow2_box(int extent, int maxbox) {
   // power-of-two box <= maxbox covering `extent` with the least padding (ties -> larger box);
   // boxes below 8 are only used when the extent itself is smaller
@@ -2018,6 +2049,9 @@ static int pick_pow2_box(int extent, int maxbox) {
 // (<= 128 always required); 0 disables.  Default chosen from per-layer measurements (profiles/).
 static int swap_min_cout() { return policy(DCB_POLICY_SWAP_MIN_COUT); }
 static bool swap_allowed(int Nout) { return swap_min_cout() > 0 && Nout >= swap_min_cout() && Nout <= 128; }
+
+// maximum dynamic shared memory of each kernel family (cudaFuncAttributeMaxDynamicSharedMemorySize)
+constexpr int TC_SMEM_MAX = 206 * 1024, ST_SMEM_MAX = 224 * 1024, FL_SMEM_MAX = 224 * 1024;
 
 // strip kernel plan for a launch that computes Nsub of the layer's Nout output channels (Nsub < Nout: the layer is
 // run as Nout / Nsub launches because the weights of all channels do not fit next to a useful halo ring);
@@ -2066,17 +2100,17 @@ static bool plan_strip(const TapGeom& g, int C0, int C1, int Nout, int Nsub, boo
   return true;
 }
 
+struct FlatPlan { TcFlatParams p; size_t dyn; int grid; bool stats; };
 
-// flat halo-tile kernel: plan + launch; returns DCB_ERR_UNSUPPORTED (nothing launched) when the layer is not eligible
-static int run_tc_flat(const TapGeom& g, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout, void* out,
-                       const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st, TcStats* stats = nullptr) {
+// flat halo-tile kernel plan; false when the layer is not eligible
+static bool plan_flat(const TapGeom& g, int C0, int C1, int Nout, int out_f32, bool stats, FlatPlan& fp) {
   const int flat_policy = policy(DCB_POLICY_FLAT);
-  if (flat_policy == 0 || g.ntaps != 9 || g.zsub > 1 || g.sy != 1) return DCB_ERR_UNSUPPORTED;
-  if (C0 % 64 != 0 || C1 % 64 != 0 || Nout < 64 || g.GW > 64 || g.GW < 16) return DCB_ERR_UNSUPPORTED;
+  if (flat_policy == 0 || g.ntaps != 9 || g.zsub > 1 || g.sy != 1) return false;
+  if (C0 % 64 != 0 || C1 % 64 != 0 || Nout < 64 || g.GW > 64 || g.GW < 16) return false;
   const int Wp = g.GW + 2;
   const long long positions = (long long)g.GH * Wp;
-  if (positions < 512) return DCB_ERR_UNSUPPORTED;     // tiny maps: too much of a 192..256-position tile would be padding
-  TcFlatParams p;
+  if (positions < 512) return false;     // tiny maps: too much of a 192..256-position tile would be padding
+  TcFlatParams& p = fp.p;
   memset(&p, 0, sizeof(p));
   const size_t stile = out_f32 ? 4096 : 2048;            // per-warp transpose tile of the epilogue
   const size_t budget = 223 * 1024 - 2 * (size_t)FL_WSLOT - FL_QUARTETS * 4 * stile;
@@ -2086,281 +2120,40 @@ static int run_tc_flat(const TapGeom& g, const void* s0, int C0, const void* s1,
     pbuf = ((uint32_t)R * Wp * 128u + 1023u) & ~1023u;
     if (R <= 256 && 2 * (size_t)pbuf <= budget) { NT = cand; break; }
   }
-  if (!NT) return DCB_ERR_UNSUPPORTED;
+  if (!NT) return false;
   // Measured (scripts/one_layer.py, profiles/r1_flat_kernel_ab.txt): the coarse work items (NT positions x 128 channels x all
   // of K) only pay when every SM gets several of them; otherwise the generic kernel's finer tiles balance better.
   {
     const bool force = flat_policy >= 2;
     const long long items = (long long)g.N * ((positions + NT - 1) / NT) * cdiv(Nout, 128);
-    if (!force && items < 4LL * sm_count()) return DCB_ERR_UNSUPPORTED;
+    if (!force && items < 4LL * sm_count()) return false;
   }
   p.N = g.N; p.H = g.GH; p.W = g.GW; p.Wp = Wp; p.C0 = C0; p.C1 = C1; p.nkc = (C0 + C1) / 64;
   p.Cout = Nout; p.mtiles = cdiv(Nout, 128); p.NT = NT; p.ptiles = (int)((positions + NT - 1) / NT); p.R = R;
   p.wrows = Nout < 128 ? Nout : 128; p.pbuf_bytes = pbuf; p.stile = (int)stile;
-  p.relu = relu; p.out_f32 = out_f32; p.out = out; p.scale = scale; p.shift = shift; p.f16 = g.f16;
-  CUtensorMap mA0, mA1, mB;
-  auto mk = [&](CUtensorMap* m, const void* ptr, int C) -> int {
-    uint64_t dims[4] = {(uint64_t)C, (uint64_t)g.IW, (uint64_t)g.IH, (uint64_t)g.N};
-    uint64_t str[3] = {(uint64_t)C * 2, (uint64_t)g.IW * C * 2, (uint64_t)g.IH * g.IW * C * 2};
-    uint32_t box[4] = {64u, (uint32_t)Wp, (uint32_t)R, 1u};
-    return make_map(m, ptr, 4, dims, str, box, 128);
-  };
-  if (int e = mk(&mA0, s0, C0)) return e;
-  if (C1 > 0) { if (int e = mk(&mA1, s1, C1)) return e; } else mA1 = mA0;
-  {
-    const int Ktot = 9 * (C0 + C1);
-    uint64_t dims[2] = {(uint64_t)Ktot, (uint64_t)Nout};
-    uint64_t str[1] = {(uint64_t)Ktot * 2};
-    uint32_t box[2] = {64u, (uint32_t)p.wrows};
-    if (int e = make_map(&mB, B, 2, dims, str, box, 128)) return e;
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_flat_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_flat_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-    if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
-  const size_t dyn = 2 * (size_t)pbuf + 2 * (size_t)FL_WSLOT + FL_QUARTETS * 4 * stile + 1024;
+  p.out_f32 = out_f32; p.f16 = g.f16;
+  fp.dyn = 2 * (size_t)pbuf + 2 * (size_t)FL_WSLOT + FL_QUARTETS * 4 * stile + 1024;
   const int items = p.N * p.ptiles * p.mtiles;
-  int grid = items < sm_count() ? items : sm_count();
+  fp.grid = items < sm_count() ? items : sm_count();
+  fp.stats = false;
   // The flat kernel is bound by its four epilogue warps (one 32 x 32 transpose per 32 pixels); the statistics add ~70 % to
   // that loop (measured 28 -> 47 us on the 64 -> 64 layer of a 32 x 64^2 batch, profiles/r2_stats_epilogue_bench.txt) - more
   // than the BatchNorm pass they save.  Only on request (policy fused_bn = 3, the tests).
-  if (stats && !out_f32 && stats->sums && policy(DCB_POLICY_FUSED_BN) >= 3) {
+  if (stats && !out_f32 && policy(DCB_POLICY_FUSED_BN) >= 3) {
     // every CTA keeps one channel tile (its threads accumulate one channel each)
-    const int gs = grid - grid % p.mtiles;
-    if (gs >= p.mtiles) {
-      p.stat_sums = stats->sums;
-      const cudaError_t le = launch_k(tapgemm_tc_flat_kernel<true>, gs, FL_THREADS, dyn, st, policy(DCB_POLICY_PDL) != 0, mA0, mA1, mB, p);
-      if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_flat_kernel (stats) failed: %s", cudaGetErrorString(le));
-      g_launches += 1;
-      stats->done = 1;
-      note_kernel("flat_stats");
-      return DCB_OK;
-    }
+    const int gs = fp.grid - fp.grid % p.mtiles;
+    if (gs >= p.mtiles) { fp.grid = gs; fp.stats = true; }
   }
-  {
-    const cudaError_t le = launch_k(tapgemm_tc_flat_kernel<false>, grid, FL_THREADS, dyn, st, policy(DCB_POLICY_PDL) != 0, mA0, mA1, mB, p);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_flat_kernel failed: %s", cudaGetErrorString(le));
-  }
-  g_launches += 1;
-  note_kernel("flat");
-  return DCB_OK;
+  return true;
 }
 
-static int run_tc_generic(const TapGeom& g, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout, void* out,
-                          int out_pitch, const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st,
-                          void* pool_out = nullptr, TcStats* stats = nullptr);
+struct GenericPlan { TcFwdParams p; size_t dyn; int grid; bool pool, stats; };
 
-// fuse != nullptr: the caller wants the head and/or the 2x2 max-pool computed in the conv epilogue; returns
-// DCB_ERR_UNSUPPORTED (without launching) when this layer shape cannot take the fused path.
-int run_tc_fwd(const TapGeom& g, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout, void* out,
-               const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st, const TcFusion* fuse, TcStats* stats) {
-  t_map_f16 = g.f16;
-  if (stats) stats->done = 0;
-  if (stats && (fuse || out_f32)) return fail(DCB_ERR_INVALID_ARGUMENT, "batch statistics: plain 16-bit forward only");
-  // Small outputs keep the channel-slab BatchNorm kernel, which takes statistics and applies them in ~7 us (2 MB) - less
-  // than the one-pass kernel plus the epilogue's extra work (measured gate; policy fused_bn = 3 = wherever available)
-  if (stats && policy(DCB_POLICY_FUSED_BN) < 3 &&
-      (long long)g.N * g.OH * g.OW * Nout * 2 < (4LL << 20))
-    stats = nullptr;
-  if (C0 % 32 != 0 || C1 % 32 != 0 || Nout % 32 != 0)
-    return fail(DCB_ERR_UNSUPPORTED, "bf16 tensor-core path needs channel counts that are multiples of 32 "
-                "(got C0=%d C1=%d Cout=%d); use the fp32 check mode for other widths", C0, C1, Nout);
-  if (Nout > 512) {
-    // wide outputs (the dgrad of a 768-channel concat in the 'upsampling' graph): slices of <= 512 channels through the
-    // generic kernel, each writing its channel range of the full-pitch output
-    if (fuse) return fail(DCB_ERR_UNSUPPORTED, "fused epilogue not available for this layer");
-    const size_t esz = out_f32 ? 4 : 2;
-    const size_t wrow = (size_t)g.ntaps * (C0 + C1) * (g.zsub > 1 ? g.zsub : 1);
-    if (g.zsub > 1) return fail(DCB_ERR_UNSUPPORTED, "bf16 convT with more than 512 output channels is not built");
-    for (int n0 = 0; n0 < Nout; n0 += 512) {
-      const int ns = Nout - n0 < 512 ? Nout - n0 : 512;
-      if (int e = run_tc_generic(g, s0, C0, s1, C1, reinterpret_cast<const __nv_bfloat16*>(B) + (size_t)n0 * wrow, ns,
-                                 reinterpret_cast<uint8_t*>(out) + (size_t)n0 * esz, Nout, scale ? scale + n0 : nullptr,
-                                 shift ? shift + n0 : nullptr, relu, out_f32, st))
-        return e;
-    }
-    return DCB_OK;
-  }
-  {
-    TcStripParams sp;
-    size_t dyn = 0;
-    const bool fused = fuse != nullptr;
-    if (fused && out_f32) return fail(DCB_ERR_UNSUPPORTED, "fused epilogue not available for this layer");
-    // a pool-only fusion that the strip kernel cannot take (more than 64 output channels, narrow images) goes to the
-    // generic kernel's pooled epilogue
-    const bool pool_only = fused && fuse->pool_out && !fuse->head_kernel;
-    const bool strip_stats = stats && stats->sums && plan_strip(g, C0, C1, Nout, Nout, false, sp, dyn, true);
-    bool strip_ok = strip_stats || (!(fused && fuse->pool_out && Nout > 64) && plan_strip(g, C0, C1, Nout, Nout, fused, sp, dyn));
-    const bool no_nsplit = !policy(DCB_POLICY_NSPLIT);
-    if (!strip_ok && !fused && !no_nsplit && Nout == 64) strip_ok = plan_strip(g, C0, C1, Nout, 32, fused, sp, dyn);
-    if (fused && !strip_ok) {
-      if (pool_only) return run_tc_generic(g, s0, C0, s1, C1, B, Nout, out, Nout, scale, shift, relu, out_f32, st, fuse->pool_out);
-      return fail(DCB_ERR_UNSUPPORTED, "fused epilogue not available for this layer");
-    }
-    if (strip_ok) {
-      sp.relu = relu; sp.out_f32 = out_f32; sp.out = reinterpret_cast<__nv_bfloat16*>(out); sp.scale = scale; sp.shift = shift;
-      sp.f16 = g.f16;
-      sp.need_y = 1;
-      if (fused) {
-        sp.head_kernel = fuse->head_kernel; sp.head_bias = fuse->head_bias; sp.logit = fuse->logit; sp.prob = fuse->prob;
-        sp.need_y = fuse->need_y; sp.pool_out = reinterpret_cast<__nv_bfloat16*>(fuse->pool_out);
-      }
-      CUtensorMap mA0, mA1, mT0, mT1, mB;
-      auto mk = [&](CUtensorMap* m, const void* ptr, int C, uint32_t boxw) -> int {
-        uint64_t dims[4] = {(uint64_t)C, (uint64_t)g.IW, (uint64_t)g.IH, (uint64_t)g.N};
-        uint64_t str[3] = {(uint64_t)C * 2, (uint64_t)g.IW * C * 2, (uint64_t)g.IH * g.IW * C * 2};
-        uint32_t box[4] = {(uint32_t)sp.BK, boxw, 1u, 1u};
-        return make_map(m, ptr, 4, dims, str, box, sp.BK * 2);
-      };
-      const uint32_t mainw = sp.swap ? 256u : 130u;
-      if (int e = mk(&mA0, s0, C0, mainw)) return e;
-      if (int e = mk(&mT0, s0, C0, 2u)) return e;
-      if (C1 > 0) { if (int e = mk(&mA1, s1, C1, mainw)) return e; if (int e = mk(&mT1, s1, C1, 2u)) return e; }
-      else { mA1 = mA0; mT1 = mT0; }
-      {
-        const int Ktot = 9 * (C0 + C1);
-        uint64_t dims[2] = {(uint64_t)Ktot, (uint64_t)Nout};
-        uint64_t str[1] = {(uint64_t)Ktot * 2};
-        uint32_t box[2] = {(uint32_t)sp.BK, (uint32_t)sp.Cout};
-        if (int e = make_map(&mB, B, 2, dims, str, box, sp.BK * 2)) return e;
-      }
-      static bool attr_set_strip = false;
-      if (!attr_set_strip) {
-        cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_strip_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_strip_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_strip_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_strip_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_strip_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-        if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(e));
-        attr_set_strip = true;
-      }
-      const bool pdl = policy(DCB_POLICY_PDL) != 0;
-      // CTA-pair variant of the folded loop (cta_group::2 MMAs): the stacked weights take 5/3 of the single-CTA footprint
-      // per CTA (one region per span shape); used when a ring of at least three row pairs still fits next to them
-      if (sp.fold && !strip_stats && policy(DCB_POLICY_PAIR) && (sp.N * sp.wsegs) % 2 == 0 && sp.H % 2 == 0 && sm_count() >= 2) {
-        const size_t w2 = ((size_t)15 * sp.nkc * sp.Cout * sp.BK * 2 + 1023) & ~(size_t)1023;
-        const size_t budget = 223 * 1024;
-        const size_t rowb = (size_t)sp.nkc * sp.slot_bytes;
-        int ring2 = w2 < budget ? (int)((budget - w2) / rowb) : 0;
-        if (ring2 > ST_MAX_RING) ring2 = ST_MAX_RING;
-        ring2 &= ~1;
-        if (ring2 >= 6) {
-          CUtensorMap mBh;
-          {
-            const int Ktot = 9 * (C0 + C1);
-            uint64_t dims[2] = {(uint64_t)Ktot, (uint64_t)Nout};
-            uint64_t str[1] = {(uint64_t)Ktot * 2};
-            uint32_t box[2] = {(uint32_t)sp.BK, (uint32_t)(sp.Cout / 2)};
-            if (int e = make_map(&mBh, B, 2, dims, str, box, sp.BK * 2)) return e;
-          }
-          static bool attr_set_pair = false;
-          if (!attr_set_pair) {
-            cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_strip2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_strip2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
-            if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(e));
-            attr_set_pair = true;
-          }
-          TcStripParams sp2 = sp;
-          sp2.ring = ring2;
-          const size_t dyn2 = w2 + (size_t)ring2 * rowb + 1024;
-          const long long units2 = (long long)(sp.N * sp.wsegs / 2) * (sp.H / 2);
-          const int pairs = units2 < sm_count() / 2 ? (int)units2 : sm_count() / 2;
-          for (sp2.n0 = 0; sp2.n0 < Nout; sp2.n0 += sp2.Cout) {
-            const cudaError_t le = fused ? launch_kc(tapgemm_tc_strip2_kernel<true>, 2 * pairs, ST_THREADS, dyn2, st, pdl, 2, mA0, mA1, mBh, sp2)
-                                         : launch_kc(tapgemm_tc_strip2_kernel<false>, 2 * pairs, ST_THREADS, dyn2, st, pdl, 2, mA0, mA1, mBh, sp2);
-            if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_strip2_kernel failed: %s", cudaGetErrorString(le));
-            g_launches += 1;
-          }
-          note_kernel(fused ? "strip_pair_fused" : (sp.Cout < Nout ? "strip_pair_nsplit" : "strip_pair"));
-#ifdef DCB_STRIP_TIMING
-          if (getenv("DCB_STRIP_TIMING_PRINT")) {
-            cudaStreamSynchronize(st);
-            static unsigned long long h[148 * 8];
-            cudaMemcpyFromSymbol(h, g_strip_dbg, sizeof(h));
-            double a[8] = {0};
-            for (int b = 0; b < pairs; ++b) for (int q = 0; q < 8; ++q) a[q] += (double)h[b * 8 + q] / pairs;
-            fprintf(stderr, "[strip pair timing] per leader: steps (two halo rows of both CTAs) %.0f | cycles/step: row_full wait %.0f, tempty wait "
-                    "%.0f, issue %.0f, commit %.0f, total %.0f | loop cycles %.0f\n", a[5], a[0] / a[5], a[1] / a[5], a[2] / a[5], a[3] / a[5],
-                    a[4] / a[5], a[6]);
-          }
-#endif
-          return DCB_OK;
-        }
-      }
-      const long long units = (long long)sp.N * sp.wsegs * cdiv(sp.H, sp.gran);
-      const int grid = units < sm_count() ? (int)units : sm_count();
-      if (strip_stats) {
-        sp.n0 = 0; sp.nclu = 1; sp.stat_sums = stats->sums;
-        const cudaError_t le = launch_k(tapgemm_tc_strip_kernel<false, true, true>, grid, ST_THREADS, dyn, st, pdl, mA0, mA1, mT0, mT1, mB, sp);
-        if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_strip_kernel (stats) failed: %s", cudaGetErrorString(le));
-        g_launches += 1;
-        stats->done = 1;
-        note_kernel("strip_fold_stats");
-        return DCB_OK;
-      }
-      // channel-split layer (two groups of output channels): ONE launch of two-CTA clusters that share every halo row
-      // through TMA multicast instead of two launches that each read the whole input
-      if (sp.fold && !fused && Nout == 2 * sp.Cout && sp.nkc % 2 == 0 && policy(DCB_POLICY_NSPLIT) == 1 && sm_count() >= 2) {
-        sp.n0 = 0; sp.nclu = 2;
-        const int parts = units < sm_count() / 2 ? (int)units : sm_count() / 2;
-        const cudaError_t le = launch_kc(tapgemm_tc_strip_kernel<false, true>, 2 * parts, ST_THREADS, dyn, st, pdl, 2, mA0, mA1, mT0, mT1, mB, sp);
-        if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_strip_kernel (cluster) failed: %s", cudaGetErrorString(le));
-        g_launches += 1;
-        note_kernel("strip_fold_nsplit_cluster");
-        return DCB_OK;
-      }
-      sp.nclu = 1;
-      for (sp.n0 = 0; sp.n0 < Nout; sp.n0 += sp.Cout) {          // one launch per group of output channels
-        cudaError_t le;
-        if (fused && sp.fold) le = launch_k(tapgemm_tc_strip_kernel<true, true>, grid, ST_THREADS, dyn, st, pdl, mA0, mA1, mT0, mT1, mB, sp);
-        else if (fused) le = launch_k(tapgemm_tc_strip_kernel<true, false>, grid, ST_THREADS, dyn, st, pdl, mA0, mA1, mT0, mT1, mB, sp);
-        else if (sp.fold) le = launch_k(tapgemm_tc_strip_kernel<false, true>, grid, ST_THREADS, dyn, st, pdl, mA0, mA1, mT0, mT1, mB, sp);
-        else le = launch_k(tapgemm_tc_strip_kernel<false, false>, grid, ST_THREADS, dyn, st, pdl, mA0, mA1, mT0, mT1, mB, sp);
-        if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_strip_kernel failed: %s", cudaGetErrorString(le));
-        g_launches += 1;
-      }
-      note_kernel(sp.fold ? (fused ? "strip_fold_fused" : (sp.Cout < Nout ? "strip_fold_nsplit" : "strip_fold"))
-                          : (sp.swap ? "strip_swap" : (fused ? "strip_fused" : "strip")));
-#ifdef DCB_STRIP_TIMING
-      if (sp.fold && getenv("DCB_STRIP_TIMING_PRINT")) {
-        cudaStreamSynchronize(st);
-        static unsigned long long h[148 * 8];
-        cudaMemcpyFromSymbol(h, g_strip_dbg, sizeof(h));
-        double a[8] = {0};
-        for (int b = 0; b < grid; ++b) for (int q = 0; q < 8; ++q) a[q] += (double)h[b * 8 + q] / grid;
-        static unsigned long long h2[148 * 16];
-        cudaMemcpyFromSymbol(h2, g_strip_dbg2, sizeof(h2));
-        double e[16] = {0};
-        for (int b = 0; b < grid; ++b) for (int q = 0; q < 16; ++q) e[q] += (double)h2[b * 16 + q] / grid;
-        fprintf(stderr, "[strip timing] producer: rows %.0f, row_empty wait %.0f cycles/row | epilogue quartet 0: tiles %.0f, tfull wait %.0f, "
-                "work %.0f (tmem ld %.0f, math+store %.0f) cycles/tile | quartet 1: tiles %.0f, tfull wait %.0f, work %.0f (ld %.0f, math %.0f)\n",
-                e[1], e[0] / e[1], e[3], e[2] / e[3], e[4] / e[3], e[5] / e[3], e[6] / e[3], e[8], e[7] / e[8], e[9] / e[8], e[10] / e[8], e[11] / e[8]);
-        fprintf(stderr, "[strip timing] per CTA: fast rows %.0f | cycles/row: row_full wait %.0f, tempty wait %.0f, issue %.0f, commit %.0f, "
-                "total %.0f | loop cycles %.0f\n", a[5], a[0] / a[5], a[1] / a[5], a[2] / a[5], a[3] / a[5], a[4] / a[5], a[6]);
-      }
-#endif
-      return DCB_OK;
-    }
-  }
-  // A training forward that wants its batch statistics goes to the generic kernel (statistics in the epilogue, +2 us)
-  // rather than to the flat kernel (no statistics at the default policy): what the flat kernel gains on the conv (~20 %
-  // on 64-pixel rows) is less than the separate statistics pass it would leave to the BatchNorm kernel
-  // (scripts/train_time.py flat=0 / 1: 2.589 vs 2.609 ms per step before this rule).
-  if (!(stats && stats->sums && policy(DCB_POLICY_FUSED_BN) == 2)) {
-    const int e = run_tc_flat(g, s0, C0, s1, C1, B, Nout, out, scale, shift, relu, out_f32, st, stats);
-    if (e != DCB_ERR_UNSUPPORTED) return e;
-  }
-  return run_tc_generic(g, s0, C0, s1, C1, B, Nout, out, Nout, scale, shift, relu, out_f32, st, nullptr, stats);
-}
-
-// generic kernel: Nout output channels written with a channel pitch of out_pitch (>= Nout) starting at `out`
-static int run_tc_generic(const TapGeom& g, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout, void* out,
-                          int out_pitch, const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st,
-                          void* pool_out, TcStats* stats) {
-  TcFwdParams p;
+// generic kernel plan for Nout output channels written with a channel pitch of out_pitch (>= Nout); pool: the 2x2
+// max-pooled copy in the epilogue; stats: batch statistics requested.  Returns null, or why the layer is not supported.
+static const char* plan_generic(const TapGeom& g, int C0, int C1, int Nout, int out_pitch, int out_f32, bool pool, bool stats,
+                                GenericPlan& gp) {
+  TcFwdParams& p = gp.p;
   memset(&p, 0, sizeof(p));
   const int ntaps = g.ntaps;
   const bool convT_fwd = g.zsub > 1;
@@ -2371,12 +2164,11 @@ static int run_tc_generic(const TapGeom& g, const void* s0, int C0, const void* 
   for (int t = 0; t < ntaps; ++t) { p.dy[t] = g.dy[t]; p.dx[t] = g.dx[t]; }
   p.C0 = C0; p.C1 = C1;
   p.BK = (C0 % 64 == 0 && C1 % 64 == 0) ? 64 : 32;
-  const int swz = p.BK * 2;
   p.Cz = Nout;
   p.Ntot = convT_fwd ? 4 * Nout : Nout;
   p.OH = g.OH; p.OW = g.OW; p.OC = out_pitch;
   p.osy = g.osy; p.osx = g.osx; p.ody = g.ody; p.odx = g.odx;
-  p.relu = relu; p.out_f32 = out_f32; p.out = reinterpret_cast<__nv_bfloat16*>(out); p.scale = scale; p.shift = shift;
+  p.out_f32 = out_f32;
   p.f16 = g.f16;
   // Swapped orientation for narrow outputs: with <= 128 output channels the normal orientation spends the
   // A-operand read time (128 pixel rows per MMA) on an N of 32..128; swapped, every MMA covers 256 pixels.
@@ -2384,14 +2176,14 @@ static int run_tc_generic(const TapGeom& g, const void* s0, int C0, const void* 
     const long long px = (long long)g.N * g.GH * g.GW;
     // measured (profiles/r1_layer_ab.txt): pays for conv3x3 with 64..128 output channels, not for the 1-tap convT GEMMs
     // the pooled epilogue is cheaper in the pixels-as-M orientation (two epilogue quartets; profiles/r2_pool_ab.txt)
-    p.swap = (p.mode == 0 && !pool_out && !stats && swap_allowed(Nout) && px / 256 * cdiv(p.Ntot, 128) >= sm_count() / 2) ? 1 : 0;
+    p.swap = (p.mode == 0 && !pool && !stats && swap_allowed(Nout) && px / 256 * cdiv(p.Ntot, 128) >= sm_count() / 2) ? 1 : 0;
   }
   const int TM = p.swap ? 256 : TC_BM;
   // ---- M tiling
   if (p.mode == 0) {
     p.bw = pick_pow2_box(g.GW, TM);
     // the pooled epilogue needs whole 2x2 windows inside a tile: rows wide enough for a one-row tile are split in two
-    if (pool_out && p.bw == TM && TM >= 4) p.bw = TM / 2;
+    if (pool && p.bw == TM && TM >= 4) p.bw = TM / 2;
     p.bh = pick_pow2_box(g.GH, TM / p.bw);
     p.bn = TM / (p.bw * p.bh);
     p.tiles_w = cdiv(g.GW, p.bw); p.tiles_h = cdiv(g.GH, p.bh); p.tiles_n = cdiv(g.N, p.bn);
@@ -2401,12 +2193,11 @@ static int run_tc_generic(const TapGeom& g, const void* s0, int C0, const void* 
     p.tiles_w = cdiv(g.GW, p.bw); p.tiles_h = cdiv((long long)g.N * g.GH, p.bh); p.tiles_n = 1;
   }
   const int num_mtiles = p.tiles_w * p.tiles_h * p.tiles_n;
-  if (pool_out) {
-    // pooled epilogue: conv3x3 only, 16-bit outputs, whole 2x2 windows inside every tile
-    if (p.mode != 0 || out_f32 || (g.GH & 1) || (g.GW & 1) || (p.bw & 1) || (p.bh & 1) || (p.swap && p.bw % 32 != 0) || out_pitch != Nout)
-      return fail(DCB_ERR_UNSUPPORTED, "fused max-pool not available for this layer shape");
-    p.pool_out = reinterpret_cast<__nv_bfloat16*>(pool_out);
-  }
+  // pooled epilogue: conv3x3 only, 16-bit outputs, whole 2x2 windows inside every tile
+  if (pool && (p.mode != 0 || out_f32 || (g.GH & 1) || (g.GW & 1) || (p.bw & 1) || (p.bh & 1) || (p.swap && p.bw % 32 != 0) ||
+               out_pitch != Nout))
+    return "fused max-pool not available for this layer shape";
+  gp.pool = pool;
   // ---- N tiling: largest tile that still gives every SM work
   // an N tile may span several convT sub-positions (the epilogue resolves them per 32-column block)
   // Cost model from the issue-rate probes (profiles/r1_umma_rate_probe.log): one M=128 MMA occupies the tensor pipe for
@@ -2430,98 +2221,299 @@ static int run_tc_generic(const TapGeom& g, const void* s0, int C0, const void* 
   // scattered 64-byte runs saturate the LSU pipe as plain stores (profiles/r2_convT_ncu.txt).  The conv3x3 layers on this
   // kernel are operand-traffic bound and lose more from the smaller stage ring than the stores gain (measured; policy 2
   // = TMA stores there too).
-  const bool with_stats = stats && !pool_out && !out_f32 && p.mode != 2 && out_pitch == Nout && stats->sums;
-  p.tma_store = (!p.swap && !out_f32 && !pool_out && !with_stats && p.mode != 2 &&
+  const bool with_stats = stats && !pool && !out_f32 && p.mode != 2 && out_pitch == Nout;
+  p.tma_store = (!p.swap && !out_f32 && !pool && !with_stats && p.mode != 2 &&
                  (policy(DCB_POLICY_TMA_STORE) >= 2 || (policy(DCB_POLICY_TMA_STORE) == 1 && p.mode == 1))) ? 1 : 0;
   const size_t staging = p.tma_store ? 2 * 16384 : 0;
   int stages = (int)((200 * 1024 - staging) / stage_bytes);
   if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
-  if (stages < 2) return fail(DCB_ERR_UNSUPPORTED, "tile does not fit shared memory");
+  if (stages < 2) return "tile does not fit shared memory";
   p.stages = stages;
-  const size_t dyn_smem = stages * stage_bytes + staging + 1024;
-
-  // ---- tensor maps
-  CUtensorMap mA0, mA1, mB;
-  auto make_src_map = [&](CUtensorMap* m, const void* ptr, int C) -> int {
-    if (p.mode == 0) {
-      uint64_t dims[4] = {(uint64_t)C, (uint64_t)g.IW, (uint64_t)g.IH, (uint64_t)g.N};
-      uint64_t str[3] = {(uint64_t)C * 2, (uint64_t)g.IW * C * 2, (uint64_t)g.IH * g.IW * C * 2};
-      uint32_t box[4] = {(uint32_t)p.BK, (uint32_t)p.bw, (uint32_t)p.bh, (uint32_t)p.bn};
-      return make_map(m, ptr, 4, dims, str, box, swz);
-    } else if (p.mode == 1) {
-      uint64_t dims[3] = {(uint64_t)C, (uint64_t)g.IW, (uint64_t)g.N * g.IH};
-      uint64_t str[2] = {(uint64_t)C * 2, (uint64_t)g.IW * C * 2};
-      uint32_t box[3] = {(uint32_t)p.BK, (uint32_t)p.bw, (uint32_t)p.bh};
-      return make_map(m, ptr, 3, dims, str, box, swz);
-    } else {
-      // dy [N][2h][2w][C] viewed as [N*h][a=2][w][b=2][C] -> innermost first {C, b, w, a, N*h}
-      uint64_t dims[5] = {(uint64_t)C, 2, (uint64_t)g.GW, 2, (uint64_t)g.N * g.GH};
-      uint64_t str[4] = {(uint64_t)C * 2, (uint64_t)2 * C * 2, (uint64_t)g.IW * C * 2, (uint64_t)2 * g.IW * C * 2};
-      uint32_t box[5] = {(uint32_t)p.BK, 1, (uint32_t)p.bw, 1, (uint32_t)p.bh};
-      return make_map(m, ptr, 5, dims, str, box, swz);
-    }
-  };
-  if (int e = make_src_map(&mA0, s0, C0)) return e;
-  if (C1 > 0) { if (int e = make_src_map(&mA1, s1, C1)) return e; }
-  else mA1 = mA0;
-  {
-    const int Ktot = ntaps * (C0 + C1);
-    uint64_t dims[2] = {(uint64_t)Ktot, (uint64_t)p.Ntot};
-    uint64_t str[1] = {(uint64_t)Ktot * 2};
-    uint32_t box[2] = {(uint32_t)p.BK, (uint32_t)BN};
-    if (int e = make_map(&mB, B, 2, dims, str, box, swz)) return e;
-  }
-
-  CUtensorMap mO = mB;
-  if (p.tma_store) {
-    if (p.mode == 0) {
-      uint64_t dims[4] = {(uint64_t)Nout, (uint64_t)g.OW, (uint64_t)g.OH, (uint64_t)g.N};
-      uint64_t str[3] = {(uint64_t)out_pitch * 2, (uint64_t)g.OW * out_pitch * 2, (uint64_t)g.OH * g.OW * out_pitch * 2};
-      uint32_t box[4] = {32u, (uint32_t)p.bw, (uint32_t)p.bh, (uint32_t)p.bn};
-      if (int e = make_map(&mO, out, 4, dims, str, box, 64)) return e;
-    } else {
-      // convT fwd: y [N][2h][2w][C] viewed as [N*h][dy][w][dx][C] -> innermost first {C, dx, w, dy, N*h}
-      uint64_t dims[5] = {(uint64_t)Nout, 2, (uint64_t)g.GW, 2, (uint64_t)g.N * g.GH};
-      uint64_t str[4] = {(uint64_t)out_pitch * 2, (uint64_t)2 * out_pitch * 2, (uint64_t)g.OW * out_pitch * 2,
-                         (uint64_t)2 * g.OW * out_pitch * 2};
-      uint32_t box[5] = {32u, 1, (uint32_t)p.bw, 1, (uint32_t)p.bh};
-      if (int e = make_map(&mO, out, 5, dims, str, box, 64)) return e;
-    }
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_fwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 206 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_fwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 206 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(tapgemm_tc_fwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 206 * 1024);
-    if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
+  gp.dyn = stages * stage_bytes + staging + 1024;
   const int num_ntiles = p.swap ? cdiv(p.Ntot, 128) : p.Ntot / BN;
   const int num_tiles = num_mtiles * num_ntiles;
-  int grid = num_tiles < sm_count() ? num_tiles : sm_count();
-  const bool pdl = policy(DCB_POLICY_PDL) != 0;
-  if (with_stats) {
-    // every CTA keeps ONE N tile (its register accumulators are per 32-column block of the tile): the round-robin
-    // schedule tile = blockIdx.x + i * gridDim.x does that when the grid is a multiple of the N-tile count
-    grid -= grid % num_ntiles;
-    if (grid >= num_ntiles) {
-      p.stat_sums = stats->sums;
-      const cudaError_t le = launch_k(tapgemm_tc_fwd_kernel<false, true>, grid, TC_THREADS, dyn_smem, st, pdl, mA0, mA1, mB, mO, p);
-      if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_fwd_kernel (stats) failed: %s", cudaGetErrorString(le));
-      g_launches += 1;
-      stats->done = 1;
-      note_kernel("generic_stats");
-      return DCB_OK;
+  gp.grid = num_tiles < sm_count() ? num_tiles : sm_count();
+  // every CTA keeps ONE N tile (its register accumulators are per 32-column block of the tile): the round-robin
+  // schedule tile = blockIdx.x + i * gridDim.x does that when the grid is a multiple of the N-tile count
+  const int stats_grid = gp.grid - gp.grid % num_ntiles;
+  gp.stats = with_stats && stats_grid >= num_ntiles;
+  if (gp.stats) gp.grid = stats_grid;
+  return nullptr;
+}
+
+// The forward variant of one call and its complete plan (choose_fwd).
+struct FwdPlan {
+  enum Kind { UNSUPPORTED, GENERIC, FLAT, STRIP, STRIP_CLUSTER, STRIP_PAIR } kind;
+  const char* error;        // UNSUPPORTED: why
+  bool fused;               // STRIP / STRIP_PAIR: head and / or pool in the epilogue
+  bool stats;               // the launch also writes the batch statistics
+  int slice;                // GENERIC: output channels per launch (Nout, or 512 for wider outputs)
+  GenericPlan gen;          // GENERIC: plan of the first slice
+  FlatPlan flat;
+  TcStripParams sp;         // STRIP*: parameters of one launch (n0 set per launch)
+  size_t strip_dyn;
+  int strip_grid;
+};
+
+// Which kernel a forward-type call (conv3x3 fwd / dgrad, convT2x2 fwd / dgrad) runs, from the shape, the requested
+// epilogue fusions and statistics, and the dispatch policy.  Reads only policy() and sm_count().
+static FwdPlan choose_fwd(const TapGeom& g, int C0, int C1, int Nout, const TcFusion* fuse, bool stats, int out_f32) {
+  FwdPlan c;
+  memset(&c, 0, sizeof(c));
+  auto unsupported = [&](const char* why) { c.kind = FwdPlan::UNSUPPORTED; c.error = why; return c; };
+  auto generic = [&](int slice, bool pool, bool with_stats) {
+    c.kind = FwdPlan::GENERIC; c.slice = slice;
+    if (const char* why = plan_generic(g, C0, C1, slice, Nout, out_f32, pool, with_stats, c.gen)) return unsupported(why);
+    c.stats = c.gen.stats;
+    return c;
+  };
+  // Small outputs keep the channel-slab BatchNorm kernel, which takes statistics and applies them in ~7 us (2 MB) - less
+  // than the one-pass kernel plus the epilogue's extra work (measured gate; policy fused_bn = 3 = wherever available)
+  if (stats && policy(DCB_POLICY_FUSED_BN) < 3 &&
+      (long long)g.N * g.OH * g.OW * Nout * 2 < (4LL << 20))
+    stats = false;
+  const bool fused = fuse != nullptr;
+  if (Nout > 512) {
+    // wide outputs (the dgrad of a 768-channel concat in the 'upsampling' graph): slices of <= 512 channels through the
+    // generic kernel, each writing its channel range of the full-pitch output
+    if (fused) return unsupported("fused epilogue not available for this layer");
+    if (g.zsub > 1) return unsupported("bf16 convT with more than 512 output channels is not built");
+    return generic(512, false, false);
+  }
+  if (fused && out_f32) return unsupported("fused epilogue not available for this layer");
+  // a pool-only fusion that the strip kernel cannot take (more than 64 output channels, narrow images) goes to the
+  // generic kernel's pooled epilogue
+  const bool pool_only = fused && fuse->pool_out && !fuse->head_kernel;
+  TcStripParams& sp = c.sp;
+  const bool strip_stats = stats && plan_strip(g, C0, C1, Nout, Nout, false, sp, c.strip_dyn, true);
+  bool strip_ok = strip_stats || (!(fused && fuse->pool_out && Nout > 64) && plan_strip(g, C0, C1, Nout, Nout, fused, sp, c.strip_dyn));
+  const bool no_nsplit = !policy(DCB_POLICY_NSPLIT);
+  if (!strip_ok && !fused && !no_nsplit && Nout == 64) strip_ok = plan_strip(g, C0, C1, Nout, 32, fused, sp, c.strip_dyn);
+  if (fused && !strip_ok) {
+    if (pool_only) return generic(Nout, true, false);
+    return unsupported("fused epilogue not available for this layer");
+  }
+  if (strip_ok) {
+    c.fused = fused;
+    // CTA-pair variant of the folded loop (cta_group::2 MMAs): the stacked weights take 5/3 of the single-CTA footprint
+    // per CTA (one region per span shape); used when a ring of at least three row pairs still fits next to them
+    if (sp.fold && !strip_stats && policy(DCB_POLICY_PAIR) && (sp.N * sp.wsegs) % 2 == 0 && sp.H % 2 == 0 && sm_count() >= 2) {
+      const size_t w2 = ((size_t)15 * sp.nkc * sp.Cout * sp.BK * 2 + 1023) & ~(size_t)1023;
+      const size_t budget = 223 * 1024;
+      const size_t rowb = (size_t)sp.nkc * sp.slot_bytes;
+      int ring2 = w2 < budget ? (int)((budget - w2) / rowb) : 0;
+      if (ring2 > ST_MAX_RING) ring2 = ST_MAX_RING;
+      ring2 &= ~1;
+      if (ring2 >= 6) {
+        c.kind = FwdPlan::STRIP_PAIR;
+        sp.ring = ring2;
+        c.strip_dyn = w2 + (size_t)ring2 * rowb + 1024;
+        const long long units2 = (long long)(sp.N * sp.wsegs / 2) * (sp.H / 2);
+        c.strip_grid = 2 * (units2 < sm_count() / 2 ? (int)units2 : sm_count() / 2);
+        return c;
+      }
     }
-    grid = num_tiles < sm_count() ? num_tiles : sm_count();
+    const long long units = (long long)sp.N * sp.wsegs * cdiv(sp.H, sp.gran);
+    c.kind = FwdPlan::STRIP;
+    c.strip_grid = units < sm_count() ? (int)units : sm_count();
+    sp.nclu = 1;
+    if (strip_stats) { c.stats = true; return c; }
+    // channel-split layer (two groups of output channels): ONE launch of two-CTA clusters that share every halo row
+    // through TMA multicast instead of two launches that each read the whole input
+    if (sp.fold && !fused && Nout == 2 * sp.Cout && sp.nkc % 2 == 0 && policy(DCB_POLICY_NSPLIT) == 1 && sm_count() >= 2) {
+      c.kind = FwdPlan::STRIP_CLUSTER;
+      sp.nclu = 2;
+      c.strip_grid = 2 * (units < sm_count() / 2 ? (int)units : sm_count() / 2);
+    }
+    return c;
   }
-  {
-    const cudaError_t le = p.pool_out ? launch_k(tapgemm_tc_fwd_kernel<true, false>, grid, TC_THREADS, dyn_smem, st, pdl, mA0, mA1, mB, mO, p)
-                                      : launch_k(tapgemm_tc_fwd_kernel<false, false>, grid, TC_THREADS, dyn_smem, st, pdl, mA0, mA1, mB, mO, p);
-    if (le != cudaSuccess) return fail(DCB_ERR_CUDA, "launch of tapgemm_tc_fwd_kernel failed: %s", cudaGetErrorString(le));
+  // A training forward that wants its batch statistics goes to the generic kernel (statistics in the epilogue, +2 us)
+  // rather than to the flat kernel (no statistics at the default policy): what the flat kernel gains on the conv (~20 %
+  // on 64-pixel rows) is less than the separate statistics pass it would leave to the BatchNorm kernel
+  // (scripts/train_time.py flat=0 / 1: 2.589 vs 2.609 ms per step before this rule).
+  if (!(stats && policy(DCB_POLICY_FUSED_BN) == 2) && plan_flat(g, C0, C1, Nout, out_f32, stats, c.flat)) {
+    c.kind = FwdPlan::FLAT;
+    c.stats = c.flat.stats;
+    return c;
   }
-  g_launches += 1;
-  note_kernel(p.pool_out ? (p.swap ? "generic_swap_pool" : "generic_pool") : (p.swap ? "generic_swap" : "generic"));
+  return generic(Nout, false, stats);
+}
+
+// dcb_last_kernel() name of a planned forward (tests and profiles/ refer to these names)
+static const char* fwd_kernel_name(const FwdPlan& c) {
+  const TcStripParams& sp = c.sp;
+  switch (c.kind) {
+    case FwdPlan::GENERIC:
+      if (c.stats) return "generic_stats";
+      if (c.gen.pool) return c.gen.p.swap ? "generic_swap_pool" : "generic_pool";
+      return c.gen.p.swap ? "generic_swap" : "generic";
+    case FwdPlan::FLAT: return c.stats ? "flat_stats" : "flat";
+    case FwdPlan::STRIP_PAIR: return c.fused ? "strip_pair_fused" : (sp.Cout < sp.OC ? "strip_pair_nsplit" : "strip_pair");
+    case FwdPlan::STRIP_CLUSTER: return "strip_fold_nsplit_cluster";
+    case FwdPlan::STRIP:
+      if (c.stats) return "strip_fold_stats";
+      return sp.fold ? (c.fused ? "strip_fold_fused" : (sp.Cout < sp.OC ? "strip_fold_nsplit" : "strip_fold"))
+                     : (sp.swap ? "strip_swap" : (c.fused ? "strip_fused" : "strip"));
+    default: return "";
+  }
+}
+
+#ifdef DCB_STRIP_TIMING
+static void print_strip_timing(const FwdPlan& c, cudaStream_t st) {
+  cudaStreamSynchronize(st);
+  if (c.kind == FwdPlan::STRIP_PAIR) {
+    const int pairs = c.strip_grid / 2;
+    static unsigned long long h[148 * 8];
+    cudaMemcpyFromSymbol(h, g_strip_dbg, sizeof(h));
+    double a[8] = {0};
+    for (int b = 0; b < pairs; ++b) for (int q = 0; q < 8; ++q) a[q] += (double)h[b * 8 + q] / pairs;
+    fprintf(stderr, "[strip pair timing] per leader: steps (two halo rows of both CTAs) %.0f | cycles/step: row_full wait %.0f, tempty wait "
+            "%.0f, issue %.0f, commit %.0f, total %.0f | loop cycles %.0f\n", a[5], a[0] / a[5], a[1] / a[5], a[2] / a[5], a[3] / a[5],
+            a[4] / a[5], a[6]);
+    return;
+  }
+  const int grid = c.strip_grid;
+  static unsigned long long h[148 * 8];
+  cudaMemcpyFromSymbol(h, g_strip_dbg, sizeof(h));
+  double a[8] = {0};
+  for (int b = 0; b < grid; ++b) for (int q = 0; q < 8; ++q) a[q] += (double)h[b * 8 + q] / grid;
+  static unsigned long long h2[148 * 16];
+  cudaMemcpyFromSymbol(h2, g_strip_dbg2, sizeof(h2));
+  double e[16] = {0};
+  for (int b = 0; b < grid; ++b) for (int q = 0; q < 16; ++q) e[q] += (double)h2[b * 16 + q] / grid;
+  fprintf(stderr, "[strip timing] producer: rows %.0f, row_empty wait %.0f cycles/row | epilogue quartet 0: tiles %.0f, tfull wait %.0f, "
+          "work %.0f (tmem ld %.0f, math+store %.0f) cycles/tile | quartet 1: tiles %.0f, tfull wait %.0f, work %.0f (ld %.0f, math %.0f)\n",
+          e[1], e[0] / e[1], e[3], e[2] / e[3], e[4] / e[3], e[5] / e[3], e[6] / e[3], e[8], e[7] / e[8], e[9] / e[8], e[10] / e[8], e[11] / e[8]);
+  fprintf(stderr, "[strip timing] per CTA: fast rows %.0f | cycles/row: row_full wait %.0f, tempty wait %.0f, issue %.0f, commit %.0f, "
+          "total %.0f | loop cycles %.0f\n", a[5], a[0] / a[5], a[1] / a[5], a[2] / a[5], a[3] / a[5], a[4] / a[5], a[6]);
+}
+#endif
+
+// strip kernel launches of a STRIP / STRIP_CLUSTER / STRIP_PAIR plan: one launch per group of output channels
+static int launch_strip(const TapGeom& g, FwdPlan& c, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout,
+                        void* out, const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st,
+                        const TcFusion* fuse, TcStats* stats) {
+  TcStripParams& sp = c.sp;
+  sp.relu = relu; sp.out_f32 = out_f32; sp.out = reinterpret_cast<__nv_bfloat16*>(out); sp.scale = scale; sp.shift = shift;
+  sp.f16 = g.f16;
+  sp.need_y = 1;
+  if (c.fused) {
+    sp.head_kernel = fuse->head_kernel; sp.head_bias = fuse->head_bias; sp.logit = fuse->logit; sp.prob = fuse->prob;
+    sp.need_y = fuse->need_y; sp.pool_out = reinterpret_cast<__nv_bfloat16*>(fuse->pool_out);
+  }
+  if (c.stats) sp.stat_sums = stats->sums;
+  const bool pair = c.kind == FwdPlan::STRIP_PAIR;
+  CUtensorMap mA0, mA1, mT0{}, mT1{}, mB;
+  const int swz = sp.BK * 2;
+  const uint32_t mainw = sp.swap ? 256u : 130u;
+  if (int e = map_nhwc(&mA0, g.f16, s0, g.N, g.IH, g.IW, C0, C0, sp.BK, mainw, 1, 1, swz)) return e;
+  if (!pair) { if (int e = map_nhwc(&mT0, g.f16, s0, g.N, g.IH, g.IW, C0, C0, sp.BK, 2, 1, 1, swz)) return e; }
+  if (C1 > 0) {
+    if (int e = map_nhwc(&mA1, g.f16, s1, g.N, g.IH, g.IW, C1, C1, sp.BK, mainw, 1, 1, swz)) return e;
+    if (!pair) { if (int e = map_nhwc(&mT1, g.f16, s1, g.N, g.IH, g.IW, C1, C1, sp.BK, 2, 1, 1, swz)) return e; }
+  } else { mA1 = mA0; mT1 = mT0; }
+  // the pair kernel's CTAs each load half of the weight rows of a launch
+  if (int e = map_weights(&mB, g.f16, B, 9 * (C0 + C1), Nout, sp.BK, pair ? sp.Cout / 2 : sp.Cout, swz)) return e;
+  const bool pdl = policy(DCB_POLICY_PDL) != 0;
+  const int per_launch = c.kind == FwdPlan::STRIP_CLUSTER ? Nout : sp.Cout;   // output channels of one launch
+  for (sp.n0 = 0; sp.n0 < Nout; sp.n0 += per_launch) {
+    int e;
+    if (pair) {
+      e = launch(c.fused ? tapgemm_tc_strip2_kernel<true> : tapgemm_tc_strip2_kernel<false>, "tapgemm_tc_strip2_kernel", c.strip_grid,
+                 ST_THREADS, c.strip_dyn, ST_SMEM_MAX, st, pdl, 2, mA0, mA1, mB, sp);
+    } else {
+      auto* k = c.stats ? tapgemm_tc_strip_kernel<false, true, true>
+                : c.fused ? (sp.fold ? tapgemm_tc_strip_kernel<true, true> : tapgemm_tc_strip_kernel<true, false>)
+                          : (sp.fold ? tapgemm_tc_strip_kernel<false, true> : tapgemm_tc_strip_kernel<false, false>);
+      e = launch(k, "tapgemm_tc_strip_kernel", c.strip_grid, ST_THREADS, c.strip_dyn, ST_SMEM_MAX, st, pdl,
+                 c.kind == FwdPlan::STRIP_CLUSTER ? 2 : 0, mA0, mA1, mT0, mT1, mB, sp);
+    }
+    if (e) return e;
+  }
+#ifdef DCB_STRIP_TIMING
+  if ((pair || (c.kind == FwdPlan::STRIP && !c.stats && sp.fold)) && getenv("DCB_STRIP_TIMING_PRINT")) print_strip_timing(c, st);
+#endif
+  return DCB_OK;
+}
+
+// generic kernel launches of a GENERIC plan: one per slice of c.slice output channels (a narrower last slice is planned
+// here, so c.gen ends as the plan of the last launch)
+static int launch_generic(const TapGeom& g, FwdPlan& c, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout,
+                          void* out, const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st,
+                          const TcFusion* fuse, TcStats* stats) {
+  const size_t esz = out_f32 ? 4 : 2;
+  const size_t wrow = (size_t)g.ntaps * (C0 + C1);
+  for (int n0 = 0; n0 < Nout; n0 += c.slice) {
+    const int ns = Nout - n0 < c.slice ? Nout - n0 : c.slice;
+    if (ns != c.gen.p.Cz) {
+      if (const char* why = plan_generic(g, C0, C1, ns, Nout, out_f32, false, false, c.gen)) return fail(DCB_ERR_UNSUPPORTED, "%s", why);
+    }
+    TcFwdParams& p = c.gen.p;
+    const void* Bs = reinterpret_cast<const __nv_bfloat16*>(B) + (size_t)n0 * wrow;
+    void* o = reinterpret_cast<uint8_t*>(out) + (size_t)n0 * esz;
+    p.relu = relu; p.out = reinterpret_cast<__nv_bfloat16*>(o);
+    p.scale = scale ? scale + n0 : nullptr; p.shift = shift ? shift + n0 : nullptr;
+    if (c.gen.pool) p.pool_out = reinterpret_cast<__nv_bfloat16*>(fuse->pool_out);
+    if (c.gen.stats) p.stat_sums = stats->sums;
+    const int swz = p.BK * 2;
+    CUtensorMap mA0, mA1, mB;
+    auto make_src_map = [&](CUtensorMap* m, const void* ptr, int C) -> int {
+      if (p.mode == 0) return map_nhwc(m, g.f16, ptr, g.N, g.IH, g.IW, C, C, p.BK, p.bw, p.bh, p.bn, swz);
+      if (p.mode == 1) return map_rows(m, g.f16, ptr, (long long)g.N * g.IH, g.IW, C, p.BK, p.bw, p.bh, swz);
+      return map_subpixel(m, g.f16, ptr, (long long)g.N * g.GH, g.GW, C, C, p.BK, p.bw, p.bh, swz);   // dy [N][2h][2w][C]
+    };
+    if (int e = make_src_map(&mA0, s0, C0)) return e;
+    if (C1 > 0) { if (int e = make_src_map(&mA1, s1, C1)) return e; }
+    else mA1 = mA0;
+    if (int e = map_weights(&mB, g.f16, Bs, g.ntaps * (C0 + C1), p.Ntot, p.BK, p.BN, swz)) return e;
+    CUtensorMap mO = mB;
+    if (p.tma_store) {
+      const int e = p.mode == 0 ? map_nhwc(&mO, g.f16, o, g.N, g.OH, g.OW, ns, Nout, 32, p.bw, p.bh, p.bn, 64)
+                                : map_subpixel(&mO, g.f16, o, (long long)g.N * g.GH, g.GW, ns, Nout, 32, p.bw, p.bh, 64);   // convT fwd y
+      if (e) return e;
+    }
+    auto* k = c.gen.stats ? tapgemm_tc_fwd_kernel<false, true> : c.gen.pool ? tapgemm_tc_fwd_kernel<true, false>
+                                                                           : tapgemm_tc_fwd_kernel<false, false>;
+    if (int e = launch(k, "tapgemm_tc_fwd_kernel", c.gen.grid, TC_THREADS, c.gen.dyn, TC_SMEM_MAX, st, policy(DCB_POLICY_PDL) != 0,
+                       0, mA0, mA1, mB, mO, p))
+      return e;
+  }
+  return DCB_OK;
+}
+
+static int launch_flat(const TapGeom& g, FwdPlan& c, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout,
+                       void* out, const float* scale, const float* shift, int relu, cudaStream_t st, TcStats* stats) {
+  TcFlatParams& p = c.flat.p;
+  p.relu = relu; p.out = out; p.scale = scale; p.shift = shift;
+  if (c.flat.stats) p.stat_sums = stats->sums;
+  CUtensorMap mA0, mA1, mB;
+  if (int e = map_nhwc(&mA0, g.f16, s0, g.N, g.IH, g.IW, C0, C0, 64, p.Wp, p.R, 1, 128)) return e;
+  if (C1 > 0) { if (int e = map_nhwc(&mA1, g.f16, s1, g.N, g.IH, g.IW, C1, C1, 64, p.Wp, p.R, 1, 128)) return e; } else mA1 = mA0;
+  if (int e = map_weights(&mB, g.f16, B, 9 * (C0 + C1), Nout, 64, p.wrows, 128)) return e;
+  return launch(c.flat.stats ? tapgemm_tc_flat_kernel<true> : tapgemm_tc_flat_kernel<false>, "tapgemm_tc_flat_kernel", c.flat.grid,
+                FL_THREADS, c.flat.dyn, FL_SMEM_MAX, st, policy(DCB_POLICY_PDL) != 0, 0, mA0, mA1, mB, p);
+}
+
+// fuse != nullptr: the caller wants the head and/or the 2x2 max-pool computed in the conv epilogue; returns
+// DCB_ERR_UNSUPPORTED (without launching) when this layer shape cannot take the fused path.
+int run_tc_fwd(const TapGeom& g, const void* s0, int C0, const void* s1, int C1, const void* B, int Nout, void* out,
+               const float* scale, const float* shift, int relu, int out_f32, cudaStream_t st, const TcFusion* fuse, TcStats* stats) {
+  if (stats) stats->done = 0;
+  if (stats && (fuse || out_f32)) return fail(DCB_ERR_INVALID_ARGUMENT, "batch statistics: plain 16-bit forward only");
+  if (C0 % 32 != 0 || C1 % 32 != 0 || Nout % 32 != 0)
+    return fail(DCB_ERR_UNSUPPORTED, "bf16 tensor-core path needs channel counts that are multiples of 32 "
+                "(got C0=%d C1=%d Cout=%d); use the fp32 check mode for other widths", C0, C1, Nout);
+  FwdPlan c = choose_fwd(g, C0, C1, Nout, fuse, stats != nullptr, out_f32);
+  int e = DCB_OK;
+  switch (c.kind) {
+    case FwdPlan::UNSUPPORTED: return fail(DCB_ERR_UNSUPPORTED, "%s", c.error);
+    case FwdPlan::GENERIC: e = launch_generic(g, c, s0, C0, s1, C1, B, Nout, out, scale, shift, relu, out_f32, st, fuse, stats); break;
+    case FwdPlan::FLAT: e = launch_flat(g, c, s0, C0, s1, C1, B, Nout, out, scale, shift, relu, st, stats); break;
+    default: e = launch_strip(g, c, s0, C0, s1, C1, B, Nout, out, scale, shift, relu, out_f32, st, fuse, stats); break;
+  }
+  if (e) return e;
+  if (stats) stats->done = c.stats ? 1 : 0;
+  note_kernel(fwd_kernel_name(c));
   return DCB_OK;
 }
 
@@ -2952,31 +2944,16 @@ static int run_tc_wgrad_strip(const TapGeom& g, const WgradBlock* blk, int nblk,
   if (!ws || ws_bytes < need) return fail(DCB_ERR_WORKSPACE, "wgrad (bf16 strip): workspace %zu B < required %zu B", ws_bytes, need);
   p.part = reinterpret_cast<float*>(ws);
   CUtensorMap mA0, mA1, mG;
-  auto mk = [&](CUtensorMap* m, const WgradBlock& b) -> int {
-    uint64_t dims[4] = {(uint64_t)b.C, (uint64_t)g.IW, (uint64_t)g.IH, (uint64_t)g.N};
-    uint64_t str[3] = {(uint64_t)b.C * 2, (uint64_t)g.IW * b.C * 2, (uint64_t)g.IH * g.IW * b.C * 2};
-    uint32_t box[4] = {32, 66, 1, 1};
-    return make_map(m, b.ptr, 4, dims, str, box, 64);
-  };
-  if (int e = mk(&mA0, blk[0])) return e;
-  if (nblk > 1) { if (int e = mk(&mA1, blk[1])) return e; } else mA1 = mA0;
-  {
-    uint64_t dims[4] = {(uint64_t)Nout, (uint64_t)g.GW, (uint64_t)g.GH, (uint64_t)g.N};
-    uint64_t str[3] = {(uint64_t)Nout * 2, (uint64_t)g.GW * Nout * 2, (uint64_t)g.GH * g.GW * Nout * 2};
-    uint32_t box[4] = {(uint32_t)Nout, (uint32_t)WS_PX, 1, 1};
-    if (int e = make_map(&mG, G, 4, dims, str, box, Nout * 2)) return e;
-  }
+  if (int e = map_nhwc(&mA0, g.f16, blk[0].ptr, g.N, g.IH, g.IW, blk[0].C, blk[0].C, 32, 66, 1, 1, 64)) return e;
+  if (nblk > 1) { if (int e = map_nhwc(&mA1, g.f16, blk[1].ptr, g.N, g.IH, g.IW, blk[1].C, blk[1].C, 32, 66, 1, 1, 64)) return e; }
+  else mA1 = mA0;
+  if (int e = map_nhwc(&mG, g.f16, G, g.N, g.GH, g.GW, Nout, Nout, Nout, WS_PX, 1, 1, Nout * 2)) return e;
   const size_t dyn = (size_t)WS_RING * nblk * 5120 + (size_t)WS_GRING * WS_PX * Nout * 2 + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_wgrad_strip_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-    if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
-  tapgemm_tc_wgrad_strip_kernel<<<grid, WG_THREADS, dyn, st>>>(mA0, mA1, mG, p);
-  DCB_LAUNCH_OK("tapgemm_tc_wgrad_strip_kernel");
+  if (int e = launch(tapgemm_tc_wgrad_strip_kernel, "tapgemm_tc_wgrad_strip_kernel", grid, WG_THREADS, dyn, 160 * 1024, st, false, 0,
+                     mA0, mA1, mG, p))
+    return e;
   launch_reduce_splits_rows(p.part, grid, 9, K * Nout, dW + (size_t)k_off * Nout, (size_t)K_total * Nout, st);
-  g_launches += 2;
+  g_launches += 1;
   DCB_LAUNCH_OK("reduce_splits_kernel");
   note_kernel("wgrad_strip");
   return DCB_OK;
@@ -2985,7 +2962,6 @@ static int run_tc_wgrad_strip(const TapGeom& g, const WgradBlock* blk, int nblk,
 int run_tc_wgrad(const TapGeom& g, const void* s0, int C0, const void* s1, int C1, const void* G, int Nout, float* dW,
                  void* ws, size_t ws_bytes, cudaStream_t st) {
   if (g.f16) return fail(DCB_ERR_UNSUPPORTED, "the fp16 mode is inference only: gradients are computed in bf16 (or fp32 check) mode");
-  t_map_f16 = 0;
   if (C0 % 32 != 0 || C1 % 32 != 0 || Nout % 32 != 0)
     return fail(DCB_ERR_UNSUPPORTED, "bf16 tensor-core wgrad needs channel counts that are multiples of 32 "
                 "(got C0=%d C1=%d N=%d)", C0, C1, Nout);
@@ -3015,44 +2991,23 @@ int run_tc_wgrad(const TapGeom& g, const void* s0, int C0, const void* s1, int C
 
   CUtensorMap mA0, mA1, mG;
   auto make_a = [&](CUtensorMap* m, const void* ptr, int C) -> int {
-    if (!convT) {
-      uint64_t dims[4] = {(uint64_t)C, (uint64_t)g.IW, (uint64_t)g.IH, (uint64_t)g.N};
-      uint64_t str[3] = {(uint64_t)C * 2, (uint64_t)g.IW * C * 2, (uint64_t)g.IH * g.IW * C * 2};
-      uint32_t box[4] = {(uint32_t)w.CB, (uint32_t)w.bw, (uint32_t)w.bh, (uint32_t)w.bn};
-      return make_map(m, ptr, 4, dims, str, box, w.CB * 2);
-    }
-    uint64_t dims[5] = {(uint64_t)C, 2, (uint64_t)g.GW, 2, (uint64_t)g.N * g.GH};
-    uint64_t str[4] = {(uint64_t)C * 2, (uint64_t)2 * C * 2, (uint64_t)g.IW * C * 2, (uint64_t)2 * g.IW * C * 2};
-    uint32_t box[5] = {(uint32_t)w.CB, 1, (uint32_t)w.bw, 1, (uint32_t)w.bh};
-    return make_map(m, ptr, 5, dims, str, box, w.CB * 2);
+    if (!convT) return map_nhwc(m, g.f16, ptr, g.N, g.IH, g.IW, C, C, w.CB, w.bw, w.bh, w.bn, w.CB * 2);
+    return map_subpixel(m, g.f16, ptr, (long long)g.N * g.GH, g.GW, C, C, w.CB, w.bw, w.bh, w.CB * 2);
   };
   if (int e = make_a(&mA0, s0, C0)) return e;
   if (C1 > 0) { if (int e = make_a(&mA1, s1, C1)) return e; } else mA1 = mA0;
-  if (!convT) {
-    uint64_t dims[4] = {(uint64_t)Nout, (uint64_t)g.GW, (uint64_t)g.GH, (uint64_t)g.N};
-    uint64_t str[3] = {(uint64_t)Nout * 2, (uint64_t)g.GW * Nout * 2, (uint64_t)g.GH * g.GW * Nout * 2};
-    uint32_t box[4] = {(uint32_t)w.CBG, (uint32_t)w.bw, (uint32_t)w.bh, (uint32_t)w.bn};
-    if (int e = make_map(&mG, G, 4, dims, str, box, w.CBG * 2)) return e;
-  } else {
-    uint64_t dims[3] = {(uint64_t)Nout, (uint64_t)g.GW, (uint64_t)g.N * g.GH};
-    uint64_t str[2] = {(uint64_t)Nout * 2, (uint64_t)g.GW * Nout * 2};
-    uint32_t box[3] = {(uint32_t)w.CBG, (uint32_t)w.bw, (uint32_t)w.bh};
-    if (int e = make_map(&mG, G, 3, dims, str, box, w.CBG * 2)) return e;
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 206 * 1024);
-    if (e != cudaSuccess) return fail(DCB_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
+  if (int e = convT ? map_rows(&mG, g.f16, G, (long long)g.N * g.GH, g.GW, Nout, w.CBG, w.bw, w.bh, w.CBG * 2)
+                    : map_nhwc(&mG, g.f16, G, g.N, g.GH, g.GW, Nout, Nout, w.CBG, w.bw, w.bh, w.bn, w.CBG * 2))
+    return e;
   const size_t stage_bytes = (size_t)WG_P * 128 * 2 + (size_t)WG_P * w.BN * 2;
   const size_t dyn_smem = w.stages * stage_bytes + 1024;
   const int num_items = cdiv(K, 128) * (Nout / w.BN) * g.ntaps * w.splits;
   const int grid = num_items < sm_count() ? num_items : sm_count();
-  tapgemm_tc_wgrad_kernel<<<grid, WG_THREADS, dyn_smem, st>>>(mA0, mA1, mG, p);
-  DCB_LAUNCH_OK("tapgemm_tc_wgrad_kernel");
+  if (int e = launch(tapgemm_tc_wgrad_kernel, "tapgemm_tc_wgrad_kernel", grid, WG_THREADS, dyn_smem, TC_SMEM_MAX, st, false, 0,
+                     mA0, mA1, mG, p))
+    return e;
   launch_reduce_splits(p.part, w.splits, (size_t)g.ntaps * K * Nout, dW, st);
-  g_launches += 2;
+  g_launches += 1;
   DCB_LAUNCH_OK("reduce_splits_kernel");
   note_kernel("wgrad");
   return DCB_OK;

@@ -231,11 +231,16 @@ def test_policy_roundtrip_and_kernel_names(cuda):
     assert run(2, 32, 32, 64, 64) in ('generic', 'generic_swap')          # too few work items for the flat kernel
 
 
+CONVT_CASES = [
+    # N, h, w, Cin, Cout
+    (1, 8, 8, 64, 32), (2, 4, 4, 512, 256), (1, 16, 16, 128, 64), (3, 2, 2, 256, 128), (4, 64, 64, 128, 64), (8, 64, 64, 64, 32),
+    (2, 4, 4, 1024, 512),          # up3 of nb_filters_base 64
+    (8, 10, 10, 256, 128),         # a 640 tile's 80^2 level
+]
+
+
 @pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
-@pytest.mark.parametrize('case', [(1, 8, 8, 64, 32), (2, 4, 4, 512, 256), (1, 16, 16, 128, 64), (3, 2, 2, 256, 128),
-                                  (4, 64, 64, 128, 64), (8, 64, 64, 64, 32),
-                                  (2, 4, 4, 1024, 512),          # up3 of nb_filters_base 64
-                                  (8, 10, 10, 256, 128)])        # a 640 tile's 80^2 level
+@pytest.mark.parametrize('case', CONVT_CASES)
 def test_convT2x2_fwd_dgrad_wgrad(cuda, precision, case):
     from deepcalcium.engine import ops
     N, h, w_, Cin, Cout = case
@@ -289,13 +294,19 @@ def test_convT2x2_fwd_dgrad_wgrad(cuda, precision, case):
         assert torch.max(torch.abs(dW.cpu().double() - kt.grad)).item() < tol(precision, 1 + kt.grad.abs().max().item())
 
 
+FUSED_SHAPES = [
+    # N, H, W, Cin, Cout
+    (2, 16, 128, 32, 32), (1, 6, 256, 64, 64), (1, 8, 24, 32, 32), (2, 40, 256, 32, 32), (1, 44, 512, 64, 32),
+    (2, 8, 512, 64, 64), (8, 4, 640, 64, 64),        # full-resolution 64 -> 64 (nfb 64)
+    # pooled epilogue of the generic kernel: pixels-as-M tiles (several tile shapes, an N tile narrower than Cout),
+    # weights-as-M tiles of 128x2 and 64x4 pixels
+    (2, 32, 32, 128, 128), (3, 8, 8, 256, 256), (8, 64, 64, 128, 256),
+    (8, 128, 128, 64, 128), (16, 64, 64, 64, 128), (1, 16, 128, 64, 128),
+]
+
+
 @pytest.mark.parametrize('precision', ['fp32', 'bf16', 'fp16'])
-@pytest.mark.parametrize('shape', [(2, 16, 128, 32, 32), (1, 6, 256, 64, 64), (1, 8, 24, 32, 32), (2, 40, 256, 32, 32), (1, 44, 512, 64, 32),
-                                   (2, 8, 512, 64, 64), (8, 4, 640, 64, 64),        # full-resolution 64 -> 64 (nfb 64)
-                                   # pooled epilogue of the generic kernel: pixels-as-M tiles (several tile shapes, an N tile
-                                   # narrower than Cout), weights-as-M tiles of 128x2 and 64x4 pixels
-                                   (2, 32, 32, 128, 128), (3, 8, 8, 256, 256), (8, 64, 64, 128, 256),
-                                   (8, 128, 128, 64, 128), (16, 64, 64, 64, 128), (1, 16, 128, 64, 128)])
+@pytest.mark.parametrize('shape', FUSED_SHAPES)
 def test_conv3x3_fused_pool_and_head_equal_the_unfused_composition(cuda, precision, shape):
     """dcb_conv3x3_fwd_fused (max-pool / softmax head folded into the conv epilogue) must reproduce the separate
     kernels - including shapes where the library falls back to the unfused composition.  fp32: exactly.  bf16: the
